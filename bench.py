@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the stereo hot path on N B200s (one process per GPU).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): stereo pairs/s for costvol + dispreg + reproj at 544x960,
 D = 192, and the fraction of the HBM roofline the dominant kernel reaches.
@@ -233,6 +233,24 @@ def make_inputs(nb, seed, device="cpu", pin=False):
     return ts
 
 
+VOLUME_SAMPLE = 1 << 22  # cost-volume elements --dump-outputs keeps (16 MB of the 3.3 GB volume)
+
+
+def dump_outputs(out_dir, outputs):
+    """Write what one step returns to its caller as float32 <name>.npy files in `out_dir`: the disparity, the loss and
+    the fold image whole, and of the cost volume the VOLUME_SAMPLE elements at flat indices drawn from a generator
+    seeded with 0, in increasing index order (50 MB in all at B = 8)."""
+    import numpy as np
+
+    vol, disp, loss, vis = outputs
+    idx = torch.randint(vol.numel(), (VOLUME_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+    arrays = {"cost_volume_sample": vol.reshape(-1)[idx.to(vol.device)], "disparity": disp, "loss": loss,
+              "fold_image": vis}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 def time_cpu_reference(steps, warmup):
     from oracle import stereo_oracle as so
 
@@ -360,6 +378,8 @@ def run_b200(args, rank, world, local_rank):
         launches = launches_per_step * args.steps
         ms_total = start.elapsed_time(stop)
         loss_graph = float(gout[2])
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, gout)
         del gout, graph
 
         # ---- end to end: pinned host -> device, compute, results back, every step ----
@@ -770,7 +790,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-train-variant", action="store_true")
     ap.add_argument("--no-stock-variant", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="B200 arm: after the timed steps, write the outputs of the last one as DIR/<name>.npy "
+                         "(rank 0's batch)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -51,6 +51,29 @@ def test_committed_b200_line_has_the_contract_keys():
     assert abs(bp["value"] - pairs / (bp["ms_per_step"] * 1e-3)) <= 1e-6 * bp["value"] and 0.8 < bp["pipeline_frac"] < 1.0
 
 
+def test_dump_outputs_writes_the_step_outputs_as_float32(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+
+    import bench
+
+    # at the bench's shapes: at most 64 MB in all
+    assert 4 * (2 * bench.B * bench.H * bench.W + 1 + bench.VOLUME_SAMPLE) <= 64e6
+    monkeypatch.setattr(bench, "VOLUME_SAMPLE", 100)
+    vol = torch.randn(2, 8, 3, 5, 7)
+    disp, vis = torch.rand(2, 1, 20, 28), torch.rand(2, 1, 20, 28)
+    loss = torch.tensor(0.25)
+    bench.dump_outputs(str(tmp_path / "out"), (vol, disp, loss, vis))
+    got = {p.stem: np.load(p) for p in (tmp_path / "out").glob("*.npy")}
+    assert sorted(got) == ["cost_volume_sample", "disparity", "fold_image", "loss"]
+    assert all(a.dtype == np.float32 for a in got.values())
+    assert np.array_equal(got["disparity"], disp.numpy()) and np.array_equal(got["fold_image"], vis.numpy())
+    assert got["loss"] == np.float32(0.25)
+    # the sample is fixed: the same flat indices on every run
+    idx = torch.randint(vol.numel(), (bench.VOLUME_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+    assert np.array_equal(got["cost_volume_sample"], vol.reshape(-1)[idx].numpy())
+
+
 def test_reference_arm_runs_and_prints_one_json_line():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1",
                           "--warmup", "0"], capture_output=True, text=True, timeout=600, cwd=ROOT)
