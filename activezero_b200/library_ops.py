@@ -18,7 +18,10 @@ operators instead of Python:
     torch.ops.az_stereo.local_contrast_norm(image, kernel_size, eps) -> (normed, std) (reprojection.py:175-200)
 
 The first six are differentiable (each backward is itself a registered op, so a compiled backward graph stays
-opaque too); the last three are the non-differentiable operators of SURVEY.md §8b.
+opaque too); the last three are the non-differentiable operators of SURVEY.md §8b.  Importing this module also
+registers the differentiable first aggregation convolution on the implicit volume (``_volume_conv_library``):
+
+    torch.ops.az_stereo.volume_conv(ref, tgt, weight, num_disp) -> out               (psmnet.py:151-168)
 
 The convenience wrappers below return what the reference-named functions return.  Nothing here computes on the
 host: every implementation enqueues the CUDA kernels of ``libaz_stereo.so`` (no CPU fallback).
@@ -30,10 +33,16 @@ from typing import Tuple
 import torch
 from torch import Tensor
 
-from . import _lib
+from . import _lib, _volume_conv_library
 from .ops import _cuda_f32, _mask_u8, _ptr, _stream, check_feature_pair, check_reproj_inputs, linspace_table
 
 NS = "az_stereo"
+
+
+def volume_conv(ref: Tensor, tgt: Tensor, weight: Tensor, num_disp: int) -> Tensor:
+    """conv3d(concat_volume(ref, tgt, num_disp), weight, padding=1) without the volume, differentiable in all three
+    inputs (``torch.ops.az_stereo.volume_conv``)."""
+    return _volume_conv_library.volume_conv(ref, tgt, weight, int(num_disp))
 
 
 # ---------------------------------------------------------------------------------------------

@@ -142,6 +142,10 @@ class PSMNetBase(nn.Module):
         # concat volume's values straight from the two feature maps (SURVEY.md §8f rank 2, implicit clause): the
         # [B,64,D/4,H/4,W/4] volume is never written nor re-read.  TF32 operands like cuDNN's default conv path.
         self.fuse_volume_conv = False
+        # True: every forward that records gradients (training, or eval with grad enabled) computes dres0's first Conv3d
+        # on the implicit volume too (ops.volume_conv: tcgen05 TF32 forward, volume-free fp32 backward); its BatchNorm3d
+        # (in the module's own mode) and ReLU stay in torch.  Neither the volume nor its gradient is materialised.
+        self.fuse_volume_conv_train = False
         self._vc_cache = None
         self.feature_extraction = feature_extraction
         self.dres0 = nn.Sequential(convbn_3d(64, 32, 3, 1, 1), nn.ReLU(inplace=True),
@@ -229,11 +233,19 @@ class PSMNetBase(nn.Module):
                 first = first.contiguous(memory_format=torch.channels_last_3d)
             _, _, cost3 = self._aggregate(None, first)
             return self._disparity_head(cost3, H, W)
-        if self.volume_channels_last:
-            cost = ops.build_concat_volume(ref_feat, tgt_feat, self.maxdisp // 4, channels_last=True)
+        if self.fuse_volume_conv_train and torch.is_grad_enabled():
+            # dres0[0] = Conv3d + BatchNorm3d, dres0[1] = ReLU
+            conv = ops.volume_conv(ref_feat, tgt_feat, self.dres0[0][0].weight, self.maxdisp // 4)
+            first = self.dres0[1](self.dres0[0][1](conv))
+            if self.volume_channels_last:
+                first = first.contiguous(memory_format=torch.channels_last_3d)
+            cost1, cost2, cost3 = self._aggregate(None, first)
         else:
-            cost = ops.build_concat_volume(ref_feat, tgt_feat, self.maxdisp // 4)  # replaces psmnet.py:151-165
-        cost1, cost2, cost3 = self._aggregate(cost)
+            if self.volume_channels_last:
+                cost = ops.build_concat_volume(ref_feat, tgt_feat, self.maxdisp // 4, channels_last=True)
+            else:
+                cost = ops.build_concat_volume(ref_feat, tgt_feat, self.maxdisp // 4)  # replaces psmnet.py:151-165
+            cost1, cost2, cost3 = self._aggregate(cost)
         pred3 = self._disparity_head(cost3, H, W)
         if self.training:
             pred1 = self._disparity_head(cost1, H, W)

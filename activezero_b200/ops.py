@@ -170,6 +170,76 @@ def volume_conv0(ref_feat, tgt_feat, wpacked, num_disp: int, scale=None, shift=N
     return out
 
 
+def check_volume_conv_inputs(ref_feat, tgt_feat, weight, num_disp: int, what: str):
+    """Shared by ops and library_ops: features CUDA float32 [B,32,H,W], weight [32,64,3,3,3] on their device."""
+    L, R = check_feature_pair(ref_feat, tgt_feat, what)
+    if L.shape[1] != 32:
+        raise ValueError(f"{what}: PSMNet's 32 feature channels expected, got {L.shape[1]}")
+    w = _cuda_f32(weight, "weight")
+    if tuple(w.shape) != (32, 64, 3, 3, 3) or w.device != L.device:
+        raise ValueError(f"{what}: expected a [32,64,3,3,3] Conv3d weight on the features' device, got {tuple(w.shape)}")
+    if int(num_disp) <= 0:
+        raise ValueError(f"{what}: num_disp must be positive")
+    return L, R, w
+
+
+def volume_conv_backward_into(gout, L, R, w, gL, gR, gW):
+    """Enqueues az_volume_conv0_bwd for the validated tensors; gL / gR / gW may each be None (skipped)."""
+    B, C, H, W = L.shape
+    Dq = gout.shape[2]
+    if tuple(gout.shape) != (B, 32, Dq, H, W) or gout.device != L.device:
+        raise ValueError(f"volume conv backward: grad_out must be [B,32,Dq,H,W] = {(B, 32, Dq, H, W)} on the features' "
+                         f"device, got {tuple(gout.shape)}")
+    if B == 0:
+        if gW is not None:
+            gW.zero_()  # a sum over no position
+        return
+    ws = torch.empty((_lib.query("az_volume_conv0_bwd_workspace_bytes", B, H, W, Dq),), dtype=torch.uint8, device=L.device)
+    with torch.cuda.device(L.device):
+        _lib.call("az_volume_conv0_bwd", _ptr(gout), _ptr(L), _ptr(R), _ptr(w), _ptr(gL), _ptr(gR), _ptr(gW), _ptr(ws),
+                  B, C, H, W, Dq, _stream(), batch=B)
+
+
+class VolumeConv0Fn(torch.autograd.Function):
+    """conv3d(concat_volume(ref, tgt, num_disp), weight, padding=1) -- dres0[0][0] on the implicit volume
+    (psmnet.py:151-168) -- differentiable in all three inputs.  Forward: the tcgen05 kernel (TF32 operands, fp32
+    accumulation).  Backward: the volume-free fp32 kernels of csrc/volume_conv_bwd.cu.  Saves the features and the
+    weight only (feature-sized, not volume-sized)."""
+
+    @staticmethod
+    @_fwd32
+    def forward(ctx, ref_feat, tgt_feat, weight, num_disp: int):
+        L, R, w = check_volume_conv_inputs(ref_feat, tgt_feat, weight, num_disp, "volume conv")
+        B, C, H, W = L.shape
+        out = torch.empty((B, 32, int(num_disp), H, W), dtype=torch.float32, device=L.device)
+        if B > 0:
+            wp = pack_volume_conv_weight(w)
+            with torch.cuda.device(L.device):
+                _lib.call("az_volume_conv0_fwd", _ptr(L), _ptr(R), _ptr(wp), _NULL, _NULL, _ptr(out), B, C, H, W,
+                          int(num_disp), 0, _stream(), batch=B)
+        ctx.save_for_backward(L, R, w)
+        return out
+
+    @staticmethod
+    @once_differentiable
+    @_bwd
+    def backward(ctx, gout):
+        L, R, w = ctx.saved_tensors
+        g = _cuda_f32(gout, "grad_out")
+        gL = torch.empty_like(L) if ctx.needs_input_grad[0] else None
+        gR = torch.empty_like(R) if ctx.needs_input_grad[1] else None
+        gW = torch.empty_like(w) if ctx.needs_input_grad[2] else None
+        volume_conv_backward_into(g, L, R, w, gL, gR, gW)
+        return gL, gR, gW, None
+
+
+def volume_conv(ref_feat, tgt_feat, weight, num_disp: int):
+    """[B,32,H,W] x2, Conv3d weight [32,64,3,3,3] -> conv3d(concat_volume(ref, tgt, num_disp), weight, padding=1),
+    [B,32,num_disp,H,W], with autograd; the concat volume and its gradient are never materialised.  The raw
+    convolution: no BatchNorm fold, no ReLU (``volume_conv0`` is the inference form with both)."""
+    return VolumeConv0Fn.apply(ref_feat, tgt_feat, weight, num_disp)
+
+
 # ----------------------------------------------------------------------------
 # a3 group-wise correlation volume (no reference counterpart)
 # ----------------------------------------------------------------------------

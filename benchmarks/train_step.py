@@ -112,6 +112,8 @@ def main():
                     help="emit the cost volume in channels_last_3d (SURVEY 8f rank 2, layout clause)")
     ap.add_argument("--fuse-upsample", action="store_true",
                     help="use the fused trilinear-upsample + soft-argmin kernel for the three heads (SURVEY §8f-1)")
+    ap.add_argument("--fuse-volume-conv", action="store_true",
+                    help="dres0's first Conv3d on the implicit volume in training too (PSMNet.fuse_volume_conv_train)")
     ap.add_argument("--profile", action="store_true", help="after the timed region: kernel-time shares via torch.profiler")
     args = ap.parse_args()
 
@@ -122,6 +124,7 @@ def main():
     torch.manual_seed(1)  # cfg.SOLVER.SEED, configs/config.py:100
     model = PSMNet(maxdisp=MAX_DISP).to(dev)
     model.fuse_upsample = args.fuse_upsample
+    model.fuse_volume_conv_train = args.fuse_volume_conv
     if args.channels_last_3d:
         model.use_channels_last_3d(True)
     if world > 1:
@@ -190,7 +193,7 @@ def main():
             "steps": args.steps, "ms_per_iteration": ms / args.steps, "scaling": "weak",
             "config": {"workload": f"config{'3' if args.no_real else '4'}: PSMNet_3 train step {args.height}x{args.width}, "
                                    f"D={MAX_DISP}, batch {args.batch}/GPU, patch reproj ps={PATCH}, T={args.frames}",
-                       "ddp": world > 1, "fuse_upsample": args.fuse_upsample,
+                       "ddp": world > 1, "fuse_upsample": args.fuse_upsample, "fuse_volume_conv": args.fuse_volume_conv,
                        "channels_last_3d": args.channels_last_3d},
             "device_time_shares_rank0": shares,
             "final_loss": float(last)}), flush=True)

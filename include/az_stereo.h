@@ -63,6 +63,23 @@ int az_concat_volume_bwd_ndhwc(const float* gvol, float* gL, float* gR,
 int az_volume_conv0_pack(const float* weight, float* wpacked, void* stream);
 int az_volume_conv0_fwd(const float* L, const float* R, const float* wpacked, const float* scale, const float* shift,
                         float* out, int64_t B, int64_t C, int64_t H, int64_t W, int64_t Dq, int relu, void* stream);
+/* Backward of the raw convolution above (no scale/shift, no ReLU), without the volume or its gradient.  With
+ * gout = dLoss/d out [B,32,Dq,H,W], Wl = weight[:, :32], Wr = weight[:, 32:] and, for each tap (kd,kx),
+ * lo = max(0,1-kd), hi = min(Dq-1,Dq-kd):
+ *   A[kd,kx][b,o,y,x] = sum_{d=lo}^{min(x+kx-kd,hi)} gout[b,o,d,y,x]
+ *   Z[kd,kx][b,o,y,u] = sum_{d=lo}^{hi} gout[b,o,d,y,u+d+kd-kx]  over the d with 0 <= u+d+kd-kx <= min(W-1,W-kx)
+ *   gL[b,c,y',x'] = sum_{o,kd,ky,kx} Wl[o,c,kd,ky,kx] * A[kd,kx][b,o,y'-ky+1,x'-kx+1]   (zero outside the image)
+ *   gR[b,c,y',u]  = sum_{o,kd,ky,kx} Wr[o,c,kd,ky,kx] * Z[kd,kx][b,o,y'-ky+1,u]
+ *   gW[o,c,kd,ky,kx]    = sum_{b,y',x'} A[kd,kx][b,o,y'-ky+1,x'-kx+1] * L[b,c,y',x']
+ *   gW[o,32+c,kd,ky,kx] = sum_{b,y',u}  Z[kd,kx][b,o,y'-ky+1,u]       * R[b,c,y',u]
+ * fp32 on the CUDA cores, fixed summation order, atomic-free (bit-identical run to run).  weight: the plain Conv3d
+ * weight [32,64,3,3,3] (not the packed copy); L,R,gL,gR: [B,32,H,W]; gW: [32,64,3,3,3]; each of gL, gR, gW may be
+ * NULL (that part is skipped) and all three are fully written.  C must be 32; any Dq.
+ * workspace: az_volume_conv0_bwd_workspace_bytes(B,H,W,Dq) bytes, 16-byte aligned (holds the 18 planes A, Z). */
+int64_t az_volume_conv0_bwd_workspace_bytes(int64_t B, int64_t H, int64_t W, int64_t Dq);
+int az_volume_conv0_bwd(const float* gout, const float* L, const float* R, const float* weight,
+                        float* gL, float* gR, float* gW, void* workspace,
+                        int64_t B, int64_t C, int64_t H, int64_t W, int64_t Dq, void* stream);
 
 /* ---- a3: group-wise correlation volume -- NOT IN THE REFERENCE (SURVEY.md fact 1; parity unpinned) ----
  * vol[b,g,i,y,x] = (1/(C/G)) * sum_{c in group g} L[b,c,y,x]*R[b,c,y,x-i]  (x >= i, else 0); vol: [B,G,Dq,H,W]. */
