@@ -32,8 +32,12 @@ SIGNATURES = {
     "az_concat_volume_bwd": (ctypes.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "az_concat_volume_fwd_ndhwc": (ctypes.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "az_concat_volume_bwd_ndhwc": (ctypes.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _P]),
+    "az_concat_volume_fwd_16": (ctypes.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, ctypes.c_int, _P]),
+    "az_concat_volume_bwd_16": (ctypes.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, ctypes.c_int, ctypes.c_int, _P]),
     "az_volume_conv0_pack": (ctypes.c_int, [_P, _P, _P]),
     "az_volume_conv0_fwd": (ctypes.c_int, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, ctypes.c_int, _P]),
+    "az_volume_conv0_pack_16": (ctypes.c_int, [_P, _P, ctypes.c_int, _P]),
+    "az_volume_conv0_fwd_16": (ctypes.c_int, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, ctypes.c_int, ctypes.c_int, _P]),
     "az_volume_conv0_bwd_workspace_bytes": (_I, [_I, _I, _I, _I]),
     "az_volume_conv0_bwd": (ctypes.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "az_gwc_volume_fwd": (ctypes.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),

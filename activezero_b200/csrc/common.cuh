@@ -1,5 +1,7 @@
 // Shared device/host helpers for libaz_stereo (sm_100a only).
 #pragma once
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdlib.h>
@@ -50,6 +52,16 @@ __device__ __forceinline__ void st_stream8(float* p, const float8& r) {  // evic
                  "f"(r.v[3]), "f"(r.v[4]), "f"(r.v[5]), "f"(r.v[6]), "f"(r.v[7])
                  : "memory");
 }
+
+// ---- fp32 / 16-bit element access for kernels templated on the tensor dtype ----------------------------
+// ld_f32: load one element and widen it to fp32 (exact for bf16 and fp16); st_from_f32: round once to the element
+// type, to nearest even, and store.
+__device__ __forceinline__ float ld_f32(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ld_f32(const __nv_bfloat16* p) { return __bfloat162float(__ldg(p)); }
+__device__ __forceinline__ float ld_f32(const __half* p) { return __half2float(__ldg(p)); }
+__device__ __forceinline__ void st_from_f32(float* p, float v) { *p = v; }
+__device__ __forceinline__ void st_from_f32(__nv_bfloat16* p, float v) { *p = __float2bfloat16_rn(v); }
+__device__ __forceinline__ void st_from_f32(__half* p, float v) { *p = __float2half_rn(v); }
 
 // ---- block reductions ---------------------------------------------------------------------
 __device__ __forceinline__ float warp_sum(float v) {

@@ -50,10 +50,12 @@ __device__ __forceinline__ float to_tf32(float x) {
     return __uint_as_float(u);
 }
 
-__global__ void __launch_bounds__(kVcThreads) volume_conv0_kernel(const float* __restrict__ L, const float* __restrict__ R,
+// T = the features' and the output's element type: float, or bf16 / fp16 (widened at the gather, rounded once at the store)
+template <typename T>
+__global__ void __launch_bounds__(kVcThreads) volume_conv0_kernel(const T* __restrict__ L, const T* __restrict__ R,
                                                                   const float* __restrict__ wpacked,
                                                                   const float* __restrict__ scale,
-                                                                  const float* __restrict__ shift, float* __restrict__ out,
+                                                                  const float* __restrict__ shift, T* __restrict__ out,
                                                                   int B, int H, int W, int Dq, int relu) {
     extern __shared__ __align__(128) unsigned char vsm[];
     __shared__ __align__(8) uint64_t bars[2];
@@ -106,12 +108,12 @@ __global__ void __launch_bounds__(kVcThreads) volume_conv0_kernel(const float* _
             for (int h = 0; h < 2; ++h) {
                 const int ci = 4 * (2 * warp + h) + e;
                 const bool right = ci >= kVcC;
-                const float* plane = (right ? R : L) + ((size_t)b * kVcC + (right ? ci - kVcC : ci)) * HW + (size_t)yp * W;
+                const T* plane = (right ? R : L) + ((size_t)b * kVcC + (right ? ci - kVcC : ci)) * HW + (size_t)yp * W;
                 const int sh = right ? dp : 0;
 #pragma unroll
                 for (int ug = 0; ug < kVcSlabGroups; ++ug) {
                     const int xp = x0 + 8 * ug + r - 1;
-                    v[h][ug] = (xp >= dp && xp < W && xp >= 0) ? __ldg(plane + xp - sh) : 0.f;
+                    v[h][ug] = (xp >= dp && xp < W && xp >= 0) ? ld_f32(plane + xp - sh) : 0.f;
                 }
             }
 #pragma unroll
@@ -168,14 +170,14 @@ __global__ void __launch_bounds__(kVcThreads) volume_conv0_kernel(const float* _
         asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
         const int x = x0 + 32 * warp + lane;
         if (x < W) {
-            float* o = out + (((size_t)b * kVcN) * Dq + d) * HW + (size_t)y * W + x;
+            T* o = out + (((size_t)b * kVcN) * Dq + d) * HW + (size_t)y * W + x;
             const size_t cstride = (size_t)Dq * HW;
 #pragma unroll
             for (int n = 0; n < kVcN; ++n) {
                 float val = __uint_as_float(v[n]);
                 if (scale != nullptr) val = fmaf(val, __ldg(scale + n), __ldg(shift + n));
                 if (relu) val = fmaxf(val, 0.f);
-                o[(size_t)n * cstride] = val;
+                st_from_f32(o + (size_t)n * cstride, val);
             }
         }
     }
@@ -186,12 +188,18 @@ __global__ void __launch_bounds__(kVcThreads) volume_conv0_kernel(const float* _
 
 // Packs a Conv3d weight [32][64][3][3][3] into the per-tap core-matrix order the kernel copies into shared memory:
 // wpacked[tap][j = k/8][kc = (k/4)&1][ng = n/8][r = n%8][e = k%4], rounded to TF32.  grid = 27, 256 threads.
+// DT = AZ_DTYPE_BF16 / AZ_DTYPE_F16 rounds each weight to that dtype first (RNE; what torch.autocast does to the weight
+// of a cuDNN convolution), which TF32 then holds exactly; DT = 0 rounds to TF32 only.
+template <int DT>
 __global__ void __launch_bounds__(256) volume_conv0_pack_kernel(const float* __restrict__ w, float* __restrict__ wpacked) {
     const int tap = blockIdx.x;
     for (int t = threadIdx.x; t < kVcN * kVcK; t += 256) {
         const int e = t & 3, r = (t >> 2) & 7, ng = (t >> 5) & 3, kc = (t >> 7) & 1, j = t >> 8;
         const int n = 8 * ng + r, k = 8 * j + 4 * kc + e;
-        const float v = to_tf32(__ldg(w + ((size_t)n * kVcK + k) * 27 + tap));
+        float v = __ldg(w + ((size_t)n * kVcK + k) * 27 + tap);
+        if (DT == AZ_DTYPE_BF16) v = __bfloat162float(__float2bfloat16_rn(v));
+        if (DT == AZ_DTYPE_F16) v = __half2float(__float2half_rn(v));
+        v = to_tf32(v);
         wpacked[(size_t)tap * kVcN * kVcK + t] = v;
         // second copy of the LEFT half (k < 32) in the N = 96 operand order of volume_conv_v2.cu, after the 27 tap
         // blocks: [kd*3+ky][j][kc][kx][ng][r][e] -- 12 KB per (kd, ky), one bulk copy each
@@ -203,8 +211,29 @@ __global__ void __launch_bounds__(256) volume_conv0_pack_kernel(const float* __r
 }
 
 // volume_conv_v2.cu: shifted-coordinate, feature-stationary form (default when Dq <= 55)
-int volume_conv0_v2_launch(const float* L, const float* R, const float* wpacked, const float* scale, const float* shift,
-                           float* out, int B, int H, int W, int Dq, int relu, cudaStream_t st, bool* done);
+template <typename T>
+int volume_conv0_v2_launch(const T* L, const T* R, const float* wpacked, const float* scale, const float* shift,
+                           T* out, int B, int H, int W, int Dq, int relu, cudaStream_t st, bool* done);
+
+template <typename T>
+int volume_conv0_fwd_launch(const T* L, const T* R, const float* wpacked, const float* scale, const float* shift, T* out,
+                            int64_t B, int64_t H, int64_t W, int64_t Dq, int relu, cudaStream_t st) {
+    if (tuning("AZ_VCONV", 2) == 2) {
+        bool done = false;
+        const int rc = volume_conv0_v2_launch<T>(L, R, wpacked, scale, shift, out, (int)B, (int)H, (int)W, (int)Dq, relu,
+                                                 st, &done);
+        if (rc != 0) return rc;
+        if (done) return 0;
+    }
+    const size_t smem = 2 * (size_t)kVcStage;
+    cudaError_t e = cudaFuncSetAttribute(volume_conv0_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return (int)e;
+    dim3 grid((unsigned)ceil_div(W, kVcM), (unsigned)H, (unsigned)(Dq * B));
+    volume_conv0_kernel<T><<<grid, kVcThreads, smem, st>>>(L, R, wpacked, scale, shift, out, (int)B, (int)H, (int)W, (int)Dq,
+                                                         relu);
+    AZ_LAUNCH_CHECK();
+    return 0;
+}
 
 }  // namespace az
 
@@ -212,30 +241,46 @@ using namespace az;
 
 extern "C" int az_volume_conv0_pack(const float* weight, float* wpacked, void* stream) {
     if (!weight || !wpacked) return AZ_ERR_BAD_ARG;
-    volume_conv0_pack_kernel<<<27, 256, 0, (cudaStream_t)stream>>>(weight, wpacked);
+    volume_conv0_pack_kernel<0><<<27, 256, 0, (cudaStream_t)stream>>>(weight, wpacked);
     AZ_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int az_volume_conv0_pack_16(const float* weight, float* wpacked, int dtype, void* stream) {
+    if (!weight || !wpacked || (dtype != AZ_DTYPE_BF16 && dtype != AZ_DTYPE_F16)) return AZ_ERR_BAD_ARG;
+    if (dtype == AZ_DTYPE_BF16) volume_conv0_pack_kernel<AZ_DTYPE_BF16><<<27, 256, 0, (cudaStream_t)stream>>>(weight, wpacked);
+    else volume_conv0_pack_kernel<AZ_DTYPE_F16><<<27, 256, 0, (cudaStream_t)stream>>>(weight, wpacked);
+    AZ_LAUNCH_CHECK();
+    return 0;
+}
+
+static int volume_conv0_check(const void* L, const void* R, const float* wpacked, const float* scale, const float* shift,
+                              const void* out, int64_t B, int64_t C, int64_t H, int64_t W, int64_t Dq) {
+    if (!L || !R || !wpacked || !out || B <= 0 || H <= 0 || W <= 0 || Dq <= 0) return AZ_ERR_BAD_ARG;
+    if (C != kVcC || (scale == nullptr) != (shift == nullptr)) return AZ_ERR_BAD_ARG;  // PSMNet: 32 + 32 -> 32 channels
+    if (H > 65535 || Dq * B > 65535 || H * W >= (1ll << 31) || !aligned16(wpacked)) return AZ_ERR_BAD_ARG;
     return 0;
 }
 
 extern "C" int az_volume_conv0_fwd(const float* L, const float* R, const float* wpacked, const float* scale,
                                    const float* shift, float* out, int64_t B, int64_t C, int64_t H, int64_t W,
                                    int64_t Dq, int relu, void* stream) {
-    if (!L || !R || !wpacked || !out || B <= 0 || H <= 0 || W <= 0 || Dq <= 0) return AZ_ERR_BAD_ARG;
-    if (C != kVcC || (scale == nullptr) != (shift == nullptr)) return AZ_ERR_BAD_ARG;  // PSMNet: 32 + 32 -> 32 channels
-    if (H > 65535 || Dq * B > 65535 || H * W >= (1ll << 31) || !aligned16(wpacked)) return AZ_ERR_BAD_ARG;
-    if (tuning("AZ_VCONV", 2) == 2) {
-        bool done = false;
-        const int rc = volume_conv0_v2_launch(L, R, wpacked, scale, shift, out, (int)B, (int)H, (int)W, (int)Dq, relu,
-                                              (cudaStream_t)stream, &done);
-        if (rc != 0) return rc;
-        if (done) return 0;
-    }
-    const size_t smem = 2 * (size_t)kVcStage;
-    cudaError_t e = cudaFuncSetAttribute(volume_conv0_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return (int)e;
-    dim3 grid((unsigned)ceil_div(W, kVcM), (unsigned)H, (unsigned)(Dq * B));
-    volume_conv0_kernel<<<grid, kVcThreads, smem, (cudaStream_t)stream>>>(L, R, wpacked, scale, shift, out, (int)B, (int)H,
-                                                                         (int)W, (int)Dq, relu);
-    AZ_LAUNCH_CHECK();
-    return 0;
+    const int rc = volume_conv0_check(L, R, wpacked, scale, shift, out, B, C, H, W, Dq);
+    if (rc != 0) return rc;
+    return volume_conv0_fwd_launch<float>(L, R, wpacked, scale, shift, out, B, H, W, Dq, relu, (cudaStream_t)stream);
+}
+
+extern "C" int az_volume_conv0_fwd_16(const void* L, const void* R, const float* wpacked, const float* scale,
+                                      const float* shift, void* out, int64_t B, int64_t C, int64_t H, int64_t W,
+                                      int64_t Dq, int relu, int dtype, void* stream) {
+    const int rc = volume_conv0_check(L, R, wpacked, scale, shift, out, B, C, H, W, Dq);
+    if (rc != 0) return rc;
+    if (dtype == AZ_DTYPE_BF16)
+        return volume_conv0_fwd_launch<__nv_bfloat16>(static_cast<const __nv_bfloat16*>(L), static_cast<const __nv_bfloat16*>(R),
+                                                      wpacked, scale, shift, static_cast<__nv_bfloat16*>(out), B, H, W, Dq,
+                                                      relu, (cudaStream_t)stream);
+    if (dtype == AZ_DTYPE_F16)
+        return volume_conv0_fwd_launch<__half>(static_cast<const __half*>(L), static_cast<const __half*>(R), wpacked, scale,
+                                               shift, static_cast<__half*>(out), B, H, W, Dq, relu, (cudaStream_t)stream);
+    return AZ_ERR_BAD_ARG;
 }

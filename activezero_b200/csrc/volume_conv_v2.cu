@@ -128,8 +128,10 @@ __device__ __forceinline__ float v2_dot32(const float* __restrict__ wt, int n, c
 }
 
 // Stage three feature rows (y-1, y, y+1) of `src` in the operand layout: cache[ky][chunk kq][row][4 channels], row r
-// holding image column col0 + r (zero outside the image / outside the rows), rounded to TF32.
-__device__ __forceinline__ void v2_stage_rows(float* __restrict__ cache, const float* __restrict__ src, int b, int y, int H,
+// holding image column col0 + r (zero outside the image / outside the rows), rounded to TF32 (16-bit features are
+// widened first, which TF32 holds exactly).
+template <typename T>
+__device__ __forceinline__ void v2_stage_rows(float* __restrict__ cache, const T* __restrict__ src, int b, int y, int H,
                                               int W, int col0, int nrows) {
     const size_t HW = (size_t)H * W;
     for (int it = threadIdx.x; it < 3 * 8 * nrows; it += kV2Threads) {
@@ -137,11 +139,11 @@ __device__ __forceinline__ void v2_stage_rows(float* __restrict__ cache, const f
         const int yp = y + ky - 1, col = col0 + r;
         float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
         if (yp >= 0 && yp < H && col >= 0 && col < W) {
-            const float* p = src + ((size_t)b * kV2C + 4 * kq) * HW + (size_t)yp * W + col;
-            v.x = v2_tf32(__ldg(p));
-            v.y = v2_tf32(__ldg(p + HW));
-            v.z = v2_tf32(__ldg(p + 2 * HW));
-            v.w = v2_tf32(__ldg(p + 3 * HW));
+            const T* p = src + ((size_t)b * kV2C + 4 * kq) * HW + (size_t)yp * W + col;
+            v.x = v2_tf32(ld_f32(p));
+            v.y = v2_tf32(ld_f32(p + HW));
+            v.z = v2_tf32(ld_f32(p + 2 * HW));
+            v.w = v2_tf32(ld_f32(p + 3 * HW));
         }
         reinterpret_cast<float4*>(cache)[(size_t)(ky * 8 + kq) * nrows + r] = v;
     }
@@ -158,10 +160,13 @@ __device__ __forceinline__ void v2_copy_weights_left96(float* ws, const float* _
     for (int k = 0; k < 9; ++k) bulk_g2s(ws + k * 3072, wpacked + (size_t)27 * 2048 + (size_t)k * 3072, 12288u, bar);
 }
 
-__global__ void __launch_bounds__(kV2Threads, 1) volume_conv0_v2_kernel(const float* __restrict__ L, const float* __restrict__ R,
+// T = the features' and the output's element type: float, or bf16 / fp16 (torch.autocast; the epilogue stays fp32 and
+// rounds once at the store)
+template <typename T>
+__global__ void __launch_bounds__(kV2Threads, 1) volume_conv0_v2_kernel(const T* __restrict__ L, const T* __restrict__ R,
                                                                        const float* __restrict__ wpacked,
                                                                        const float* __restrict__ scale,
-                                                                       const float* __restrict__ shift, float* __restrict__ out,
+                                                                       const float* __restrict__ shift, T* __restrict__ out,
                                                                        int B, int H, int W, int Dq, int relu) {
     extern __shared__ __align__(128) unsigned char vsm[];
     __shared__ __align__(8) uint64_t bar_q, bar_w, full[kV2Slots], empty[kV2Slots];
@@ -398,7 +403,7 @@ __global__ void __launch_bounds__(kV2Threads, 1) volume_conv0_v2_kernel(const fl
                     for (int n = 0; n < 32; ++n) v[n] = __float_as_uint(__uint_as_float(v[n]) - __uint_as_float(t[n]));
                 }
             }
-            float* o = out + ((size_t)b * kV2N * Dq + d) * HW + (size_t)y * W;
+            T* o = out + ((size_t)b * kV2N * Dq + d) * HW + (size_t)y * W;
             if (m < kV2MT && x >= 0 && x < W) {
                 const float* cr = Cr + (size_t)d * 32;
                 const bool xr = x == W - 1;  // one row per plane
@@ -409,7 +414,7 @@ __global__ void __launch_bounds__(kV2Threads, 1) volume_conv0_v2_kernel(const fl
                     float val = __uint_as_float(v[n]) + qs[n] - (xr ? c : 0.f);
                     val = fmaf(val, sc.x, sc.y);
                     if (relu) val = fmaxf(val, 0.f);
-                    o[(size_t)n * cstride + x] = val;
+                    st_from_f32(o + (size_t)n * cstride + x, val);
                 }
             }
             // columns x <= d - 3 (shifted column <= -3): every tap is masked -> the epilogue of zero
@@ -419,7 +424,7 @@ __global__ void __launch_bounds__(kV2Threads, 1) volume_conv0_v2_kernel(const fl
                     float val = 0.f;
                     if (scale != nullptr) val = __ldg(shift + n);
                     if (relu) val = fmaxf(val, 0.f);
-                    o[(size_t)n * cstride + m] = val;
+                    st_from_f32(o + (size_t)n * cstride + m, val);
                 }
             }
         }
@@ -429,17 +434,24 @@ __global__ void __launch_bounds__(kV2Threads, 1) volume_conv0_v2_kernel(const fl
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512));
 }
 
-int volume_conv0_v2_launch(const float* L, const float* R, const float* wpacked, const float* scale, const float* shift,
-                           float* out, int B, int H, int W, int Dq, int relu, cudaStream_t st, bool* done) {
+template <typename T>
+int volume_conv0_v2_launch(const T* L, const T* R, const float* wpacked, const float* scale, const float* shift,
+                           T* out, int B, int H, int W, int Dq, int relu, cudaStream_t st, bool* done) {
     *done = false;
     if (Dq > kV2MaxDq || B > 65535 || H > 65535) return 0;
-    cudaError_t e = cudaFuncSetAttribute(volume_conv0_v2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kV2Smem);
+    cudaError_t e = cudaFuncSetAttribute(volume_conv0_v2_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, kV2Smem);
     if (e != cudaSuccess) return (int)e;
     // shifted columns -2 .. W - 1 (plane 0) must be covered
     dim3 grid((unsigned)ceil_div(W + 2, kV2MT), (unsigned)H, (unsigned)B);
-    volume_conv0_v2_kernel<<<grid, kV2Threads, kV2Smem, st>>>(L, R, wpacked, scale, shift, out, B, H, W, Dq, relu);
+    volume_conv0_v2_kernel<T><<<grid, kV2Threads, kV2Smem, st>>>(L, R, wpacked, scale, shift, out, B, H, W, Dq, relu);
     *done = true;
     return (int)cudaGetLastError();
 }
+template int volume_conv0_v2_launch<float>(const float*, const float*, const float*, const float*, const float*, float*, int,
+                                           int, int, int, int, cudaStream_t, bool*);
+template int volume_conv0_v2_launch<__nv_bfloat16>(const __nv_bfloat16*, const __nv_bfloat16*, const float*, const float*,
+                                                   const float*, __nv_bfloat16*, int, int, int, int, int, cudaStream_t, bool*);
+template int volume_conv0_v2_launch<__half>(const __half*, const __half*, const float*, const float*, const float*, __half*,
+                                            int, int, int, int, int, cudaStream_t, bool*);
 
 }  // namespace az

@@ -34,9 +34,12 @@ import torch
 from torch import Tensor
 
 from . import _lib, _volume_conv_library
-from .ops import _cuda_f32, _mask_u8, _ptr, _stream, check_feature_pair, check_reproj_inputs, linspace_table
+from .ops import DTYPE16, _cuda_f32, _mask_u8, _ptr, _stream, check_feature_pair, check_reproj_inputs, linspace_table
+from .ops import concat_volume_backward as concat_volume_backward_into
+from .ops import concat_volume_forward
 
 NS = "az_stereo"
+_FLOAT_DTYPES = (torch.float32, *DTYPE16)
 
 
 def volume_conv(ref: Tensor, tgt: Tensor, weight: Tensor, num_disp: int) -> Tensor:
@@ -50,17 +53,11 @@ def volume_conv(ref: Tensor, tgt: Tensor, weight: Tensor, num_disp: int) -> Tens
 # ---------------------------------------------------------------------------------------------
 @torch.library.custom_op(f"{NS}::concat_volume", mutates_args=(), device_types="cuda")
 def concat_volume(ref: Tensor, tgt: Tensor, num_disp: int, channels_last: bool) -> Tensor:
-    L, R = check_feature_pair(ref, tgt, "az_stereo::concat_volume")
+    # float32 features, or two bfloat16 / two float16 features (the volume has their dtype; ops.build_concat_volume)
+    L, R = check_feature_pair(ref, tgt, "az_stereo::concat_volume", allow16=True)
     if num_disp <= 0:
         raise ValueError("az_stereo::concat_volume: num_disp must be positive")
-    B, C, H, W = L.shape
-    ndhwc = channels_last and C % 4 == 0
-    vol = torch.empty((B, 2 * C, num_disp, H, W), dtype=torch.float32, device=L.device,
-                      memory_format=torch.channels_last_3d if ndhwc else torch.contiguous_format)
-    with torch.cuda.device(L.device):
-        _lib.call("az_concat_volume_fwd_ndhwc" if ndhwc else "az_concat_volume_fwd", _ptr(L), _ptr(R), _ptr(vol),
-                  B, C, H, W, num_disp, _stream(), batch=B)
-    return vol.contiguous(memory_format=torch.channels_last_3d) if channels_last and not ndhwc else vol
+    return concat_volume_forward(L, R, num_disp, channels_last)
 
 
 @concat_volume.register_fake
@@ -72,17 +69,11 @@ def _(ref, tgt, num_disp, channels_last):
 
 @torch.library.custom_op(f"{NS}::concat_volume_backward", mutates_args=(), device_types="cuda")
 def concat_volume_backward(gvol: Tensor, C: int) -> Tuple[Tensor, Tensor]:
-    if gvol.dim() != 5 or gvol.shape[1] != 2 * C or not gvol.is_cuda or gvol.dtype != torch.float32:
-        raise ValueError("az_stereo::concat_volume_backward: gvol must be a CUDA float32 [B,2C,Dq,H,W] tensor")
-    B, _, Dq, H, W = gvol.shape
-    ndhwc = C % 4 == 0 and gvol.is_contiguous(memory_format=torch.channels_last_3d) and not gvol.is_contiguous()
-    g = gvol if ndhwc else _cuda_f32(gvol, "grad_volume")
-    gL = torch.empty((B, C, H, W), dtype=torch.float32, device=g.device)
-    gR = torch.empty_like(gL)
-    with torch.cuda.device(g.device):
-        _lib.call("az_concat_volume_bwd_ndhwc" if ndhwc else "az_concat_volume_bwd", _ptr(g), _ptr(gL), _ptr(gR),
-                  B, C, H, W, Dq, _stream(), batch=B)
-    return gL, gR
+    # gL, gR have gvol's dtype, which autograd makes the volume's, i.e. the features' dtype
+    if gvol.dim() != 5 or gvol.shape[1] != 2 * C or not gvol.is_cuda or gvol.dtype not in _FLOAT_DTYPES:
+        raise ValueError("az_stereo::concat_volume_backward: gvol must be a CUDA float32, bfloat16 or float16 "
+                         "[B,2C,Dq,H,W] tensor")
+    return concat_volume_backward_into(gvol, C)
 
 
 @concat_volume_backward.register_fake

@@ -12,6 +12,7 @@ Layer hyper-parameters follow ``/root/reference/nets/psmnet/psmnet_submodule.py`
 """
 from __future__ import annotations
 
+import contextlib
 import math
 
 import torch
@@ -185,13 +186,14 @@ class PSMNetBase(nn.Module):
         return self
 
     def _first_conv_implicit(self, ref_feat, tgt_feat):
-        """dres0[0] (Conv3d 64->32 + BatchNorm3d, eval statistics) + dres0[1] (ReLU) on the IMPLICIT volume."""
+        """dres0[0] (Conv3d 64->32 + BatchNorm3d, eval statistics) + dres0[1] (ReLU) on the IMPLICIT volume.  16-bit
+        features give a 16-bit output, with the weight rounded to their dtype as autocast rounds cuDNN's."""
         from ... import ops
 
         conv, bn = self.dres0[0][0], self.dres0[0][1]
-        key = (conv.weight.data_ptr(), conv.weight._version, str(conv.weight.device))
+        key = (conv.weight.data_ptr(), conv.weight._version, str(conv.weight.device), ref_feat.dtype)
         if self._vc_cache is None or self._vc_cache[0] != key:
-            self._vc_cache = (key, ops.pack_volume_conv_weight(conv.weight))
+            self._vc_cache = (key, ops.pack_volume_conv_weight(conv.weight, dtype=ref_feat.dtype))
         scale = bn.weight.detach() * torch.rsqrt(bn.running_var + bn.eps)
         shift = bn.bias.detach() - bn.running_mean * scale
         return ops.volume_conv0(ref_feat, tgt_feat, self._vc_cache[1], self.maxdisp // 4, scale, shift, relu=True)
@@ -223,12 +225,26 @@ class PSMNetBase(nn.Module):
         up = F.interpolate(cost, (self.maxdisp, 4 * H, 4 * W), mode="trilinear", align_corners=False)
         return ops.soft_argmin(torch.squeeze(up, 1))
 
+    @staticmethod
+    def _native16(ref_feat, tgt_feat):
+        """A context in which the volume operators take the features as they are: under torch.autocast with features of
+        the autocast dtype (bf16 / fp16; the feature extractor ends in a Conv2d), autocast is switched off around
+        the call, so the volume (or the first convolution's output) is produced in 16 bits directly instead of in
+        fp32 and cast down by the next convolution.  The concat volume and its gradients are bit-identical to that
+        dataflow's (DESIGN.md §4.11).  Otherwise a no-op."""
+        if torch.is_autocast_enabled("cuda"):
+            dt = torch.get_autocast_dtype("cuda")
+            if dt in (torch.bfloat16, torch.float16) and ref_feat.dtype == dt and tgt_feat.dtype == dt:
+                return torch.autocast("cuda", enabled=False)
+        return contextlib.nullcontext()
+
     def _forward_features(self, ref_feat, tgt_feat):
         from ... import ops
 
         H, W = ref_feat.shape[-2:]
         if self.fuse_volume_conv and not self.training and not torch.is_grad_enabled() and ref_feat.shape[1] == 32:
-            first = self._first_conv_implicit(ref_feat, tgt_feat)
+            with self._native16(ref_feat, tgt_feat):
+                first = self._first_conv_implicit(ref_feat, tgt_feat)
             if self.volume_channels_last:
                 first = first.contiguous(memory_format=torch.channels_last_3d)
             _, _, cost3 = self._aggregate(None, first)
@@ -241,10 +257,11 @@ class PSMNetBase(nn.Module):
                 first = first.contiguous(memory_format=torch.channels_last_3d)
             cost1, cost2, cost3 = self._aggregate(None, first)
         else:
-            if self.volume_channels_last:
-                cost = ops.build_concat_volume(ref_feat, tgt_feat, self.maxdisp // 4, channels_last=True)
-            else:
-                cost = ops.build_concat_volume(ref_feat, tgt_feat, self.maxdisp // 4)  # replaces psmnet.py:151-165
+            with self._native16(ref_feat, tgt_feat):
+                if self.volume_channels_last:
+                    cost = ops.build_concat_volume(ref_feat, tgt_feat, self.maxdisp // 4, channels_last=True)
+                else:
+                    cost = ops.build_concat_volume(ref_feat, tgt_feat, self.maxdisp // 4)  # replaces psmnet.py:151-165
             cost1, cost2, cost3 = self._aggregate(cost)
         pred3 = self._disparity_head(cost3, H, W)
         if self.training:

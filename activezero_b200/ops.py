@@ -33,20 +33,27 @@ def _stream():
     return ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
-def _cuda_f32(t: torch.Tensor, name: str) -> torch.Tensor:
+# the 16-bit dtypes of torch.autocast -> the C ABI's dtype codes (AZ_DTYPE_BF16, AZ_DTYPE_F16 in include/az_stereo.h)
+DTYPE16 = {torch.bfloat16: 1, torch.float16: 2}
+
+
+def _cuda_f32(t: torch.Tensor, name: str, allow16: bool = False) -> torch.Tensor:
     if not isinstance(t, torch.Tensor) or not t.is_cuda:
         raise ValueError(f"{name}: expected a CUDA tensor (activezero_b200 has no CPU path)")
-    if t.dtype != torch.float32:
-        raise ValueError(f"{name}: expected float32, got {t.dtype}")
+    if t.dtype != torch.float32 and not (allow16 and t.dtype in DTYPE16):
+        raise ValueError(f"{name}: expected float32{', bfloat16 or float16' if allow16 else ''}, got {t.dtype}")
     return t if t.is_contiguous() else t.contiguous()
 
 
-def check_feature_pair(ref_feat, tgt_feat, what: str):
-    """Shared by ops and library_ops: both features CUDA float32 [B,C,H,W] of the SAME shape and device."""
-    L = _cuda_f32(ref_feat, "ref_feat")
-    R = _cuda_f32(tgt_feat, "tgt_feat")
+def check_feature_pair(ref_feat, tgt_feat, what: str, allow16: bool = False):
+    """Shared by ops and library_ops: both features CUDA float32 [B,C,H,W] of the SAME shape and device
+    (``allow16``: or both bfloat16, or both float16)."""
+    L = _cuda_f32(ref_feat, "ref_feat", allow16)
+    R = _cuda_f32(tgt_feat, "tgt_feat", allow16)
     if L.dim() != 4 or L.shape != R.shape:
         raise ValueError(f"{what}: features must both be [B,C,H,W] with identical shapes, got {tuple(L.shape)} and {tuple(R.shape)}")
+    if L.dtype != R.dtype:
+        raise ValueError(f"{what}: features of different dtypes ({L.dtype} and {R.dtype})")
     if L.device != R.device:
         raise ValueError(f"{what}: features live on different devices")
     return L, R
@@ -84,73 +91,111 @@ def linspace_table(n: int, device: torch.device) -> torch.Tensor:
 # ----------------------------------------------------------------------------
 # a1/a2 concat volume
 # ----------------------------------------------------------------------------
+def concat_volume_forward(L, R, num_disp: int, channels_last: bool):
+    """Enqueues the concat volume of validated features (float32, or both bfloat16 / both float16: the volume has
+    the features' dtype).  Shared by ConcatVolumeFn and library_ops."""
+    B, C, H, W = L.shape
+    dt = DTYPE16.get(L.dtype)
+    # the kernels write channels_last_3d directly when a position's 2C values are whole 16-byte vectors
+    ndhwc = bool(channels_last) and C % (4 if dt is None else 8) == 0
+    vol = torch.empty((B, 2 * C, num_disp, H, W), dtype=L.dtype, device=L.device,
+                      memory_format=torch.channels_last_3d if ndhwc else torch.contiguous_format)
+    with torch.cuda.device(L.device):
+        if dt is None:
+            _lib.call("az_concat_volume_fwd_ndhwc" if ndhwc else "az_concat_volume_fwd", _ptr(L), _ptr(R), _ptr(vol),
+                      B, C, H, W, num_disp, _stream(), batch=B)
+        else:
+            _lib.call("az_concat_volume_fwd_16", _ptr(L), _ptr(R), _ptr(vol), B, C, H, W, num_disp, 1 if ndhwc else 0,
+                      _stream(), batch=B)
+    if channels_last and not ndhwc:  # C not a multiple of 4 (8 for 16 bits): torch's layout conversion (on the device)
+        vol = vol.contiguous(memory_format=torch.channels_last_3d)
+    return vol
+
+
+def concat_volume_backward(gvol, C: int, need_l: bool = True, need_r: bool = True):
+    """gL, gR (each None when not needed) of the concat volume for a CUDA gradient [B,2C,Dq,H,W] of dtype float32,
+    bfloat16 or float16; the gradients have gvol's dtype.  Shared by ConcatVolumeFn and library_ops."""
+    dt = DTYPE16.get(gvol.dtype)
+    B, _, Dq, H, W = gvol.shape
+    # a gradient that arrives in channels_last_3d (what cuDNN returns for a channels_last_3d input) is consumed
+    # in place; anything else is made NCDHW-contiguous
+    ndhwc = C % (4 if dt is None else 8) == 0 and Dq * H * W > 1 \
+        and gvol.is_contiguous(memory_format=torch.channels_last_3d) and not gvol.is_contiguous()
+    g = gvol if ndhwc else _cuda_f32(gvol, "grad_volume", allow16=True)
+    gL = torch.empty((B, C, H, W), dtype=g.dtype, device=g.device) if need_l else None
+    gR = torch.empty((B, C, H, W), dtype=g.dtype, device=g.device) if need_r else None
+    with torch.cuda.device(g.device):
+        if dt is None:
+            _lib.call("az_concat_volume_bwd_ndhwc" if ndhwc else "az_concat_volume_bwd", _ptr(g), _ptr(gL), _ptr(gR),
+                      B, C, H, W, Dq, _stream(), batch=B)
+        else:
+            _lib.call("az_concat_volume_bwd_16", _ptr(g), _ptr(gL), _ptr(gR), B, C, H, W, Dq, dt, 1 if ndhwc else 0,
+                      _stream(), batch=B)
+    return gL, gR
+
+
 class ConcatVolumeFn(torch.autograd.Function):
-    """nets/psmnet/psmnet.py:151-165 and its autograd."""
+    """nets/psmnet/psmnet.py:151-165 and its autograd.  Outside torch.autocast, two bfloat16 (or two float16) features
+    give a volume of their dtype and gradients of their dtype (RNE of the fp32 sums, DESIGN.md §4.11); inside autocast the
+    inputs are cast to float32 as before."""
 
     @staticmethod
     @_fwd32
     def forward(ctx, ref_feat, tgt_feat, num_disp: int, channels_last: bool = False):
-        L, R = check_feature_pair(ref_feat, tgt_feat, "concat volume")
+        L, R = check_feature_pair(ref_feat, tgt_feat, "concat volume", allow16=True)
         if int(num_disp) <= 0:
             raise ValueError("concat volume: num_disp must be positive")
-        B, C, H, W = L.shape
-        ndhwc = bool(channels_last) and C % 4 == 0
-        vol = torch.empty((B, 2 * C, int(num_disp), H, W), dtype=torch.float32, device=L.device,
-                          memory_format=torch.channels_last_3d if ndhwc else torch.contiguous_format)
-        with torch.cuda.device(L.device):
-            _lib.call("az_concat_volume_fwd_ndhwc" if ndhwc else "az_concat_volume_fwd", _ptr(L), _ptr(R), _ptr(vol),
-                      B, C, H, W, int(num_disp), _stream(), batch=B)
-        ctx.dims = (B, C, H, W, int(num_disp))
-        if channels_last and not ndhwc:  # C not a multiple of 4: torch's layout conversion (still on the device)
-            vol = vol.contiguous(memory_format=torch.channels_last_3d)
-        return vol
+        ctx.dims = (L.shape[1], int(num_disp), L.dtype)
+        return concat_volume_forward(L, R, int(num_disp), channels_last)
 
     @staticmethod
     @once_differentiable
     @_bwd
     def backward(ctx, gvol):
-        B, C, H, W, Dq = ctx.dims
-        if not isinstance(gvol, torch.Tensor) or not gvol.is_cuda or gvol.dtype != torch.float32:
-            raise ValueError("grad_volume: expected a float32 CUDA tensor")
-        # a gradient that arrives in channels_last_3d (what cuDNN returns for a channels_last_3d input) is consumed
-        # in place; anything else is made NCDHW-contiguous
-        ndhwc = C % 4 == 0 and Dq * H * W > 1 and gvol.is_contiguous(memory_format=torch.channels_last_3d) \
-            and not gvol.is_contiguous()
-        g = gvol if ndhwc else _cuda_f32(gvol, "grad_volume")
-        gL = torch.empty((B, C, H, W), dtype=torch.float32, device=g.device) if ctx.needs_input_grad[0] else None
-        gR = torch.empty((B, C, H, W), dtype=torch.float32, device=g.device) if ctx.needs_input_grad[1] else None
-        with torch.cuda.device(g.device):
-            _lib.call("az_concat_volume_bwd_ndhwc" if ndhwc else "az_concat_volume_bwd", _ptr(g), _ptr(gL), _ptr(gR),
-                      B, C, H, W, Dq, _stream(), batch=B)
+        C, Dq, dtype = ctx.dims
+        if not isinstance(gvol, torch.Tensor) or not gvol.is_cuda or gvol.dtype != dtype:
+            raise ValueError(f"grad_volume: expected a {dtype} CUDA tensor")
+        gL, gR = concat_volume_backward(gvol, C, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
         return gL, gR, None, None
 
 
 def build_concat_volume(ref_feat, tgt_feat, num_disp: int, channels_last: bool = False):
     """[B,C,H,W] x2 -> [B,2C,num_disp,H,W] (replaces psmnet.py:151-165).  ``channels_last=True`` returns the
     same tensor in ``torch.channels_last_3d`` memory format (SURVEY.md §8f rank 2): the values and the shape are
-    unchanged, only the strides differ, and cuDNN's 3-D convolutions consume it without a layout pass."""
+    unchanged, only the strides differ, and cuDNN's 3-D convolutions consume it without a layout pass.
+    float32 features give a float32 volume; outside torch.autocast, two bfloat16 or two float16 features give a volume
+    of their dtype (the same values: a copy), and the backward returns gradients of their dtype."""
     return ConcatVolumeFn.apply(ref_feat, tgt_feat, num_disp, channels_last)
 
 
 # ----------------------------------------------------------------------------
 # §8f rank 2: dres0's first convolution with the concat volume left implicit (tcgen05 TF32 implicit GEMM)
 # ----------------------------------------------------------------------------
-def pack_volume_conv_weight(weight: torch.Tensor) -> torch.Tensor:
+def pack_volume_conv_weight(weight: torch.Tensor, dtype: torch.dtype = torch.float32) -> torch.Tensor:
     """Conv3d weight [32,64,3,3,3] (dres0[0][0].weight, psmnet.py:85-90) -> the per-tap core-matrix order of the
-    tensor-core kernel, rounded to TF32; do this once per weight tensor."""
+    tensor-core kernel, rounded to TF32; do this once per weight tensor.  ``dtype`` = the dtype of the features it
+    will be used with: bfloat16 / float16 round each weight to that dtype first (RNE), as torch.autocast rounds the
+    weight of a cuDNN convolution."""
     w = _cuda_f32(weight.detach(), "weight")
     if tuple(w.shape) != (32, 64, 3, 3, 3):
         raise ValueError(f"volume conv: expected a [32,64,3,3,3] Conv3d weight, got {tuple(w.shape)}")
+    if dtype != torch.float32 and dtype not in DTYPE16:
+        raise ValueError(f"volume conv: dtype must be float32, bfloat16 or float16, got {dtype}")
     packed = torch.empty((27 * 3072,), dtype=torch.float32, device=w.device)  # AZ_VOLUME_CONV0_PACKED_FLOATS
     with torch.cuda.device(w.device):
-        _lib.call("az_volume_conv0_pack", _ptr(w), _ptr(packed), _stream())
+        if dtype == torch.float32:
+            _lib.call("az_volume_conv0_pack", _ptr(w), _ptr(packed), _stream())
+        else:
+            _lib.call("az_volume_conv0_pack_16", _ptr(w), _ptr(packed), DTYPE16[dtype], _stream())
     return packed
 
 
 def volume_conv0(ref_feat, tgt_feat, wpacked, num_disp: int, scale=None, shift=None, relu: bool = False):
     """conv3d(concat_volume(ref, tgt, num_disp), weight, padding=1) without the volume (forward only; TF32 operands,
-    fp32 accumulation): [B,32,H,W] x2 -> [B,32,num_disp,H,W].  ``scale``/``shift`` [32] fold an eval-mode BatchNorm."""
-    L, R = check_feature_pair(ref_feat.detach(), tgt_feat.detach(), "volume conv")
+    fp32 accumulation): [B,32,H,W] x2 -> [B,32,num_disp,H,W].  ``scale``/``shift`` [32] fold an eval-mode BatchNorm.
+    Two bfloat16 (or float16) features give an output of their dtype, rounded once after the fold and the ReLU;
+    ``wpacked`` should then come from ``pack_volume_conv_weight(weight, dtype=<that dtype>)``."""
+    L, R = check_feature_pair(ref_feat.detach(), tgt_feat.detach(), "volume conv", allow16=True)
     B, C, H, W = L.shape
     if C != 32:
         raise ValueError("volume conv: PSMNet's 32 feature channels expected")
@@ -163,10 +208,15 @@ def volume_conv0(ref_feat, tgt_feat, wpacked, num_disp: int, scale=None, shift=N
     sh = _cuda_f32(shift.detach().reshape(-1), "shift") if shift is not None else None
     if sc is not None and (sc.numel() != 32 or sh.numel() != 32):
         raise ValueError("volume conv: scale / shift must hold 32 values")
-    out = torch.empty((B, 32, int(num_disp), H, W), dtype=torch.float32, device=L.device)
+    out = torch.empty((B, 32, int(num_disp), H, W), dtype=L.dtype, device=L.device)
+    dt = DTYPE16.get(L.dtype)
     with torch.cuda.device(L.device):
-        _lib.call("az_volume_conv0_fwd", _ptr(L), _ptr(R), _ptr(wp), _ptr(sc), _ptr(sh), _ptr(out), B, C, H, W, int(num_disp),
-                  1 if relu else 0, _stream(), batch=B)
+        if dt is None:
+            _lib.call("az_volume_conv0_fwd", _ptr(L), _ptr(R), _ptr(wp), _ptr(sc), _ptr(sh), _ptr(out), B, C, H, W,
+                      int(num_disp), 1 if relu else 0, _stream(), batch=B)
+        else:
+            _lib.call("az_volume_conv0_fwd_16", _ptr(L), _ptr(R), _ptr(wp), _ptr(sc), _ptr(sh), _ptr(out), B, C, H, W,
+                      int(num_disp), 1 if relu else 0, dt, _stream(), batch=B)
     return out
 
 

@@ -7,9 +7,12 @@ evaluator's shape (test.py:137-146 pads 540x960 to 544x960, batch 1, maxdisp 192
   (c) (b) with the trilinear upsample fused into the soft-argmin.
 The 2-D/3-D convolutions are identical cuDNN calls in all three; the difference is the hot path.
 
-    python benchmarks/psmnet_inference.py [--batch 1] [--iters 10]
+    python benchmarks/psmnet_inference.py [--batch 1] [--iters 10] [--autocast bf16|fp16]
+
+--autocast runs every arm under torch.autocast with that dtype (the 16-bit volume of DESIGN.md §4.9).
 """
 import argparse
+import contextlib
 import json
 import os
 import sys
@@ -62,13 +65,17 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--batch", type=int, default=1)
     ap.add_argument("--iters", type=int, default=10)
+    ap.add_argument("--autocast", choices=("bf16", "fp16"), default=None,
+                    help="run every arm under torch.autocast with this dtype")
     args = ap.parse_args()
+    amp = contextlib.nullcontext() if args.autocast is None else \
+        torch.autocast("cuda", dtype=torch.bfloat16 if args.autocast == "bf16" else torch.float16)
     torch.manual_seed(1)
     net = PSMNet(maxdisp=192).cuda().eval()
     x = torch.rand(args.batch, 3, 544, 960, device="cuda")
     y = torch.rand(args.batch, 3, 544, 960, device="cuda")
     res = {}
-    with torch.no_grad():
+    with torch.no_grad(), amp:
         res["az_ops_ms"] = timed(lambda: net(x, y), args.iters)
         net.fuse_upsample = True
         res["az_ops_fused_upsample_ms"] = timed(lambda: net(x, y), args.iters)
@@ -101,7 +108,7 @@ def main():
         vol = ops.build_concat_volume(fl, fr, 48)
         res["convs_only_ms"] = timed(lambda: (net.feature_extraction(x), net.feature_extraction(y), net._aggregate(vol)),
                                      args.iters)
-    res.update(batch=args.batch, shape="544x960", maxdisp=192,
+    res.update(batch=args.batch, shape="544x960", maxdisp=192, autocast=args.autocast,
                hot_path_ms={k.replace("_ms", ""): res[k] - res["convs_only_ms"] for k in
                             ("stock_torch_ops_ms", "az_ops_ms", "az_ops_fused_upsample_ms")})
     print(json.dumps(res))

@@ -17,6 +17,7 @@ step once with this repository's CUDA operators and once with the oracle's torch
 from __future__ import annotations
 
 import argparse
+import contextlib
 import json
 import os
 import sys
@@ -115,7 +116,14 @@ def main():
     ap.add_argument("--fuse-volume-conv", action="store_true",
                     help="dres0's first Conv3d on the implicit volume in training too (PSMNet.fuse_volume_conv_train)")
     ap.add_argument("--profile", action="store_true", help="after the timed region: kernel-time shares via torch.profiler")
+    ap.add_argument("--autocast", choices=("bf16", "fp16"), default=None,
+                    help="forward passes under torch.autocast with this dtype (timing only: no GradScaler for fp16)")
     args = ap.parse_args()
+    amp_dtype = {"bf16": torch.bfloat16, "fp16": torch.float16}.get(args.autocast)
+
+    def amp():
+        return torch.autocast("cuda", dtype=amp_dtype) if amp_dtype is not None else contextlib.nullcontext()
+
 
     rank, world, local = dist_util.env_rank_world()
     torch.cuda.set_device(local)
@@ -135,12 +143,14 @@ def main():
     batch = make_batch(args.batch, args.height, args.width, dev, 100 + rank, T=args.frames)
 
     def one_iteration():
-        loss, vals = sim_step_loss(model, batch, api)
+        with amp():
+            loss, vals = sim_step_loss(model, batch, api)
         opt.zero_grad()
         loss.backward()
         opt.step()
         if not args.no_real:
-            loss_r, _ = real_step_loss(model, batch, api)
+            with amp():
+                loss_r, _ = real_step_loss(model, batch, api)
             opt.zero_grad()
             loss_r.backward()
             opt.step()
@@ -194,7 +204,7 @@ def main():
             "config": {"workload": f"config{'3' if args.no_real else '4'}: PSMNet_3 train step {args.height}x{args.width}, "
                                    f"D={MAX_DISP}, batch {args.batch}/GPU, patch reproj ps={PATCH}, T={args.frames}",
                        "ddp": world > 1, "fuse_upsample": args.fuse_upsample, "fuse_volume_conv": args.fuse_volume_conv,
-                       "channels_last_3d": args.channels_last_3d},
+                       "channels_last_3d": args.channels_last_3d, "autocast": args.autocast},
             "device_time_shares_rank0": shares,
             "final_loss": float(last)}), flush=True)
     if world > 1:

@@ -52,6 +52,23 @@ int az_concat_volume_fwd_ndhwc(const float* L, const float* R, float* vol,
 int az_concat_volume_bwd_ndhwc(const float* gvol, float* gL, float* gR,
                                int64_t B, int64_t C, int64_t H, int64_t W, int64_t Dq, void* stream);
 
+/* The same volume and gradient with 16-bit features (what torch.autocast's convolutions consume).  Every pointer is
+ * a device pointer to bf16 or fp16 elements; L, R, gL, gR, vol, gvol all have the features' dtype.
+ * Forward: vol is the formula of az_concat_volume_fwd applied to the 2-byte elements (a copy: exact, and the same
+ *   for both dtypes, so it takes no dtype code).
+ * Backward: gL / gR are the sums of az_concat_volume_bwd taken in fp32 over the upcast elements of gvol, in
+ *   ascending i, then rounded ONCE to the dtype, to nearest even:  gL = RNE16(sum_i float(gvol[..,i,..])).
+ *   This equals az_concat_volume_bwd on gvol.float() followed by .to(dtype), bit for bit.  gL / gR may each be NULL.
+ * channels_last != 0: vol / gvol are in torch.channels_last_3d memory order [B][Dq][H][W][2C]; C must then be a
+ *   multiple of 8 and vol / gvol 16-byte aligned (else AZ_ERR_BAD_ARG).  channels_last == 0: NCDHW, any C. */
+#define AZ_DTYPE_BF16 1
+#define AZ_DTYPE_F16 2
+int az_concat_volume_fwd_16(const void* L, const void* R, void* vol,
+                            int64_t B, int64_t C, int64_t H, int64_t W, int64_t Dq, int channels_last, void* stream);
+int az_concat_volume_bwd_16(const void* gvol, void* gL, void* gR,
+                            int64_t B, int64_t C, int64_t H, int64_t W, int64_t Dq, int dtype, int channels_last,
+                            void* stream);
+
 /* ---- SURVEY.md §8f rank 2, implicit clause: the first 3-D convolution of the aggregation with the volume left
  *      implicit -- nets/psmnet/psmnet.py:151-168 (volume + dres0[0] = Conv3d(64,32,3,1,1,bias=False)), psmnet_submodule.py:44-56.
  * out[b,co,d,y,x] = sum_{ci,kd,ky,kx} weight[co,ci,kd,ky,kx] * vol[b,ci,d+kd-1,y+ky-1,x+kx-1] (zero padding) with vol
@@ -63,6 +80,16 @@ int az_concat_volume_bwd_ndhwc(const float* gvol, float* gL, float* gR,
 int az_volume_conv0_pack(const float* weight, float* wpacked, void* stream);
 int az_volume_conv0_fwd(const float* L, const float* R, const float* wpacked, const float* scale, const float* shift,
                         float* out, int64_t B, int64_t C, int64_t H, int64_t W, int64_t Dq, int relu, void* stream);
+/* The same convolution with 16-bit features and output (dtype AZ_DTYPE_BF16 or AZ_DTYPE_F16), as torch.autocast runs
+ * it: L, R: [B,32,H,W] and out: [B,32,Dq,H,W] of that dtype.  az_volume_conv0_pack_16 rounds each weight to the dtype
+ * (RNE) before the TF32 packing -- what autocast does to cuDNN's weight; use its wpacked with the same dtype.  The
+ * features are converted to fp32 at staging, which TF32 represents exactly, so the MMAs stay TF32 with fp32
+ * accumulation; scale / shift (float[32] or both NULL) and the ReLU are applied in fp32, and each output is rounded
+ * ONCE, to nearest even, at the store:  out = RNE16(relu(conv * scale + shift)). */
+int az_volume_conv0_pack_16(const float* weight, float* wpacked, int dtype, void* stream);
+int az_volume_conv0_fwd_16(const void* L, const void* R, const float* wpacked, const float* scale, const float* shift,
+                           void* out, int64_t B, int64_t C, int64_t H, int64_t W, int64_t Dq, int relu, int dtype,
+                           void* stream);
 /* Backward of the raw convolution above (no scale/shift, no ReLU), without the volume or its gradient.  With
  * gout = dLoss/d out [B,32,Dq,H,W], Wl = weight[:, :32], Wr = weight[:, 32:] and, for each tap (kd,kx),
  * lo = max(0,1-kd), hi = min(Dq-1,Dq-kd):
