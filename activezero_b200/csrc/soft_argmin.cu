@@ -10,6 +10,8 @@
 // max does not move), tree-summed chunk, running sums kept in double so the result stays well
 // inside the 1e-4 px gate for flat distributions.  The forward also emits the log-sum-exp so
 // the backward is a single read-modify-write pass with no second reduction.
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace az {
@@ -31,9 +33,87 @@ template <> struct Vec<1> {
     static __device__ __forceinline__ float pack(const float* f) { return f[0]; }
 };
 
-// One thread owns V adjacent pixels.  n_vec = B*H*W/V work items; plane = H*W (floats).
+// ---- 16-bit logits (bf16 / fp16): widened exactly after the load, gradients rounded once (RNE) at the store -------
+template <typename T> struct Bits16;
+template <> struct Bits16<__nv_bfloat16> {
+    static __device__ __forceinline__ float widen(unsigned u) { return __uint_as_float(u << 16); }  // u: low 16 bits
+    static __device__ __forceinline__ unsigned narrow(float f) { return __bfloat16_as_ushort(__float2bfloat16_rn(f)); }
+};
+template <> struct Bits16<__half> {
+    static __device__ __forceinline__ float widen(unsigned u) { return __half2float(__ushort_as_half((unsigned short)u)); }
+    static __device__ __forceinline__ unsigned narrow(float f) { return __half_as_ushort(__float2half_rn(f)); }
+};
+
 template <int V>
-__global__ void __launch_bounds__(kSAThreads) soft_argmin_fwd_kernel(const float* __restrict__ cost,
+__device__ __forceinline__ void st_vec(float* p, const float* f) {
+    st_stream(reinterpret_cast<typename Vec<V>::T*>(p), Vec<V>::pack(f));
+}
+template <int V, typename T>
+__device__ __forceinline__ void st_vec(T* p, const float* f) {  // V = 4 / 8: p 8- / 16-byte aligned
+    unsigned short* q = reinterpret_cast<unsigned short*>(p);
+    if constexpr (V == 8) {
+        unsigned w[4];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) w[i] = Bits16<T>::narrow(f[2 * i]) | (Bits16<T>::narrow(f[2 * i + 1]) << 16);
+        __stcs(reinterpret_cast<uint4*>(q), make_uint4(w[0], w[1], w[2], w[3]));
+    } else if (V == 4) {
+        __stcs(reinterpret_cast<uint2*>(q), make_uint2(Bits16<T>::narrow(f[0]) | (Bits16<T>::narrow(f[1]) << 16),
+                                                       Bits16<T>::narrow(f[2]) | (Bits16<T>::narrow(f[3]) << 16)));
+    } else {
+#pragma unroll
+        for (int j = 0; j < V; ++j) __stcs(q + j, (unsigned short)Bits16<T>::narrow(f[j]));
+    }
+}
+// V adjacent logits as loaded (raw), widened to fp32 where they are used: a 16-bit pass keeps its planes in flight as
+// 16-bit words (half the registers of widened values).  Used where the pointer is aligned for the V-wide access.
+template <typename T, int V> struct Lanes {
+    using R = typename std::conditional<V == 8, uint4, typename std::conditional<V == 4, uint2, unsigned short>::type>::type;
+    static __device__ __forceinline__ R ld(const T* p) { return __ldcs(reinterpret_cast<const R*>(p)); }
+    static __device__ __forceinline__ void widen(const R& r, float* f) {
+        if constexpr (V == 8) {
+            const unsigned w[4] = {r.x, r.y, r.z, r.w};
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                f[2 * i] = Bits16<T>::widen(w[i] & 0xffffu);
+                f[2 * i + 1] = Bits16<T>::widen(w[i] >> 16);
+            }
+        } else if constexpr (V == 4) {
+            f[0] = Bits16<T>::widen(r.x & 0xffffu);
+            f[1] = Bits16<T>::widen(r.x >> 16);
+            f[2] = Bits16<T>::widen(r.y & 0xffffu);
+            f[3] = Bits16<T>::widen(r.y >> 16);
+        } else {
+            f[0] = Bits16<T>::widen(r);
+        }
+    }
+};
+template <int V> struct Lanes<float, V> {
+    using R = typename Vec<V>::T;
+    static __device__ __forceinline__ R ld(const float* p) { return ld_stream(reinterpret_cast<const R*>(p)); }
+    static __device__ __forceinline__ void widen(const R& r, float* f) { Vec<V>::unpack(r, f); }
+};
+// Four logits as raw words for the packed forward: ALIGNED = one 8-byte access, else four 2-byte ones (same bits).
+template <bool ALIGNED>
+__device__ __forceinline__ float4 ld_raw4(const float* p) { return ld_stream(reinterpret_cast<const float4*>(p)); }
+template <bool ALIGNED, typename T>
+__device__ __forceinline__ uint2 ld_raw4(const T* p) {
+    if (ALIGNED) return __ldcs(reinterpret_cast<const uint2*>(p));
+    const unsigned short* q = reinterpret_cast<const unsigned short*>(p);
+    return make_uint2(__ldcs(q) | ((unsigned)__ldcs(q + 1) << 16), __ldcs(q + 2) | ((unsigned)__ldcs(q + 3) << 16));
+}
+// four -inf logits (planes past D) as raw words
+template <typename T> __device__ __forceinline__ typename Lanes<T, 4>::R neg_inf4();
+template <> __device__ __forceinline__ float4 neg_inf4<float>() { return make_float4(-INFINITY, -INFINITY, -INFINITY, -INFINITY); }
+template <> __device__ __forceinline__ uint2 neg_inf4<__nv_bfloat16>() { return make_uint2(0xff80ff80u, 0xff80ff80u); }
+template <> __device__ __forceinline__ uint2 neg_inf4<__half>() { return make_uint2(0xfc00fc00u, 0xfc00fc00u); }
+// Chunks of 8 planes loaded per pass by a thread of V pixels.  A 16-bit thread with 4 pixels loads two (16 planes x 8 B),
+// one with 8 pixels one (8 planes x 16 B): either way its bytes per pass match the fp32 kernel's 8 planes x 16 B (what
+// reaches the read-only ceiling, DESIGN.md §4.3).  The arithmetic is unchanged.
+template <typename T, int V> constexpr int kFlight = (sizeof(T) == 4 || V == 8) ? 1 : 2;
+
+// One thread owns V adjacent pixels.  n_vec = B*H*W/V work items; plane = H*W (floats).
+template <typename T, int V>
+__global__ void __launch_bounds__(kSAThreads) soft_argmin_fwd_kernel(const T* __restrict__ cost,
                                                                     float* __restrict__ disp,
                                                                     float* __restrict__ lse, int D,
                                                                     int64_t plane, int64_t n_vec) {
@@ -42,7 +122,7 @@ __global__ void __launch_bounds__(kSAThreads) soft_argmin_fwd_kernel(const float
     if (t >= n_vec) return;
     const int64_t pix = t * V;
     const int64_t b = pix / plane, hw = pix - b * plane;
-    const float* src = cost + b * D * plane + hw;
+    const T* src = cost + b * D * plane + hw;
 
     // m = running max.  Exponents are formed as (x - m) * log2e: the subtraction is exact for the
     // entries that carry weight (x close to m), so accuracy does not depend on the magnitude of the
@@ -58,8 +138,7 @@ __global__ void __launch_bounds__(kSAThreads) soft_argmin_fwd_kernel(const float
 #pragma unroll
         for (int k = 0; k < kChunk; ++k) {
             if (d0 + k < D) {
-                const VT v = ld_stream(reinterpret_cast<const VT*>(src + (int64_t)(d0 + k) * plane));
-                Vec<V>::unpack(v, x[k]);
+                Lanes<T, V>::widen(Lanes<T, V>::ld(src + (int64_t)(d0 + k) * plane), x[k]);
             } else {
 #pragma unroll
                 for (int j = 0; j < V; ++j) x[k][j] = -INFINITY;
@@ -169,16 +248,20 @@ __device__ __forceinline__ double to_double_pos(float f) {
     return (double)f;
 }
 
-template <int POLY, bool BITS>
-__global__ void __launch_bounds__(kSAThreads) soft_argmin_fwd_packed_kernel(const float* __restrict__ cost,
+// T = float: one chunk of 8 planes per pass.  T = bf16 / fp16 (logits widened at the load): two chunks per pass, each
+// reduced exactly as the fp32 kernel reduces it; ALIGNED = false takes 2-byte loads and 4-byte stores (a view with
+// a storage offset) with the same arithmetic.
+template <typename T, int POLY, bool BITS, bool ALIGNED = true>
+__global__ void __launch_bounds__(kSAThreads) soft_argmin_fwd_packed_kernel(const T* __restrict__ cost,
                                                                            float* __restrict__ disp,
                                                                            float* __restrict__ lse, int D,
                                                                            int64_t plane, int64_t n_vec) {
+    constexpr int NF = kFlight<T, 4>;
     const int64_t t = (int64_t)blockIdx.x * kSAThreads + threadIdx.x;
     if (t >= n_vec) return;
     const int64_t pix = t * 4;
     const int64_t b = pix / plane, hw = pix - b * plane;
-    const float* src = cost + b * D * plane + hw;
+    const T* src = cost + b * D * plane + hw;
     const u64p kL2 = pk(kLog2e, kLog2e);
 
     float m[4];
@@ -186,21 +269,27 @@ __global__ void __launch_bounds__(kSAThreads) soft_argmin_fwd_packed_kernel(cons
 #pragma unroll
     for (int j = 0; j < 4; ++j) { m[j] = -INFINITY; s[j] = 0.0; ws[j] = 0.0; }
 
-    for (int d0 = 0; d0 < D; d0 += kChunk) {
-        float4 v[kChunk];
+    for (int d00 = 0; d00 < D; d00 += NF * kChunk) {
+        typename Lanes<T, 4>::R v[NF * kChunk];  // 16-bit: raw words until use (registers for all 16 planes in flight)
 #pragma unroll
-        for (int k = 0; k < kChunk; ++k) {
-            if (d0 + k < D) v[k] = ld_stream(reinterpret_cast<const float4*>(src + (int64_t)(d0 + k) * plane));
-            else v[k] = make_float4(-INFINITY, -INFINITY, -INFINITY, -INFINITY);
+        for (int k = 0; k < NF * kChunk; ++k) {
+            if (d00 + k < D) v[k] = ld_raw4<ALIGNED>(src + (int64_t)(d00 + k) * plane);
+            else v[k] = neg_inf4<T>();
         }
+#pragma unroll
+        for (int c = 0; c < NF; ++c) {
+        const int d0 = d00 + c * kChunk;
+        if (c > 0 && d0 >= D) break;  // (uniform) a pass may end in a chunk past the last plane
         const double dd0 = (double)d0;
 #pragma unroll
         for (int h = 0; h < 2; ++h) {
             float xa[kChunk], xb[kChunk];
 #pragma unroll
             for (int k = 0; k < kChunk; ++k) {
-                xa[k] = h == 0 ? v[k].x : v[k].z;
-                xb[k] = h == 0 ? v[k].y : v[k].w;
+                float f[4];
+                Lanes<T, 4>::widen(v[c * kChunk + k], f);
+                xa[k] = f[2 * h];
+                xb[k] = f[2 * h + 1];
             }
             float ca = xa[0], cb = xb[0];
 #pragma unroll
@@ -248,6 +337,7 @@ __global__ void __launch_bounds__(kSAThreads) soft_argmin_fwd_packed_kernel(cons
             ws[2 * h] += fma(dd0, dsa, to_double_pos<BITS>(cwa));
             ws[2 * h + 1] += fma(dd0, dsb, to_double_pos<BITS>(cwb));
         }
+        }
     }
     float o[4], l[4];
 #pragma unroll
@@ -255,53 +345,71 @@ __global__ void __launch_bounds__(kSAThreads) soft_argmin_fwd_packed_kernel(cons
         o[j] = (float)(ws[j] / s[j]);
         l[j] = log2f((float)s[j]);
     }
-    *reinterpret_cast<float4*>(disp + pix) = make_float4(o[0], o[1], o[2], o[3]);
-    if (lse != nullptr) {
-        const int64_t total = n_vec * 4;
-        *reinterpret_cast<float4*>(lse + pix) = make_float4(m[0], m[1], m[2], m[3]);
-        *reinterpret_cast<float4*>(lse + total + pix) = make_float4(l[0], l[1], l[2], l[3]);
+    const int64_t total = n_vec * 4;
+    if (ALIGNED) {
+        *reinterpret_cast<float4*>(disp + pix) = make_float4(o[0], o[1], o[2], o[3]);
+        if (lse != nullptr) {
+            *reinterpret_cast<float4*>(lse + pix) = make_float4(m[0], m[1], m[2], m[3]);
+            *reinterpret_cast<float4*>(lse + total + pix) = make_float4(l[0], l[1], l[2], l[3]);
+        }
+    } else {
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            disp[pix + j] = o[j];
+            if (lse != nullptr) {
+                lse[pix + j] = m[j];
+                lse[total + pix + j] = l[j];
+            }
+        }
     }
 }
 
-template <int V>
-__global__ void __launch_bounds__(kSAThreads) soft_argmin_bwd_kernel(const float* __restrict__ cost,
+// T = bf16 / fp16: the gradient is formed in fp32 exactly as for fp32 logits and rounded once (RNE) at the store.
+// V = 8 (8 pixels, 16-byte accesses, 8 planes per pass) where H*W % 8 == 0 and the pointers allow it, else V = 4 with
+// the CTA's 16 planes loaded at once: both keep the fp32 kernel's bytes per pass; V = 8 measured faster (§4.12).
+template <typename T, int V, int KF = kFlight<T, V> * kChunk>
+__global__ void __launch_bounds__(kSAThreads) soft_argmin_bwd_kernel(const T* __restrict__ cost,
                                                                     const float* __restrict__ disp,
                                                                     const float* __restrict__ lse,
                                                                     const float* __restrict__ gdisp,
-                                                                    float* __restrict__ gcost, int D,
+                                                                    T* __restrict__ gcost, int D,
                                                                     int64_t plane, int64_t n_vec, int dgroup) {
     // grid.y splits the D planes into groups of `dgroup`: short-lived CTAs keep the store half of this
     // read-modify-write stream nearer the write-only ceiling (benchmarks/micro/store_patterns.cu)
-    using VT = typename Vec<V>::T;
+    constexpr int VW = V == 8 ? 4 : V;  // fp32 vector width of the disp / lse / gdisp reads
+    using VT = typename Vec<VW>::T;
     const int64_t t = (int64_t)blockIdx.x * kSAThreads + threadIdx.x;
     if (t >= n_vec) return;
     const int64_t pix = t * V;
     const int64_t b = pix / plane, hw = pix - b * plane;
-    const float* src = cost + b * D * plane + hw;
-    float* dst = gcost + b * D * plane + hw;
+    const T* src = cost + b * D * plane + hw;
+    T* dst = gcost + b * D * plane + hw;
     const int dbeg = blockIdx.y * dgroup, dend = min(D, dbeg + dgroup);
     float o[V], mx[V], lb[V], g[V];
-    Vec<V>::unpack(*reinterpret_cast<const VT*>(disp + pix), o);
-    Vec<V>::unpack(*reinterpret_cast<const VT*>(lse + pix), mx);
-    Vec<V>::unpack(*reinterpret_cast<const VT*>(lse + n_vec * V + pix), lb);
-    Vec<V>::unpack(*reinterpret_cast<const VT*>(gdisp + pix), g);
-    for (int d0 = dbeg; d0 < dend; d0 += kChunk) {
-        VT v[kChunk];
 #pragma unroll
-        for (int k = 0; k < kChunk; ++k)
-            if (d0 + k < dend) v[k] = ld_stream(reinterpret_cast<const VT*>(src + (int64_t)(d0 + k) * plane));
+    for (int q = 0; q < V; q += VW) {
+        Vec<VW>::unpack(*reinterpret_cast<const VT*>(disp + pix + q), o + q);
+        Vec<VW>::unpack(*reinterpret_cast<const VT*>(lse + pix + q), mx + q);
+        Vec<VW>::unpack(*reinterpret_cast<const VT*>(lse + n_vec * V + pix + q), lb + q);
+        Vec<VW>::unpack(*reinterpret_cast<const VT*>(gdisp + pix + q), g + q);
+    }
+    for (int d0 = dbeg; d0 < dend; d0 += KF) {
+        typename Lanes<T, V>::R v[KF];
 #pragma unroll
-        for (int k = 0; k < kChunk; ++k) {
+        for (int k = 0; k < KF; ++k)
+            if (d0 + k < dend) v[k] = Lanes<T, V>::ld(src + (int64_t)(d0 + k) * plane);
+#pragma unroll
+        for (int k = 0; k < KF; ++k) {
             if (d0 + k < dend) {
                 float x[V], r[V];
-                Vec<V>::unpack(v[k], x);
+                Lanes<T, V>::widen(v[k], x);
                 const float dd = (float)(d0 + k);
 #pragma unroll
                 for (int j = 0; j < V; ++j) {
                     const float p = fast_ex2(fmaf(x[j] - mx[j], kLog2e, -lb[j]));
                     r[j] = p * (dd - o[j]) * g[j];
                 }
-                st_stream(reinterpret_cast<VT*>(dst + (int64_t)(d0 + k) * plane), Vec<V>::pack(r));
+                st_vec<V>(dst + (int64_t)(d0 + k) * plane, r);
             }
         }
     }
@@ -322,15 +430,15 @@ extern "C" int az_soft_argmin_fwd(const float* cost, float* disp, float* lse, in
         const unsigned grid = (unsigned)ceil_div(n, kSAThreads);
         // 0 = generic kernel; 1 = packed; 2 = packed + integer conversions; 3 / 4 = (2) + 2 / 4 polynomial exp2 per chunk
         switch (az::tuning("AZ_SA_FWD", 2)) {
-            case 0: soft_argmin_fwd_kernel<4><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, (int)D, plane, n); break;
-            case 1: soft_argmin_fwd_packed_kernel<0, false><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, (int)D, plane, n); break;
-            case 3: soft_argmin_fwd_packed_kernel<2, true><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, (int)D, plane, n); break;
-            case 4: soft_argmin_fwd_packed_kernel<4, true><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, (int)D, plane, n); break;
-            default: soft_argmin_fwd_packed_kernel<0, true><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, (int)D, plane, n); break;
+            case 0: soft_argmin_fwd_kernel<float, 4><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, (int)D, plane, n); break;
+            case 1: soft_argmin_fwd_packed_kernel<float, 0, false><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, (int)D, plane, n); break;
+            case 3: soft_argmin_fwd_packed_kernel<float, 2, true><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, (int)D, plane, n); break;
+            case 4: soft_argmin_fwd_packed_kernel<float, 4, true><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, (int)D, plane, n); break;
+            default: soft_argmin_fwd_packed_kernel<float, 0, true><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, (int)D, plane, n); break;
         }
     } else {
-        soft_argmin_fwd_kernel<1><<<(unsigned)ceil_div(total, kSAThreads), kSAThreads, 0, st>>>(cost, disp, lse, (int)D,
-                                                                                               plane, total);
+        soft_argmin_fwd_kernel<float, 1><<<(unsigned)ceil_div(total, kSAThreads), kSAThreads, 0, st>>>(
+            cost, disp, lse, (int)D, plane, total);
     }
     AZ_LAUNCH_CHECK();
     return 0;
@@ -349,12 +457,85 @@ extern "C" int az_soft_argmin_bwd(const float* cost, const float* disp, const fl
     if (vec) {
         const int64_t n = total / 4;
         dim3 grid((unsigned)ceil_div(n, kSAThreads), ngroups);
-        soft_argmin_bwd_kernel<4><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, gdisp, gcost, (int)D, plane, n, dgroup);
+        soft_argmin_bwd_kernel<float, 4><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, gdisp, gcost, (int)D, plane, n, dgroup);
     } else {
         dim3 grid((unsigned)ceil_div(total, kSAThreads), ngroups);
-        soft_argmin_bwd_kernel<1><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, gdisp, gcost, (int)D, plane, total,
-                                                               dgroup);
+        soft_argmin_bwd_kernel<float, 1><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, gdisp, gcost, (int)D, plane, total,
+                                                                      dgroup);
     }
     AZ_LAUNCH_CHECK();
     return 0;
+}
+
+// 16-bit logits.  The forward picks its arithmetic by the fp32 operator's shape rule alone (the packed kernel when
+// H*W % 4 == 0, else the generic one), never by the alignment of the 16-bit pointer, so that it matches the fp32
+// operator on cost.float() (a fresh, aligned tensor) for any view; the AZ_SA_FWD knob is not consulted.  The backward's
+// arithmetic is the same per element at every vector width, so its width follows the shape and the pointers.
+template <typename T>
+static int soft_argmin_fwd16(const T* cost, float* disp, float* lse, int64_t B, int64_t D, int64_t H, int64_t W,
+                             cudaStream_t st) {
+    const int64_t plane = H * W, total = B * plane;
+    if (plane % 4 == 0) {
+        const int64_t n = total / 4;
+        const unsigned grid = (unsigned)ceil_div(n, kSAThreads);
+        const bool al = ((reinterpret_cast<uintptr_t>(cost) & 7u) == 0) && aligned16(disp) &&
+                        (lse == nullptr || aligned16(lse));
+        if (al) soft_argmin_fwd_packed_kernel<T, 0, true, true><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, (int)D, plane, n);
+        else soft_argmin_fwd_packed_kernel<T, 0, true, false><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, (int)D, plane, n);
+    } else {
+        soft_argmin_fwd_kernel<T, 1><<<(unsigned)ceil_div(total, kSAThreads), kSAThreads, 0, st>>>(cost, disp, lse,
+                                                                                                  (int)D, plane, total);
+    }
+    AZ_LAUNCH_CHECK();
+    return 0;
+}
+
+template <typename T>
+static int soft_argmin_bwd16(const T* cost, const float* disp, const float* lse, const float* gdisp, T* gcost,
+                             int64_t B, int64_t D, int64_t H, int64_t W, cudaStream_t st) {
+    const int64_t plane = H * W, total = B * plane;
+    const bool vec = (plane % 4 == 0) && ((reinterpret_cast<uintptr_t>(cost) & 7u) == 0) &&
+                     ((reinterpret_cast<uintptr_t>(gcost) & 7u) == 0) && aligned16(disp) && aligned16(lse) &&
+                     aligned16(gdisp);
+    const int dgroup = kBwdDGroup;
+    const unsigned ngroups = (unsigned)ceil_div(D, dgroup);
+    if (ngroups > 65535) return AZ_ERR_BAD_ARG;
+    if (vec && plane % 8 == 0 && aligned16(cost) && aligned16(gcost)) {
+        const int64_t n = total / 8;
+        dim3 grid((unsigned)ceil_div(n, kSAThreads), ngroups);
+        soft_argmin_bwd_kernel<T, 8><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, gdisp, gcost, (int)D, plane, n, dgroup);
+    } else if (vec) {
+        const int64_t n = total / 4;
+        dim3 grid((unsigned)ceil_div(n, kSAThreads), ngroups);
+        soft_argmin_bwd_kernel<T, 4><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, gdisp, gcost, (int)D, plane, n, dgroup);
+    } else {
+        dim3 grid((unsigned)ceil_div(total, kSAThreads), ngroups);
+        soft_argmin_bwd_kernel<T, 1><<<grid, kSAThreads, 0, st>>>(cost, disp, lse, gdisp, gcost, (int)D, plane, total,
+                                                                  dgroup);
+    }
+    AZ_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int az_soft_argmin_fwd_16(const void* cost, float* disp, float* lse, int64_t B, int64_t D, int64_t H,
+                                     int64_t W, int dtype, void* stream) {
+    if (!cost || !disp || B <= 0 || D <= 0 || H <= 0 || W <= 0) return AZ_ERR_BAD_ARG;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dtype == AZ_DTYPE_BF16)
+        return soft_argmin_fwd16(static_cast<const __nv_bfloat16*>(cost), disp, lse, B, D, H, W, st);
+    if (dtype == AZ_DTYPE_F16) return soft_argmin_fwd16(static_cast<const __half*>(cost), disp, lse, B, D, H, W, st);
+    return AZ_ERR_BAD_ARG;
+}
+
+extern "C" int az_soft_argmin_bwd_16(const void* cost, const float* disp, const float* lse, const float* gdisp,
+                                     void* gcost, int64_t B, int64_t D, int64_t H, int64_t W, int dtype, void* stream) {
+    if (!cost || !disp || !lse || !gdisp || !gcost || B <= 0 || D <= 0 || H <= 0 || W <= 0) return AZ_ERR_BAD_ARG;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dtype == AZ_DTYPE_BF16)
+        return soft_argmin_bwd16(static_cast<const __nv_bfloat16*>(cost), disp, lse, gdisp,
+                                 static_cast<__nv_bfloat16*>(gcost), B, D, H, W, st);
+    if (dtype == AZ_DTYPE_F16)
+        return soft_argmin_bwd16(static_cast<const __half*>(cost), disp, lse, gdisp, static_cast<__half*>(gcost), B, D,
+                                 H, W, st);
+    return AZ_ERR_BAD_ARG;
 }

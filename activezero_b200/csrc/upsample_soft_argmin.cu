@@ -52,16 +52,18 @@ __device__ __forceinline__ float bil(const float* __restrict__ plane, const Taps
 }
 
 // Loads the [Dq][fh][fw] footprint of this CTA's output tile.  64 threads walk the fh*fw positions (one
-// integer division each), the 4 groups of 64 interleave over the Dq planes: no div/mod in the inner loop.
-__device__ __forceinline__ void load_tile(const float* __restrict__ low, float* __restrict__ tile, int b, int Dq, int Hq,
+// integer division each), the 4 groups of 64 interleave over the Dq planes: no div/mod in the inner loop.  16-bit
+// logits are widened (exactly) here: the tile is fp32 for every input type.
+template <typename T>
+__device__ __forceinline__ void load_tile(const T* __restrict__ low, float* __restrict__ tile, int b, int Dq, int Hq,
                                           int Wq, int h_lo, int w_lo, int fh, int fw, int FHW) {
     const int tid = threadIdx.y * kUTW + threadIdx.x;
     const int npos = fh * fw;
     const size_t plane = (size_t)Hq * Wq;
     for (int pos = tid & 63; pos < npos; pos += 64) {
         const int hh = pos / fw, ww = pos - hh * fw;
-        const float* src = low + (size_t)b * Dq * plane + (size_t)(h_lo + hh) * Wq + (w_lo + ww);
-        for (int q = tid >> 6; q < Dq; q += (kUTW * kUTH) >> 6) tile[q * FHW + pos] = __ldg(src + (size_t)q * plane);
+        const T* src = low + (size_t)b * Dq * plane + (size_t)(h_lo + hh) * Wq + (w_lo + ww);
+        for (int q = tid >> 6; q < Dq; q += (kUTW * kUTH) >> 6) tile[q * FHW + pos] = ld_f32(src + (size_t)q * plane);
     }
 }
 
@@ -81,8 +83,9 @@ __device__ __forceinline__ void build_depth_lut(float* __restrict__ l1, int* __r
 
 // grid = (ceil(W/32), ceil(H/8), B), block = (32, 8)
 // smem: tile[Dq*FHW] floats | l1[D] floats | dstart[Dq+1] ints
+template <typename T>
 __global__ void __launch_bounds__(kUTW * kUTH) upsample_soft_argmin_fwd_kernel(
-    const float* __restrict__ low, float* __restrict__ disp, float* __restrict__ stats, int Dq, int Hq, int Wq, int D,
+    const T* __restrict__ low, float* __restrict__ disp, float* __restrict__ stats, int Dq, int Hq, int Wq, int D,
     int H, int W, float sd, float sh, float sw, int FHW, int64_t total) {
     extern __shared__ float tile[];
     float* l1 = tile + (size_t)Dq * FHW;
@@ -144,8 +147,9 @@ __global__ void __launch_bounds__(kUTW * kUTH) upsample_soft_argmin_fwd_kernel(
 }
 
 // backward stage 1: per-pixel gradient w.r.t. the Dq interpolated planes v_q(y,x).  G: [B,Dq,H,W]
+template <typename T>
 __global__ void __launch_bounds__(kUTW * kUTH) upsample_soft_argmin_bwd_pix_kernel(
-    const float* __restrict__ low, const float* __restrict__ disp, const float* __restrict__ stats,
+    const T* __restrict__ low, const float* __restrict__ disp, const float* __restrict__ stats,
     const float* __restrict__ gdisp, float* __restrict__ G, int Dq, int Hq, int Wq, int D, int H, int W, float sd,
     float sh, float sw, int FHW, int64_t total) {
     extern __shared__ float tile[];
@@ -230,8 +234,9 @@ __device__ __forceinline__ Taps make_taps(float sh, float sw, int y, int x, int 
     return t;
 }
 
+template <typename T>
 __global__ void __launch_bounds__(kUTW * kUTH) upsample4_soft_argmin_fwd_kernel(
-    const float* __restrict__ low, float* __restrict__ disp, float* __restrict__ stats, int Dq, int Hq, int Wq, int H,
+    const T* __restrict__ low, float* __restrict__ disp, float* __restrict__ stats, int Dq, int Hq, int Wq, int H,
     int W, float sh, float sw, int FHW, int64_t total) {
     extern __shared__ float tile[];
     const int b = blockIdx.z;
@@ -340,8 +345,9 @@ __device__ __forceinline__ void bil4(const float* __restrict__ pl, int oa, int o
 }
 
 // grid = (ceil((Wq + 1) / 32), ceil(H / 8), B), block = (32, 8).  smem: tile[Dq][fh][33]
+template <typename T>
 __global__ void __launch_bounds__(kU4G * kU4H) upsample4x_soft_argmin_fwd_kernel(
-    const float* __restrict__ low, float* __restrict__ disp, float* __restrict__ stats, int Dq, int Hq, int Wq, int H,
+    const T* __restrict__ low, float* __restrict__ disp, float* __restrict__ stats, int Dq, int Hq, int Wq, int H,
     float sh, int fh_cap, int64_t total) {
     extern __shared__ float tile[];
     const int b = blockIdx.z, W = 4 * Wq;
@@ -357,8 +363,8 @@ __global__ void __launch_bounds__(kU4G * kU4H) upsample4x_soft_argmin_fwd_kernel
         for (int pos = tid & 63; pos < npos; pos += 64) {
             const int hh = pos / kU4FW, ww = pos - hh * kU4FW;
             const int col = min(max(c0 + ww, 0), Wq - 1);
-            const float* srcp = low + (size_t)b * Dq * plane + (size_t)(h_lo + hh) * Wq + col;
-            for (int q = tid >> 6; q < Dq; q += (kU4G * kU4H) >> 6) tile[q * FHW + pos] = __ldg(srcp + (size_t)q * plane);
+            const T* srcp = low + (size_t)b * Dq * plane + (size_t)(h_lo + hh) * Wq + col;
+            for (int q = tid >> 6; q < Dq; q += (kU4G * kU4H) >> 6) tile[q * FHW + pos] = ld_f32(srcp + (size_t)q * plane);
         }
     }
     __syncthreads();
@@ -507,8 +513,9 @@ __global__ void __launch_bounds__(kU4G * kU4H) upsample4x_soft_argmin_fwd_kernel
     }
 }
 
+template <typename T>
 __global__ void __launch_bounds__(kUTW * kUTH) upsample4_soft_argmin_bwd_pix_kernel(
-    const float* __restrict__ low, const float* __restrict__ disp, const float* __restrict__ stats,
+    const T* __restrict__ low, const float* __restrict__ disp, const float* __restrict__ stats,
     const float* __restrict__ gdisp, float* __restrict__ G, int Dq, int Hq, int Wq, int H, int W, float sh, float sw,
     int FHW, int64_t total) {
     extern __shared__ float tile[];
@@ -601,7 +608,9 @@ __global__ void __launch_bounds__(128) upsample_bwd_reduce_x_kernel(const float*
 }
 
 // backward stage 3: glow[b,q,h,w] = sum_y wy(y,h) * T[b,q,y,w].   grid = (ceil(Wq/128), Hq, B*Dq)
-__global__ void __launch_bounds__(128) upsample_bwd_reduce_y_kernel(const float* __restrict__ T, float* __restrict__ glow,
+// glow of 16 bits: the fp32 sum is rounded once, to nearest even, at the store.
+template <typename O>
+__global__ void __launch_bounds__(128) upsample_bwd_reduce_y_kernel(const float* __restrict__ T, O* __restrict__ glow,
                                                                    int H, int Hq, int Wq, float sh) {
     const int w = blockIdx.x * 128 + threadIdx.x;
     if (w >= Wq) return;
@@ -620,7 +629,7 @@ __global__ void __launch_bounds__(128) upsample_bwd_reduce_y_kernel(const float*
         if (l.i1 == h) wt += l.l1;
         if (wt != 0.f) acc = fmaf(wt, __ldg(T + (plane * H + y) * Wq + w), acc);
     }
-    glow[(plane * Hq + h) * Wq + w] = acc;
+    st_from_f32(glow + (plane * Hq + h) * Wq + w, acc);
 }
 
 static int tile_extent(int in_size, int out_size, int tile) {
@@ -646,47 +655,91 @@ static int upsample_args_ok(int64_t B, int64_t Dq, int64_t Hq, int64_t Wq, int64
     return 1;
 }
 
-extern "C" int az_upsample_soft_argmin_fwd(const float* lowres, float* disp, float* stats, int64_t B, int64_t Dq,
-                                           int64_t Hq, int64_t Wq, int64_t D, int64_t H, int64_t W, void* stream) {
-    if (!lowres || !disp || !upsample_args_ok(B, Dq, Hq, Wq, D, H, W)) return AZ_ERR_BAD_ARG;
+// fp32 (knob = the AZ_USA_FWD developer knob) and 16-bit low-res logits (knob = 1, the default: the kernel choice is a
+// function of the shape alone, as for fp32 at the default).
+template <typename T>
+static int upsample_fwd(const T* lowres, float* disp, float* stats, int64_t B, int64_t Dq, int64_t Hq, int64_t Wq,
+                        int64_t D, int64_t H, int64_t W, int knob, cudaStream_t stream) {
     const int fh = tile_extent((int)Hq, (int)H, kUTH), fw = tile_extent((int)Wq, (int)W, kUTW);
     const int FHW = fh * fw;
     const size_t smem = ((size_t)Dq * FHW + D + Dq + 1) * sizeof(float);
     if (smem > 200 * 1024) return AZ_ERR_BAD_ARG;
-    cudaError_t e = cudaFuncSetAttribute(upsample_soft_argmin_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(upsample_soft_argmin_fwd_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          200 * 1024);
     if (e != cudaSuccess) return (int)e;
     dim3 grid((unsigned)ceil_div(W, kUTW), (unsigned)ceil_div(H, kUTH), (unsigned)B);
-    if (D == 4 * Dq && Dq >= 2 && W == 4 * Wq && az::tuning("AZ_USA_FWD", 1) == 1) {
+    if (D == 4 * Dq && Dq >= 2 && W == 4 * Wq && knob == 1) {
         // x4 in depth and width (PSMNet): 4 pixels per thread, packed arithmetic, 2 ex2 per interval
         const int fh4 = tile_extent((int)Hq, (int)H, kU4H);
         const size_t smem4 = (size_t)Dq * fh4 * kU4FW * sizeof(float);
         if (smem4 <= 200 * 1024) {
-            e = cudaFuncSetAttribute(upsample4x_soft_argmin_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+            e = cudaFuncSetAttribute(upsample4x_soft_argmin_fwd_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                      200 * 1024);
             if (e != cudaSuccess) return (int)e;
             dim3 g4((unsigned)ceil_div(Wq + 1, kU4G), (unsigned)ceil_div(H, kU4H), (unsigned)B);
-            upsample4x_soft_argmin_fwd_kernel<<<g4, dim3(kU4G, kU4H), smem4, (cudaStream_t)stream>>>(
+            upsample4x_soft_argmin_fwd_kernel<T><<<g4, dim3(kU4G, kU4H), smem4, stream>>>(
                 lowres, disp, stats, (int)Dq, (int)Hq, (int)Wq, (int)H, (float)Hq / (float)H, fh4, B * H * W);
             AZ_LAUNCH_CHECK();
             return 0;
         }
     }
     if (D == 4 * Dq && Dq >= 2) {
-        e = cudaFuncSetAttribute(upsample4_soft_argmin_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        e = cudaFuncSetAttribute(upsample4_soft_argmin_fwd_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  200 * 1024);
         if (e != cudaSuccess) return (int)e;
-        upsample4_soft_argmin_fwd_kernel<<<grid, dim3(kUTW, kUTH), smem, (cudaStream_t)stream>>>(
+        upsample4_soft_argmin_fwd_kernel<T><<<grid, dim3(kUTW, kUTH), smem, stream>>>(
             lowres, disp, stats, (int)Dq, (int)Hq, (int)Wq, (int)H, (int)W, (float)Hq / (float)H, (float)Wq / (float)W,
             FHW, B * H * W);
         AZ_LAUNCH_CHECK();
         return 0;
     }
-    upsample_soft_argmin_fwd_kernel<<<grid, dim3(kUTW, kUTH), smem, (cudaStream_t)stream>>>(
+    upsample_soft_argmin_fwd_kernel<T><<<grid, dim3(kUTW, kUTH), smem, stream>>>(
         lowres, disp, stats, (int)Dq, (int)Hq, (int)Wq, (int)D, (int)H, (int)W, (float)Dq / (float)D,
         (float)Hq / (float)H, (float)Wq / (float)W, FHW, B * H * W);
     AZ_LAUNCH_CHECK();
     return 0;
+}
+
+template <typename T>
+static int upsample_bwd(const T* lowres, const float* disp, const float* stats, const float* gdisp, T* glow,
+                        void* workspace, int64_t B, int64_t Dq, int64_t Hq, int64_t Wq, int64_t D, int64_t H, int64_t W,
+                        cudaStream_t st) {
+    const int fh = tile_extent((int)Hq, (int)H, kUTH), fw = tile_extent((int)Wq, (int)W, kUTW);
+    const int FHW = fh * fw;
+    const size_t smem = ((size_t)Dq * FHW + D + Dq + 1) * sizeof(float);
+    if (smem > 200 * 1024) return AZ_ERR_BAD_ARG;
+    cudaError_t e = cudaFuncSetAttribute(upsample_soft_argmin_bwd_pix_kernel<T>,
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    if (e != cudaSuccess) return (int)e;
+    float* G = (float*)workspace;
+    float* Tw = G + B * Dq * H * W;
+    const float sd = (float)Dq / (float)D, sh = (float)Hq / (float)H, sw = (float)Wq / (float)W;
+    dim3 grid((unsigned)ceil_div(W, kUTW), (unsigned)ceil_div(H, kUTH), (unsigned)B);
+    if (D == 4 * Dq && Dq >= 2) {
+        e = cudaFuncSetAttribute(upsample4_soft_argmin_bwd_pix_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 200 * 1024);
+        if (e != cudaSuccess) return (int)e;
+        upsample4_soft_argmin_bwd_pix_kernel<T><<<grid, dim3(kUTW, kUTH), smem, st>>>(
+            lowres, disp, stats, gdisp, G, (int)Dq, (int)Hq, (int)Wq, (int)H, (int)W, sh, sw, FHW, B * H * W);
+    } else {
+        upsample_soft_argmin_bwd_pix_kernel<T><<<grid, dim3(kUTW, kUTH), smem, st>>>(
+            lowres, disp, stats, gdisp, G, (int)Dq, (int)Hq, (int)Wq, (int)D, (int)H, (int)W, sd, sh, sw, FHW,
+            B * H * W);
+    }
+    AZ_LAUNCH_CHECK();
+    dim3 gx((unsigned)ceil_div(Wq, 128), (unsigned)ceil_div(H, kRowsPerCta), (unsigned)(B * Dq));
+    upsample_bwd_reduce_x_kernel<<<gx, 128, 0, st>>>(G, Tw, (int)H, (int)W, (int)Wq, sw);
+    AZ_LAUNCH_CHECK();
+    dim3 gy((unsigned)ceil_div(Wq, 128), (unsigned)Hq, (unsigned)(B * Dq));
+    upsample_bwd_reduce_y_kernel<T><<<gy, 128, 0, st>>>(Tw, glow, (int)H, (int)Hq, (int)Wq, sh);
+    AZ_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int az_upsample_soft_argmin_fwd(const float* lowres, float* disp, float* stats, int64_t B, int64_t Dq,
+                                           int64_t Hq, int64_t Wq, int64_t D, int64_t H, int64_t W, void* stream) {
+    if (!lowres || !disp || !upsample_args_ok(B, Dq, Hq, Wq, D, H, W)) return AZ_ERR_BAD_ARG;
+    return upsample_fwd(lowres, disp, stats, B, Dq, Hq, Wq, D, H, W, az::tuning("AZ_USA_FWD", 1), (cudaStream_t)stream);
 }
 
 extern "C" int az_upsample_soft_argmin_bwd(const float* lowres, const float* disp, const float* stats,
@@ -694,35 +747,33 @@ extern "C" int az_upsample_soft_argmin_bwd(const float* lowres, const float* dis
                                            int64_t Hq, int64_t Wq, int64_t D, int64_t H, int64_t W, void* stream) {
     if (!lowres || !disp || !stats || !gdisp || !glow || !workspace || !upsample_args_ok(B, Dq, Hq, Wq, D, H, W))
         return AZ_ERR_BAD_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-    const int fh = tile_extent((int)Hq, (int)H, kUTH), fw = tile_extent((int)Wq, (int)W, kUTW);
-    const int FHW = fh * fw;
-    const size_t smem = ((size_t)Dq * FHW + D + Dq + 1) * sizeof(float);
-    if (smem > 200 * 1024) return AZ_ERR_BAD_ARG;
-    cudaError_t e = cudaFuncSetAttribute(upsample_soft_argmin_bwd_pix_kernel,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (e != cudaSuccess) return (int)e;
-    float* G = (float*)workspace;
-    float* T = G + B * Dq * H * W;
-    const float sd = (float)Dq / (float)D, sh = (float)Hq / (float)H, sw = (float)Wq / (float)W;
-    dim3 grid((unsigned)ceil_div(W, kUTW), (unsigned)ceil_div(H, kUTH), (unsigned)B);
-    if (D == 4 * Dq && Dq >= 2) {
-        e = cudaFuncSetAttribute(upsample4_soft_argmin_bwd_pix_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 200 * 1024);
-        if (e != cudaSuccess) return (int)e;
-        upsample4_soft_argmin_bwd_pix_kernel<<<grid, dim3(kUTW, kUTH), smem, st>>>(
-            lowres, disp, stats, gdisp, G, (int)Dq, (int)Hq, (int)Wq, (int)H, (int)W, sh, sw, FHW, B * H * W);
-    } else {
-        upsample_soft_argmin_bwd_pix_kernel<<<grid, dim3(kUTW, kUTH), smem, st>>>(
-            lowres, disp, stats, gdisp, G, (int)Dq, (int)Hq, (int)Wq, (int)D, (int)H, (int)W, sd, sh, sw, FHW,
-            B * H * W);
-    }
-    AZ_LAUNCH_CHECK();
-    dim3 gx((unsigned)ceil_div(Wq, 128), (unsigned)ceil_div(H, kRowsPerCta), (unsigned)(B * Dq));
-    upsample_bwd_reduce_x_kernel<<<gx, 128, 0, st>>>(G, T, (int)H, (int)W, (int)Wq, sw);
-    AZ_LAUNCH_CHECK();
-    dim3 gy((unsigned)ceil_div(Wq, 128), (unsigned)Hq, (unsigned)(B * Dq));
-    upsample_bwd_reduce_y_kernel<<<gy, 128, 0, st>>>(T, glow, (int)H, (int)Hq, (int)Wq, sh);
-    AZ_LAUNCH_CHECK();
-    return 0;
+    return upsample_bwd(lowres, disp, stats, gdisp, glow, workspace, B, Dq, Hq, Wq, D, H, W, (cudaStream_t)stream);
+}
+
+extern "C" int az_upsample_soft_argmin_fwd_16(const void* lowres, float* disp, float* stats, int64_t B, int64_t Dq,
+                                              int64_t Hq, int64_t Wq, int64_t D, int64_t H, int64_t W, int dtype,
+                                              void* stream) {
+    if (!lowres || !disp || !upsample_args_ok(B, Dq, Hq, Wq, D, H, W)) return AZ_ERR_BAD_ARG;
+    if (dtype == AZ_DTYPE_BF16)
+        return upsample_fwd(static_cast<const __nv_bfloat16*>(lowres), disp, stats, B, Dq, Hq, Wq, D, H, W, 1,
+                            (cudaStream_t)stream);
+    if (dtype == AZ_DTYPE_F16)
+        return upsample_fwd(static_cast<const __half*>(lowres), disp, stats, B, Dq, Hq, Wq, D, H, W, 1,
+                            (cudaStream_t)stream);
+    return AZ_ERR_BAD_ARG;
+}
+
+extern "C" int az_upsample_soft_argmin_bwd_16(const void* lowres, const float* disp, const float* stats,
+                                              const float* gdisp, void* glow, void* workspace, int64_t B, int64_t Dq,
+                                              int64_t Hq, int64_t Wq, int64_t D, int64_t H, int64_t W, int dtype,
+                                              void* stream) {
+    if (!lowres || !disp || !stats || !gdisp || !glow || !workspace || !upsample_args_ok(B, Dq, Hq, Wq, D, H, W))
+        return AZ_ERR_BAD_ARG;
+    if (dtype == AZ_DTYPE_BF16)
+        return upsample_bwd(static_cast<const __nv_bfloat16*>(lowres), disp, stats, gdisp,
+                            static_cast<__nv_bfloat16*>(glow), workspace, B, Dq, Hq, Wq, D, H, W, (cudaStream_t)stream);
+    if (dtype == AZ_DTYPE_F16)
+        return upsample_bwd(static_cast<const __half*>(lowres), disp, stats, gdisp, static_cast<__half*>(glow),
+                            workspace, B, Dq, Hq, Wq, D, H, W, (cudaStream_t)stream);
+    return AZ_ERR_BAD_ARG;
 }

@@ -34,7 +34,9 @@ import torch
 from torch import Tensor
 
 from . import _lib, _volume_conv_library
-from .ops import DTYPE16, _cuda_f32, _mask_u8, _ptr, _stream, check_feature_pair, check_reproj_inputs, linspace_table
+from .ops import (DTYPE16, _cuda_f32, _mask_u8, _ptr, _stream, check_feature_pair, check_reproj_inputs, linspace_table,
+                  soft_argmin_backward_into, soft_argmin_forward_into, upsample_soft_argmin_backward_into,
+                  upsample_soft_argmin_forward_into)
 from .ops import concat_volume_backward as concat_volume_backward_into
 from .ops import concat_volume_forward
 
@@ -99,26 +101,25 @@ concat_volume.register_autograd(_concat_backward, setup_context=_concat_setup)
 # ---------------------------------------------------------------------------------------------
 @torch.library.custom_op(f"{NS}::soft_argmin", mutates_args=(), device_types="cuda")
 def soft_argmin_op(cost: Tensor) -> Tuple[Tensor, Tensor]:
-    c = _cuda_f32(cost, "cost")
+    c = _cuda_f32(cost, "cost", allow16=True)
     if c.dim() != 4:
         raise ValueError("az_stereo::soft_argmin: cost must be [B,D,H,W]")
     B, D, H, W = c.shape
     disp = torch.empty((B, 1, H, W), dtype=torch.float32, device=c.device)
     lse = torch.empty((B, 2, H, W), dtype=torch.float32, device=c.device)
-    with torch.cuda.device(c.device):
-        _lib.call("az_soft_argmin_fwd", _ptr(c), _ptr(disp), _ptr(lse), B, D, H, W, _stream(), batch=B)
+    soft_argmin_forward_into(c, disp, lse)
     return disp, lse
 
 
 @soft_argmin_op.register_fake
 def _(cost):
-    B, _, H, W = cost.shape
-    return cost.new_empty((B, 1, H, W)), cost.new_empty((B, 2, H, W))
+    B, _, H, W = cost.shape  # disp and lse are float32 for 16-bit logits too
+    return cost.new_empty((B, 1, H, W), dtype=torch.float32), cost.new_empty((B, 2, H, W), dtype=torch.float32)
 
 
 @torch.library.custom_op(f"{NS}::soft_argmin_backward", mutates_args=(), device_types="cuda")
 def soft_argmin_backward(cost: Tensor, disp: Tensor, lse: Tensor, gdisp: Tensor) -> Tensor:
-    c, g = _cuda_f32(cost, "cost"), _cuda_f32(gdisp, "grad_disp")
+    c, g = _cuda_f32(cost, "cost", allow16=True), _cuda_f32(gdisp, "grad_disp")
     if c.dim() != 4:
         raise ValueError("az_stereo::soft_argmin_backward: cost must be [B,D,H,W]")
     B, D, H, W = c.shape
@@ -126,10 +127,8 @@ def soft_argmin_backward(cost: Tensor, disp: Tensor, lse: Tensor, gdisp: Tensor)
     if tuple(d_.shape) != (B, 1, H, W) or tuple(g.shape) != (B, 1, H, W) or tuple(l_.shape) != (B, 2, H, W) \
             or not (d_.device == l_.device == g.device == c.device):
         raise ValueError("az_stereo::soft_argmin_backward: disp/gdisp [B,1,H,W] and lse [B,2,H,W] on cost's device expected")
-    disp, lse = d_, l_
     gcost = torch.empty_like(c)
-    with torch.cuda.device(c.device):
-        _lib.call("az_soft_argmin_bwd", _ptr(c), _ptr(disp), _ptr(lse), _ptr(g), _ptr(gcost), B, D, H, W, _stream(), batch=B)
+    soft_argmin_backward_into(c, d_, l_, g, gcost)
     return gcost
 
 
@@ -292,7 +291,7 @@ gwc_volume.register_autograd(_gwc_backward, setup_context=_gwc_setup)
 # trilinear upsample + soft-argmin in one kernel (SURVEY.md §8f rank 1)
 # ---------------------------------------------------------------------------------------------
 def _lowres_dims(lowres: Tensor, what: str):
-    c = _cuda_f32(lowres, "lowres")
+    c = _cuda_f32(lowres, "lowres", allow16=True)
     if not (c.dim() == 4 or (c.dim() == 5 and c.shape[1] == 1)):
         raise ValueError(f"{what}: expected [B,1,Dq,Hq,Wq] or [B,Dq,Hq,Wq] low-resolution logits")
     return c, (int(c.shape[0]), int(c.shape[-3]), int(c.shape[-2]), int(c.shape[-1]))
@@ -303,15 +302,14 @@ def upsample_soft_argmin_op(lowres: Tensor, D: int, H: int, W: int) -> Tuple[Ten
     c, (B, Dq, Hq, Wq) = _lowres_dims(lowres, "az_stereo::upsample_soft_argmin")
     disp = torch.empty((B, 1, H, W), dtype=torch.float32, device=c.device)
     stats = torch.empty((B, 2, H, W), dtype=torch.float32, device=c.device)
-    with torch.cuda.device(c.device):
-        _lib.call("az_upsample_soft_argmin_fwd", _ptr(c), _ptr(disp), _ptr(stats), B, Dq, Hq, Wq, D, H, W, _stream(), batch=B)
+    upsample_soft_argmin_forward_into(c, disp, stats, (B, Dq, Hq, Wq, D, H, W))
     return disp, stats
 
 
 @upsample_soft_argmin_op.register_fake
 def _(lowres, D, H, W):
-    B = lowres.shape[0]
-    return lowres.new_empty((B, 1, H, W)), lowres.new_empty((B, 2, H, W))
+    B = lowres.shape[0]  # disp and stats are float32 for 16-bit logits too
+    return lowres.new_empty((B, 1, H, W), dtype=torch.float32), lowres.new_empty((B, 2, H, W), dtype=torch.float32)
 
 
 @torch.library.custom_op(f"{NS}::upsample_soft_argmin_backward", mutates_args=(), device_types="cuda")
@@ -324,11 +322,7 @@ def upsample_soft_argmin_backward(lowres: Tensor, disp: Tensor, stats: Tensor, g
                          "logits' device expected")
     H, W = int(d_.shape[2]), int(d_.shape[3])
     glow = torch.empty_like(c)
-    ws = torch.empty((_lib.query("az_upsample_soft_argmin_workspace_bytes", B, Dq, H, W, Wq),), dtype=torch.uint8,
-                     device=c.device)
-    with torch.cuda.device(c.device):
-        _lib.call("az_upsample_soft_argmin_bwd", _ptr(c), _ptr(d_), _ptr(s_), _ptr(g), _ptr(glow), _ptr(ws),
-                  B, Dq, Hq, Wq, D, H, W, _stream(), batch=B)
+    upsample_soft_argmin_backward_into(c, d_, s_, g, glow, (B, Dq, Hq, Wq, D, H, W))
     return glow
 
 

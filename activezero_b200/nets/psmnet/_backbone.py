@@ -194,8 +194,9 @@ class PSMNetBase(nn.Module):
         key = (conv.weight.data_ptr(), conv.weight._version, str(conv.weight.device), ref_feat.dtype)
         if self._vc_cache is None or self._vc_cache[0] != key:
             self._vc_cache = (key, ops.pack_volume_conv_weight(conv.weight, dtype=ref_feat.dtype))
-        scale = bn.weight.detach() * torch.rsqrt(bn.running_var + bn.eps)
-        shift = bn.bias.detach() - bn.running_mean * scale
+        # the fold is fp32 (the kernel applies it in fp32); a converted 16-bit model's parameters are widened exactly
+        scale = bn.weight.detach().float() * torch.rsqrt(bn.running_var.float() + bn.eps)
+        shift = bn.bias.detach().float() - bn.running_mean.float() * scale
         return ops.volume_conv0(ref_feat, tgt_feat, self._vc_cache[1], self.maxdisp // 4, scale, shift, relu=True)
 
     def _aggregate(self, cost, first=None):

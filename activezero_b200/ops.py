@@ -175,8 +175,8 @@ def pack_volume_conv_weight(weight: torch.Tensor, dtype: torch.dtype = torch.flo
     """Conv3d weight [32,64,3,3,3] (dres0[0][0].weight, psmnet.py:85-90) -> the per-tap core-matrix order of the
     tensor-core kernel, rounded to TF32; do this once per weight tensor.  ``dtype`` = the dtype of the features it
     will be used with: bfloat16 / float16 round each weight to that dtype first (RNE), as torch.autocast rounds the
-    weight of a cuDNN convolution."""
-    w = _cuda_f32(weight.detach(), "weight")
+    weight of a cuDNN convolution.  A bfloat16 / float16 weight (a converted model) is widened exactly first."""
+    w = _cuda_f32(weight.detach(), "weight", allow16=True).float()
     if tuple(w.shape) != (32, 64, 3, 3, 3):
         raise ValueError(f"volume conv: expected a [32,64,3,3,3] Conv3d weight, got {tuple(w.shape)}")
     if dtype != torch.float32 and dtype not in DTYPE16:
@@ -330,22 +330,74 @@ def build_gwc_volume(ref_feat, tgt_feat, num_disp: int, num_groups: int):
 # ----------------------------------------------------------------------------
 # a4/a5 soft-argmin
 # ----------------------------------------------------------------------------
+# The logits may be float32, bfloat16 or float16; disp, lse / stats and gdisp are always float32 and the logits'
+# gradient has the logits' dtype (16 bits: the fp32 gradient rounded once, DESIGN.md §4.12).  Shared by the
+# Functions below and library_ops.
+def soft_argmin_forward_into(c, disp, lse):
+    B, D, H, W = c.shape
+    dt = DTYPE16.get(c.dtype)
+    with torch.cuda.device(c.device):
+        if dt is None:
+            _lib.call("az_soft_argmin_fwd", _ptr(c), _ptr(disp), _ptr(lse), B, D, H, W, _stream(), batch=B)
+        else:
+            _lib.call("az_soft_argmin_fwd_16", _ptr(c), _ptr(disp), _ptr(lse), B, D, H, W, dt, _stream(), batch=B)
+
+
+def soft_argmin_backward_into(c, disp, lse, g, gcost):
+    B, D, H, W = c.shape
+    dt = DTYPE16.get(c.dtype)
+    with torch.cuda.device(c.device):
+        if dt is None:
+            _lib.call("az_soft_argmin_bwd", _ptr(c), _ptr(disp), _ptr(lse), _ptr(g), _ptr(gcost), B, D, H, W, _stream(),
+                      batch=B)
+        else:
+            _lib.call("az_soft_argmin_bwd_16", _ptr(c), _ptr(disp), _ptr(lse), _ptr(g), _ptr(gcost), B, D, H, W, dt,
+                      _stream(), batch=B)
+
+
+def upsample_soft_argmin_forward_into(c, disp, stats, dims):
+    B, Dq, Hq, Wq, D, H, W = dims
+    dt = DTYPE16.get(c.dtype)
+    with torch.cuda.device(c.device):
+        if dt is None:
+            _lib.call("az_upsample_soft_argmin_fwd", _ptr(c), _ptr(disp), _ptr(stats), B, Dq, Hq, Wq, D, H, W, _stream(),
+                      batch=B)
+        else:
+            _lib.call("az_upsample_soft_argmin_fwd_16", _ptr(c), _ptr(disp), _ptr(stats), B, Dq, Hq, Wq, D, H, W, dt,
+                      _stream(), batch=B)
+
+
+def upsample_soft_argmin_backward_into(c, disp, stats, g, glow, dims):
+    B, Dq, Hq, Wq, D, H, W = dims
+    ws = torch.empty((_lib.query("az_upsample_soft_argmin_workspace_bytes", B, Dq, H, W, Wq),), dtype=torch.uint8,
+                     device=c.device)
+    dt = DTYPE16.get(c.dtype)
+    with torch.cuda.device(c.device):
+        if dt is None:
+            _lib.call("az_upsample_soft_argmin_bwd", _ptr(c), _ptr(disp), _ptr(stats), _ptr(g), _ptr(glow), _ptr(ws),
+                      B, Dq, Hq, Wq, D, H, W, _stream(), batch=B)
+        else:
+            _lib.call("az_upsample_soft_argmin_bwd_16", _ptr(c), _ptr(disp), _ptr(stats), _ptr(g), _ptr(glow), _ptr(ws),
+                      B, Dq, Hq, Wq, D, H, W, dt, _stream(), batch=B)
+
+
 class SoftArgminFn(torch.autograd.Function):
     """F.softmax(cost, 1) + DisparityRegression (psmnet.py:200-201,
-    psmnet_submodule.py:80-89) fused; takes LOGITS."""
+    psmnet_submodule.py:80-89) fused; takes LOGITS.  Outside torch.autocast, bfloat16 / float16 logits are read as
+    they are: the disparity is float32 and equal to the float32 operator's on ``cost.float()``, and the gradient has
+    the logits' dtype; inside autocast the logits are cast to float32 as before."""
 
     @staticmethod
     @_fwd32
     def forward(ctx, cost):
-        c = _cuda_f32(cost, "cost")
+        c = _cuda_f32(cost, "cost", allow16=True)
         if c.dim() != 4:
             raise ValueError("soft_argmin: cost must be [B,D,H,W]")
         B, D, H, W = c.shape
         disp = torch.empty((B, 1, H, W), dtype=torch.float32, device=c.device)
         need_bwd = ctx.needs_input_grad[0]
         lse = torch.empty((B, 2, H, W), dtype=torch.float32, device=c.device) if need_bwd else None
-        with torch.cuda.device(c.device):
-            _lib.call("az_soft_argmin_fwd", _ptr(c), _ptr(disp), _ptr(lse), B, D, H, W, _stream(), batch=B)
+        soft_argmin_forward_into(c, disp, lse)
         if need_bwd:
             ctx.save_for_backward(c, disp, lse)
         return disp
@@ -355,28 +407,27 @@ class SoftArgminFn(torch.autograd.Function):
     @_bwd
     def backward(ctx, gdisp):
         c, disp, lse = ctx.saved_tensors
-        B, D, H, W = c.shape
         g = _cuda_f32(gdisp, "grad_disp")
         gcost = torch.empty_like(c)
-        with torch.cuda.device(c.device):
-            _lib.call("az_soft_argmin_bwd", _ptr(c), _ptr(disp), _ptr(lse), _ptr(g), _ptr(gcost), B, D, H, W, _stream(), batch=B)
+        soft_argmin_backward_into(c, disp, lse, g, gcost)
         return gcost
 
 
 def soft_argmin(cost):
-    """[B,D,H,W] logits -> [B,1,H,W] expected disparity."""
+    """[B,D,H,W] logits (float32, bfloat16 or float16) -> [B,1,H,W] float32 expected disparity."""
     return SoftArgminFn.apply(cost)
 
 
 class UpsampleSoftArgminFn(torch.autograd.Function):
     """F.interpolate(cost, (D,H,W), 'trilinear', align_corners=False) -> squeeze ->
     softmax -> DisparityRegression (psmnet.py:186-217) in one kernel that reads the
-    low-resolution logits only (SURVEY.md §8f rank 1)."""
+    low-resolution logits only (SURVEY.md §8f rank 1).  bfloat16 / float16 logits outside torch.autocast: as in
+    SoftArgminFn, a float32 disparity and a gradient of the logits' dtype."""
 
     @staticmethod
     @_fwd32
     def forward(ctx, lowres, out_size):
-        c = _cuda_f32(lowres, "lowres")
+        c = _cuda_f32(lowres, "lowres", allow16=True)
         if c.dim() == 5:
             if c.shape[1] != 1:
                 raise ValueError("upsample_soft_argmin: expected [B,1,Dq,Hq,Wq]")
@@ -387,11 +438,10 @@ class UpsampleSoftArgminFn(torch.autograd.Function):
         disp = torch.empty((B, 1, H, W), dtype=torch.float32, device=c.device)
         need_bwd = ctx.needs_input_grad[0]
         stats = torch.empty((B, 2, H, W), dtype=torch.float32, device=c.device) if need_bwd else None
-        with torch.cuda.device(c.device):
-            _lib.call("az_upsample_soft_argmin_fwd", _ptr(c), _ptr(disp), _ptr(stats), B, Dq, Hq, Wq, D, H, W, _stream(), batch=B)
+        ctx.dims = (B, Dq, Hq, Wq, D, H, W)
+        upsample_soft_argmin_forward_into(c, disp, stats, ctx.dims)
         if need_bwd:
             ctx.save_for_backward(c, disp, stats)
-        ctx.dims = (B, Dq, Hq, Wq, D, H, W)
         return disp
 
     @staticmethod
@@ -399,19 +449,15 @@ class UpsampleSoftArgminFn(torch.autograd.Function):
     @_bwd
     def backward(ctx, gdisp):
         c, disp, stats = ctx.saved_tensors
-        B, Dq, Hq, Wq, D, H, W = ctx.dims
         g = _cuda_f32(gdisp, "grad_disp")
         glow = torch.empty_like(c)
-        ws = torch.empty((_lib.query("az_upsample_soft_argmin_workspace_bytes", B, Dq, H, W, Wq),), dtype=torch.uint8,
-                         device=c.device)
-        with torch.cuda.device(c.device):
-            _lib.call("az_upsample_soft_argmin_bwd", _ptr(c), _ptr(disp), _ptr(stats), _ptr(g), _ptr(glow), _ptr(ws),
-                      B, Dq, Hq, Wq, D, H, W, _stream(), batch=B)
+        upsample_soft_argmin_backward_into(c, disp, stats, g, glow, ctx.dims)
         return glow, None
 
 
 def upsample_soft_argmin(lowres, out_size):
-    """[B,1,Dq,Hq,Wq] low-res logits -> [B,1,H,W] disparity for out_size = (D,H,W)."""
+    """[B,1,Dq,Hq,Wq] low-res logits (float32, bfloat16 or float16) -> [B,1,H,W] float32 disparity for
+    out_size = (D,H,W)."""
     return UpsampleSoftArgminFn.apply(lowres, tuple(out_size))
 
 

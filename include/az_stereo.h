@@ -126,6 +126,19 @@ int az_soft_argmin_fwd(const float* cost, float* disp, float* lse,
 /* gcost[b,d,y,x] = softmax_d * (d - disp) * gdisp[b,0,y,x], softmax_d = 2^((cost_d - m)*log2(e) - log2sum) */
 int az_soft_argmin_bwd(const float* cost, const float* disp, const float* lse, const float* gdisp, float* gcost,
                        int64_t B, int64_t D, int64_t H, int64_t W, void* stream);
+/* The same operator with 16-bit logits: cost and gcost are bf16 or fp16 (dtype AZ_DTYPE_BF16 or AZ_DTYPE_F16, else
+ * AZ_ERR_BAD_ARG); disp, lse and gdisp stay float32.
+ * Forward: each logit is widened exactly (both formats fit inside fp32) and goes through the fp32 kernels' arithmetic
+ *   unchanged, the kernel picked by the fp32 rule on the shape alone (H*W % 4 == 0 or not), never by the alignment of
+ *   cost: disp and lse equal az_soft_argmin_fwd on cost.float() (a fresh, aligned tensor), bit for bit, for any
+ *   element offset of cost.  disp stays fp32 on purpose (a bf16 disparity has a spacing of 0.5 px above 128 px).
+ * Backward: the gradient is formed in fp32 exactly as az_soft_argmin_bwd forms it and rounded ONCE, to nearest even:
+ *   gcost = RNE16(az_soft_argmin_bwd(cost.float(), ...)), bit for bit.
+ * The AZ_SA_FWD developer knob applies to the fp32 entry point only. */
+int az_soft_argmin_fwd_16(const void* cost, float* disp, float* lse,
+                          int64_t B, int64_t D, int64_t H, int64_t W, int dtype, void* stream);
+int az_soft_argmin_bwd_16(const void* cost, const float* disp, const float* lse, const float* gdisp, void* gcost,
+                          int64_t B, int64_t D, int64_t H, int64_t W, int dtype, void* stream);
 
 /* ---- SURVEY.md §8f rank 1: trilinear upsample fused into soft-argmin --
  *      nets/psmnet/psmnet.py:186-197,208-211 (F.interpolate(cost,(D,4H,4W),'trilinear',align_corners=False))
@@ -141,6 +154,17 @@ int64_t az_upsample_soft_argmin_workspace_bytes(int64_t B, int64_t Dq, int64_t H
 int az_upsample_soft_argmin_bwd(const float* lowres, const float* disp, const float* stats, const float* gdisp,
                                 float* glow, void* workspace, int64_t B, int64_t Dq, int64_t Hq, int64_t Wq,
                                 int64_t D, int64_t H, int64_t W, void* stream);
+/* The same operator with 16-bit low-resolution logits: lowres and glow are bf16 or fp16 (dtype AZ_DTYPE_BF16 or
+ * AZ_DTYPE_F16, else AZ_ERR_BAD_ARG); disp, stats, gdisp and the workspace (same size, fp32 planes) stay float32.
+ * The logits are widened exactly when they are staged, and every instruction after that, the kernel selection included
+ * (as at the AZ_USA_FWD default), is the fp32 operator's: disp and stats equal az_upsample_soft_argmin_fwd on
+ * lowres.float(), and glow = RNE16(az_upsample_soft_argmin_bwd(lowres.float(), ...)), bit for bit (the fp32 sums of
+ * the last reduction are rounded once, to nearest even, at the store). */
+int az_upsample_soft_argmin_fwd_16(const void* lowres, float* disp, float* stats, int64_t B, int64_t Dq, int64_t Hq,
+                                   int64_t Wq, int64_t D, int64_t H, int64_t W, int dtype, void* stream);
+int az_upsample_soft_argmin_bwd_16(const void* lowres, const float* disp, const float* stats, const float* gdisp,
+                                   void* glow, void* workspace, int64_t B, int64_t Dq, int64_t Hq, int64_t Wq,
+                                   int64_t D, int64_t H, int64_t W, int dtype, void* stream);
 
 /* ---- a6: bilinear disparity warp -- utils/reprojection.py:13-35 (apply_disparity) ----
  * out[b,c,i,j] = bilinear2D(img[b,c]; xs, ys), zeros padding, align_corners=False, with the reference's
