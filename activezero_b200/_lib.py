@@ -40,6 +40,7 @@ SIGNATURES = {
     "az_volume_conv0_fwd_16": (ctypes.c_int, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, ctypes.c_int, ctypes.c_int, _P]),
     "az_volume_conv0_bwd_workspace_bytes": (_I, [_I, _I, _I, _I]),
     "az_volume_conv0_bwd": (ctypes.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
+    "az_volume_conv0_bwd_16": (ctypes.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, ctypes.c_int, ctypes.c_int, _P]),
     "az_gwc_volume_fwd": (ctypes.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "az_gwc_volume_bwd": (ctypes.c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "az_soft_argmin_fwd": (ctypes.c_int, [_P, _P, _P, _I, _I, _I, _I, _P]),
@@ -71,7 +72,7 @@ SIGNATURES = {
 }
 
 # CUDA kernels enqueued by one successful call of each compute entry point
-KERNELS_PER_CALL = {"az_reproj_loss_fwd": 2, "az_warp_bwd": 2, "az_bilinear_rescale_fwd": 1, "az_temporal_ir": 3, "az_upsample_soft_argmin_bwd": 3, "az_upsample_soft_argmin_bwd_16": 3, "az_error_metrics": 2, "az_sim_ir_pattern": 4, "az_volume_conv0_bwd": 4}
+KERNELS_PER_CALL = {"az_reproj_loss_fwd": 2, "az_warp_bwd": 2, "az_bilinear_rescale_fwd": 1, "az_temporal_ir": 3, "az_upsample_soft_argmin_bwd": 3, "az_upsample_soft_argmin_bwd_16": 3, "az_error_metrics": 2, "az_sim_ir_pattern": 4, "az_volume_conv0_bwd": 4, "az_volume_conv0_bwd_16": 4}
 
 _lib = None
 launch_count = 0    # C-ABI compute calls issued

@@ -3,6 +3,9 @@
     torch.ops.az_stereo.volume_conv(ref, tgt, weight, num_disp) -> out                     (psmnet.py:151-168)
     torch.ops.az_stereo.volume_conv_backward(gout, ref, tgt, weight) -> (gref, gtgt, gweight)
 
+Both take the dtypes ``ops.volume_conv`` takes (float32, or bfloat16 / float16 features with a float32 weight or one
+of their dtype); the fake kernels follow ``ref`` and ``weight`` for the dtypes of the results.
+
 ``library_ops`` imports this module, so importing ``library_ops`` registers both operators.  They live in a module of
 their own so that the operator set defined in ``library_ops`` itself (pinned by tests/test_library_ops_fake.py) stays
 the inference / loss path's.
@@ -14,8 +17,7 @@ from typing import Tuple
 import torch
 from torch import Tensor
 
-from . import _lib
-from .ops import _NULL, _cuda_f32, _ptr, _stream, check_volume_conv_inputs, pack_volume_conv_weight, volume_conv_backward_into
+from .ops import _cuda_f32, check_volume_conv_inputs, volume_conv_backward_into, volume_conv_forward
 
 NS = "az_stereo"
 
@@ -23,14 +25,7 @@ NS = "az_stereo"
 @torch.library.custom_op(f"{NS}::volume_conv", mutates_args=(), device_types="cuda")
 def volume_conv(ref: Tensor, tgt: Tensor, weight: Tensor, num_disp: int) -> Tensor:
     L, R, w = check_volume_conv_inputs(ref, tgt, weight, num_disp, "az_stereo::volume_conv")
-    B, C, H, W = L.shape
-    out = torch.empty((B, 32, num_disp, H, W), dtype=torch.float32, device=L.device)
-    if B > 0:
-        wp = pack_volume_conv_weight(w)
-        with torch.cuda.device(L.device):
-            _lib.call("az_volume_conv0_fwd", _ptr(L), _ptr(R), _ptr(wp), _NULL, _NULL, _ptr(out), B, C, H, W, num_disp, 0,
-                      _stream(), batch=B)
-    return out
+    return volume_conv_forward(L, R, w, num_disp)
 
 
 @volume_conv.register_fake
@@ -41,7 +36,7 @@ def _(ref, tgt, weight, num_disp):
 
 @torch.library.custom_op(f"{NS}::volume_conv_backward", mutates_args=(), device_types="cuda")
 def volume_conv_backward(gout: Tensor, ref: Tensor, tgt: Tensor, weight: Tensor) -> Tuple[Tensor, Tensor, Tensor]:
-    g = _cuda_f32(gout, "grad_out")
+    g = _cuda_f32(gout, "grad_out", allow16=True)
     if g.dim() != 5:
         raise ValueError("az_stereo::volume_conv_backward: gout must be [B,32,Dq,H,W]")
     L, R, w = check_volume_conv_inputs(ref, tgt, weight, int(g.shape[2]), "az_stereo::volume_conv_backward")

@@ -147,6 +147,13 @@ class PSMNetBase(nn.Module):
         # on the implicit volume too (ops.volume_conv: tcgen05 TF32 forward, volume-free fp32 backward); its BatchNorm3d
         # (in the module's own mode) and ReLU stay in torch.  Neither the volume nor its gradient is materialised.
         self.fuse_volume_conv_train = False
+        # True: the same training convolution in the features' 16-bit dtype where they have one, so that the
+        # convolution's output, its BatchNorm and their gradients stay 16-bit as on the unfused path: under torch.autocast
+        # (features of the autocast dtype; autocast is switched off around the call as for the concat volume) and in a
+        # model converted with .to(torch.bfloat16) / .half() (DESIGN.md §4.13).  With fp32 features it is
+        # fuse_volume_conv_train.  It changes results under autocast (the flag above keeps an fp32 convolution there),
+        # hence a flag of its own; when both are set, this one applies.
+        self.fuse_volume_conv_train16 = False
         self._vc_cache = None
         self.feature_extraction = feature_extraction
         self.dres0 = nn.Sequential(convbn_3d(64, 32, 3, 1, 1), nn.ReLU(inplace=True),
@@ -250,9 +257,17 @@ class PSMNetBase(nn.Module):
                 first = first.contiguous(memory_format=torch.channels_last_3d)
             _, _, cost3 = self._aggregate(None, first)
             return self._disparity_head(cost3, H, W)
-        if self.fuse_volume_conv_train and torch.is_grad_enabled():
+        if (self.fuse_volume_conv_train or self.fuse_volume_conv_train16) and torch.is_grad_enabled():
             # dres0[0] = Conv3d + BatchNorm3d, dres0[1] = ReLU
-            conv = ops.volume_conv(ref_feat, tgt_feat, self.dres0[0][0].weight, self.maxdisp // 4)
+            weight = self.dres0[0][0].weight
+            if self.fuse_volume_conv_train16:
+                with self._native16(ref_feat, tgt_feat):
+                    conv = ops.volume_conv(ref_feat, tgt_feat, weight, self.maxdisp // 4)
+            else:
+                if ref_feat.dtype in (torch.bfloat16, torch.float16) and not torch.is_autocast_enabled("cuda"):
+                    raise ValueError("fuse_volume_conv_train computes in float32 only; a 16-bit model trains through the "
+                                     "implicit first convolution with fuse_volume_conv_train16")
+                conv = ops.volume_conv(ref_feat, tgt_feat, weight, self.maxdisp // 4)
             first = self.dres0[1](self.dres0[0][1](conv))
             if self.volume_channels_last:
                 first = first.contiguous(memory_format=torch.channels_last_3d)

@@ -221,11 +221,14 @@ def volume_conv0(ref_feat, tgt_feat, wpacked, num_disp: int, scale=None, shift=N
 
 
 def check_volume_conv_inputs(ref_feat, tgt_feat, weight, num_disp: int, what: str):
-    """Shared by ops and library_ops: features CUDA float32 [B,32,H,W], weight [32,64,3,3,3] on their device."""
-    L, R = check_feature_pair(ref_feat, tgt_feat, what)
+    """Shared by ops and library_ops: features CUDA [B,32,H,W], both float32 or both bfloat16 / both float16; weight
+    [32,64,3,3,3] on their device, float32 or the features' dtype."""
+    L, R = check_feature_pair(ref_feat, tgt_feat, what, allow16=True)
     if L.shape[1] != 32:
         raise ValueError(f"{what}: PSMNet's 32 feature channels expected, got {L.shape[1]}")
-    w = _cuda_f32(weight, "weight")
+    w = _cuda_f32(weight, "weight", allow16=True)
+    if w.dtype not in (torch.float32, L.dtype):
+        raise ValueError(f"{what}: a {w.dtype} weight with {L.dtype} features (float32 or {L.dtype} expected)")
     if tuple(w.shape) != (32, 64, 3, 3, 3) or w.device != L.device:
         raise ValueError(f"{what}: expected a [32,64,3,3,3] Conv3d weight on the features' device, got {tuple(w.shape)}")
     if int(num_disp) <= 0:
@@ -233,10 +236,33 @@ def check_volume_conv_inputs(ref_feat, tgt_feat, weight, num_disp: int, what: st
     return L, R, w
 
 
-def volume_conv_backward_into(gout, L, R, w, gL, gR, gW):
-    """Enqueues az_volume_conv0_bwd for the validated tensors; gL / gR / gW may each be None (skipped)."""
+def volume_conv_forward(L, R, w, num_disp: int):
+    """The raw convolution (no fold, no ReLU) of validated tensors; the output has the features' dtype.  Shared by
+    VolumeConv0Fn and library_ops."""
     B, C, H, W = L.shape
-    Dq = gout.shape[2]
+    out = torch.empty((B, 32, int(num_disp), H, W), dtype=L.dtype, device=L.device)
+    if B > 0:
+        dt = DTYPE16.get(L.dtype)
+        wp = pack_volume_conv_weight(w, dtype=L.dtype)
+        with torch.cuda.device(L.device):
+            if dt is None:
+                _lib.call("az_volume_conv0_fwd", _ptr(L), _ptr(R), _ptr(wp), _NULL, _NULL, _ptr(out), B, C, H, W,
+                          int(num_disp), 0, _stream(), batch=B)
+            else:
+                _lib.call("az_volume_conv0_fwd_16", _ptr(L), _ptr(R), _ptr(wp), _NULL, _NULL, _ptr(out), B, C, H, W,
+                          int(num_disp), 0, dt, _stream(), batch=B)
+    return out
+
+
+def volume_conv_backward_into(gout, L, R, w, gL, gR, gW):
+    """Enqueues az_volume_conv0_bwd (float32 features) or az_volume_conv0_bwd_16 (16-bit features) for the validated
+    tensors; gL / gR / gW may each be None (skipped).  gout must have the features' dtype."""
+    B, C, H, W = L.shape
+    if not isinstance(gout, torch.Tensor) or not gout.is_cuda or gout.dtype != L.dtype:
+        raise ValueError(f"volume conv backward: grad_out must be a {L.dtype} CUDA tensor, got "
+                         f"{getattr(gout, 'dtype', type(gout))}")
+    gout = gout.contiguous()
+    Dq = gout.shape[2] if gout.dim() == 5 else -1
     if tuple(gout.shape) != (B, 32, Dq, H, W) or gout.device != L.device:
         raise ValueError(f"volume conv backward: grad_out must be [B,32,Dq,H,W] = {(B, 32, Dq, H, W)} on the features' "
                          f"device, got {tuple(gout.shape)}")
@@ -245,28 +271,30 @@ def volume_conv_backward_into(gout, L, R, w, gL, gR, gW):
             gW.zero_()  # a sum over no position
         return
     ws = torch.empty((_lib.query("az_volume_conv0_bwd_workspace_bytes", B, H, W, Dq),), dtype=torch.uint8, device=L.device)
+    dt = DTYPE16.get(L.dtype)
     with torch.cuda.device(L.device):
-        _lib.call("az_volume_conv0_bwd", _ptr(gout), _ptr(L), _ptr(R), _ptr(w), _ptr(gL), _ptr(gR), _ptr(gW), _ptr(ws),
-                  B, C, H, W, Dq, _stream(), batch=B)
+        if dt is None:
+            _lib.call("az_volume_conv0_bwd", _ptr(gout), _ptr(L), _ptr(R), _ptr(w), _ptr(gL), _ptr(gR), _ptr(gW),
+                      _ptr(ws), B, C, H, W, Dq, _stream(), batch=B)
+        else:
+            _lib.call("az_volume_conv0_bwd_16", _ptr(gout), _ptr(L), _ptr(R), _ptr(w), _ptr(gL), _ptr(gR), _ptr(gW),
+                      _ptr(ws), B, C, H, W, Dq, dt, 0 if w.dtype == torch.float32 else dt, _stream(), batch=B)
 
 
 class VolumeConv0Fn(torch.autograd.Function):
     """conv3d(concat_volume(ref, tgt, num_disp), weight, padding=1) -- dres0[0][0] on the implicit volume
     (psmnet.py:151-168) -- differentiable in all three inputs.  Forward: the tcgen05 kernel (TF32 operands, fp32
-    accumulation).  Backward: the volume-free fp32 kernels of csrc/volume_conv_bwd.cu.  Saves the features and the
-    weight only (feature-sized, not volume-sized)."""
+    accumulation).  Backward: the volume-free kernels of csrc/volume_conv_bwd.cu (fp32 arithmetic).  Saves the features
+    and the weight only (feature-sized, not volume-sized).  Outside torch.autocast, two bfloat16 (or two float16)
+    features with a float32 weight or one of their dtype give an output and feature gradients of their dtype and a
+    weight gradient of the weight's dtype, equal to the float32 op on the widened features and the weight rounded to
+    their dtype, followed by .to(dtype) (DESIGN.md §4.13); inside autocast the inputs are cast to float32 as before."""
 
     @staticmethod
     @_fwd32
     def forward(ctx, ref_feat, tgt_feat, weight, num_disp: int):
         L, R, w = check_volume_conv_inputs(ref_feat, tgt_feat, weight, num_disp, "volume conv")
-        B, C, H, W = L.shape
-        out = torch.empty((B, 32, int(num_disp), H, W), dtype=torch.float32, device=L.device)
-        if B > 0:
-            wp = pack_volume_conv_weight(w)
-            with torch.cuda.device(L.device):
-                _lib.call("az_volume_conv0_fwd", _ptr(L), _ptr(R), _ptr(wp), _NULL, _NULL, _ptr(out), B, C, H, W,
-                          int(num_disp), 0, _stream(), batch=B)
+        out = volume_conv_forward(L, R, w, num_disp)
         ctx.save_for_backward(L, R, w)
         return out
 
@@ -275,7 +303,7 @@ class VolumeConv0Fn(torch.autograd.Function):
     @_bwd
     def backward(ctx, gout):
         L, R, w = ctx.saved_tensors
-        g = _cuda_f32(gout, "grad_out")
+        g = gout
         gL = torch.empty_like(L) if ctx.needs_input_grad[0] else None
         gR = torch.empty_like(R) if ctx.needs_input_grad[1] else None
         gW = torch.empty_like(w) if ctx.needs_input_grad[2] else None
@@ -286,7 +314,8 @@ class VolumeConv0Fn(torch.autograd.Function):
 def volume_conv(ref_feat, tgt_feat, weight, num_disp: int):
     """[B,32,H,W] x2, Conv3d weight [32,64,3,3,3] -> conv3d(concat_volume(ref, tgt, num_disp), weight, padding=1),
     [B,32,num_disp,H,W], with autograd; the concat volume and its gradient are never materialised.  The raw
-    convolution: no BatchNorm fold, no ReLU (``volume_conv0`` is the inference form with both)."""
+    convolution: no BatchNorm fold, no ReLU (``volume_conv0`` is the inference form with both).  Outside
+    torch.autocast it also takes two bfloat16 or two float16 features, with a float32 weight or one of their dtype."""
     return VolumeConv0Fn.apply(ref_feat, tgt_feat, weight, num_disp)
 
 

@@ -115,6 +115,8 @@ def main():
                     help="use the fused trilinear-upsample + soft-argmin kernel for the three heads (SURVEY §8f-1)")
     ap.add_argument("--fuse-volume-conv", action="store_true",
                     help="dres0's first Conv3d on the implicit volume in training too (PSMNet.fuse_volume_conv_train)")
+    ap.add_argument("--fuse-volume-conv16", action="store_true",
+                    help="the same in the features' 16-bit dtype under --autocast (PSMNet.fuse_volume_conv_train16)")
     ap.add_argument("--profile", action="store_true", help="after the timed region: kernel-time shares via torch.profiler")
     ap.add_argument("--autocast", choices=("bf16", "fp16"), default=None,
                     help="forward passes under torch.autocast with this dtype (timing only: no GradScaler for fp16)")
@@ -133,6 +135,7 @@ def main():
     model = PSMNet(maxdisp=MAX_DISP).to(dev)
     model.fuse_upsample = args.fuse_upsample
     model.fuse_volume_conv_train = args.fuse_volume_conv
+    model.fuse_volume_conv_train16 = args.fuse_volume_conv16
     if args.channels_last_3d:
         model.use_channels_last_3d(True)
     if world > 1:
@@ -204,6 +207,7 @@ def main():
             "config": {"workload": f"config{'3' if args.no_real else '4'}: PSMNet_3 train step {args.height}x{args.width}, "
                                    f"D={MAX_DISP}, batch {args.batch}/GPU, patch reproj ps={PATCH}, T={args.frames}",
                        "ddp": world > 1, "fuse_upsample": args.fuse_upsample, "fuse_volume_conv": args.fuse_volume_conv,
+                       "fuse_volume_conv16": args.fuse_volume_conv16,
                        "channels_last_3d": args.channels_last_3d, "autocast": args.autocast},
             "device_time_shares_rank0": shares,
             "final_loss": float(last)}), flush=True)

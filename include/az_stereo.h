@@ -107,6 +107,19 @@ int64_t az_volume_conv0_bwd_workspace_bytes(int64_t B, int64_t H, int64_t W, int
 int az_volume_conv0_bwd(const float* gout, const float* L, const float* R, const float* weight,
                         float* gL, float* gR, float* gW, void* workspace,
                         int64_t B, int64_t C, int64_t H, int64_t W, int64_t Dq, void* stream);
+/* The same backward with 16-bit tensors (dtype AZ_DTYPE_BF16 or AZ_DTYPE_F16): gout, L, R, gL and gR have that dtype.
+ * weight_dtype is 0 (weight and gW are float32: autocast's fp32 master weight) or equal to dtype (weight and gW have
+ * that dtype: a converted model); any other code, or C != 32, gives AZ_ERR_BAD_ARG.  Each 16-bit value is widened
+ * exactly where it is read; an fp32 weight is rounded to dtype (RNE) before dfeat uses it, as az_volume_conv0_pack_16
+ * and autocast round it.  The workspace (same size, fp32 planes and partials), every accumulator and every summation
+ * order are az_volume_conv0_bwd's, and each 16-bit result is rounded ONCE, to nearest even, at its store:
+ *   gL, gR = az_volume_conv0_bwd(gout.float(), L.float(), R.float(), w16.float()).to(dtype)   (w16 = weight rounded to dtype)
+ *   gW     = az_volume_conv0_bwd(...)'s gW (which does not depend on the weight), .to(dtype) when weight_dtype == dtype
+ * bit for bit.  fp16 results too large for the format become +-inf, as .to(torch.float16) makes them. */
+int az_volume_conv0_bwd_16(const void* gout, const void* L, const void* R, const void* weight,
+                           void* gL, void* gR, void* gW, void* workspace,
+                           int64_t B, int64_t C, int64_t H, int64_t W, int64_t Dq,
+                           int dtype, int weight_dtype, void* stream);
 
 /* ---- a3: group-wise correlation volume -- NOT IN THE REFERENCE (SURVEY.md fact 1; parity unpinned) ----
  * vol[b,g,i,y,x] = (1/(C/G)) * sum_{c in group g} L[b,c,y,x]*R[b,c,y,x-i]  (x >= i, else 0); vol: [B,G,Dq,H,W]. */
