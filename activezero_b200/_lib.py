@@ -57,6 +57,7 @@ SIGNATURES = {
     "az_reproj_workspace_bytes": (_I, [_I, _I]),
     "az_reproj_loss_fwd": (ctypes.c_int, [_P, _P, _P, _F, _P, _P, _P, _I, _P, _P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "az_reproj_loss_bwd": (ctypes.c_int, [_P, _P, _P, _F, _P, _I, _I, _I, _I, _I, _P]),
+    "az_reproj_loss_img_bwd": (ctypes.c_int, [_P, _P, _P, _F, _P, _P, _P, _I, _P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "az_patch_fold": (ctypes.c_int, [_P, _P, _F, _P, _P, _I, _P, _I, _I, _I, _I, _P]),
     "az_bilinear_rescale_fwd": (ctypes.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _F, _F, _F, _P]),
     "az_bilinear_rescale_bwd": (ctypes.c_int, [_P, _P, _I, _I, _I, _I, _I, _F, _F, _F, _P]),

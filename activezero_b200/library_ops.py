@@ -23,6 +23,11 @@ registers the differentiable first aggregation convolution on the implicit volum
 
     torch.ops.az_stereo.volume_conv(ref, tgt, weight, num_disp) -> out               (psmnet.py:151-168)
 
+and the image gradients of the reprojection loss (``_reproj_image_library``), which ``reproj_loss``'s autograd
+formula calls when ``tgt`` or ``src`` requires grad:
+
+    torch.ops.az_stereo.reproj_loss_image_backward(tgt, src, disp, mask, stats, gloss, sign, ps) -> (gtgt, gsrc)
+
 The convenience wrappers below return what the reference-named functions return.  Nothing here computes on the
 host: every implementation enqueues the CUDA kernels of ``libaz_stereo.so`` (no CPU fallback).
 """
@@ -33,7 +38,7 @@ from typing import Tuple
 import torch
 from torch import Tensor
 
-from . import _lib, _volume_conv_library
+from . import _lib, _reproj_image_library, _volume_conv_library
 from .ops import (DTYPE16, _cuda_f32, _mask_u8, _ptr, _stream, check_feature_pair, check_reproj_inputs, linspace_table,
                   soft_argmin_backward_into, soft_argmin_forward_into, upsample_soft_argmin_backward_into,
                   upsample_soft_argmin_forward_into)
@@ -207,14 +212,22 @@ def _(gpre, stats, gloss, sign, C, ps):
 
 
 def _rl_setup(ctx, inputs, output):
-    ctx.save_for_backward(output[2], output[3])
+    # the images (and the mask) are kept only when an image gradient will be asked for
+    need_img = ctx.needs_input_grad[0] or ctx.needs_input_grad[1]
+    ctx.save_for_backward(output[2], output[3], *(inputs[:4] if need_img else (None,) * 4))
     ctx.meta = (inputs[0].shape[1], int(inputs[4]), float(inputs[5]))
 
 
 def _rl_backward(ctx, gloss, _gw, _gp, _gs):
-    gpre, stats = ctx.saved_tensors
+    gpre, stats, tgt, src, disp, mask = ctx.saved_tensors
     C, ps, sign = ctx.meta
-    return None, None, reproj_loss_backward(gpre, stats, gloss, sign, C, ps), None, None, None
+    gdisp = reproj_loss_backward(gpre, stats, gloss, sign, C, ps) if ctx.needs_input_grad[2] else None
+    gtgt = gsrc = None
+    if ctx.needs_input_grad[0] or ctx.needs_input_grad[1]:
+        gtgt, gsrc = _reproj_image_library.reproj_loss_image_backward(tgt, src, disp, mask, stats, gloss, sign, ps)
+        gtgt = gtgt if ctx.needs_input_grad[0] else None
+        gsrc = gsrc if ctx.needs_input_grad[1] else None
+    return gtgt, gsrc, gdisp, None, None, None
 
 
 reproj_loss_op.register_autograd(_rl_backward, setup_context=_rl_setup)
@@ -222,9 +235,7 @@ reproj_loss_op.register_autograd(_rl_backward, setup_context=_rl_setup)
 
 def reproj_loss(tgt: Tensor, src: Tensor, disp: Tensor, mask: Tensor, ps: int = 1, sign: float = -1.0):
     """-> (loss, warped): masked MSE between ``tgt`` and ``apply_disparity(unfold(src), sign*disp)`` and the warped
-    image (ps = 1) / Fold image (ps > 1); differentiable w.r.t. ``disp``."""
-    if tgt.requires_grad or src.requires_grad:
-        raise ValueError("az_stereo::reproj_loss is differentiable w.r.t. disp only; use ops.warp() for image gradients")
+    image (ps = 1) / Fold image (ps > 1); differentiable w.r.t. ``disp``, ``tgt`` and ``src``."""
     loss, warped, _, _ = reproj_loss_op(tgt, src, disp, mask, ps, sign)
     return loss, warped
 

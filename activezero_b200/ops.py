@@ -547,10 +547,21 @@ def _mask_u8(mask: Optional[torch.Tensor], like: torch.Tensor) -> Optional[torch
     return m.contiguous().view(torch.uint8)
 
 
+def reproj_image_backward_into(t, s, d, mask_u8, stats, gl, sign: float, ps: int, gtgt, gsrc):
+    """Enqueues the image gradients of the reprojection loss of validated inputs (include/az_stereo.h:
+    az_reproj_loss_img_bwd): ``gtgt`` / ``gsrc`` (either may be None) are fully written, deterministically."""
+    B, C, H, W = t.shape
+    lx, ly = linspace_table(W, t.device), linspace_table(H, t.device)
+    with torch.cuda.device(t.device):
+        _lib.call("az_reproj_loss_img_bwd", _ptr(t), _ptr(s), _ptr(d), float(sign), _ptr(mask_u8), _ptr(lx), _ptr(ly),
+                  int(ps), _ptr(stats), _ptr(gl), _ptr(gtgt), _ptr(gsrc), B, C, H, W, _stream(), batch=B)
+
+
 class ReprojLossFn(torch.autograd.Function):
     """Masked MSE between ``tgt`` and ``apply_disparity(unfold(src), sign*disp)``
     (reprojection.py:81-96 for ps = 1, :99-118 for the patch loss).  Differentiable
-    w.r.t. ``disp`` only (what the trainer needs: the images are data)."""
+    w.r.t. ``disp``, ``tgt`` and ``src`` (the image gradients are recomputed from the
+    inputs, without the unfolded planes; DESIGN.md §4.14)."""
 
     @staticmethod
     @_fwd32
@@ -564,6 +575,7 @@ class ReprojLossFn(torch.autograd.Function):
         B, C, H, W = t.shape
         dev = t.device
         need_bwd = ctx.needs_input_grad[2]
+        need_img = ctx.needs_input_grad[0] or ctx.needs_input_grad[1]
         warped = torch.empty_like(t) if want_warped else None
         gpre = torch.empty_like(d) if need_bwd else None
         loss = torch.empty((1,), dtype=torch.float32, device=dev)
@@ -576,8 +588,8 @@ class ReprojLossFn(torch.autograd.Function):
         if B == 0:  # F.mse_loss of nothing (reprojection.py:118 on an empty batch) is NaN
             loss.fill_(float("nan"))
             stats.zero_()
-        if need_bwd:
-            ctx.save_for_backward(gpre, stats)
+        if need_bwd or need_img:
+            ctx.save_for_backward(gpre, stats, *((t, s, d, mask_u8) if need_img else (None,) * 4))
         ctx.meta = (B, C, H, W, int(ps), float(sign))
         if warped is not None:
             ctx.mark_non_differentiable(warped)
@@ -587,21 +599,27 @@ class ReprojLossFn(torch.autograd.Function):
     @once_differentiable
     @_bwd
     def backward(ctx, gloss, _gwarped):
-        gpre, stats = ctx.saved_tensors
+        gpre, stats, t, s, d, mask_u8 = ctx.saved_tensors
         B, C, H, W, ps, sign = ctx.meta
         gl = gloss.reshape(1).to(torch.float32).contiguous()
-        gdisp = torch.empty_like(gpre)
-        with torch.cuda.device(gpre.device):
-            _lib.call("az_reproj_loss_bwd", _ptr(gpre), _ptr(stats), _ptr(gl), sign, _ptr(gdisp), B, C, H, W, ps,
-                      _stream(), batch=B)
-        return None, None, gdisp, None, None, None, None
+        gdisp = gtgt = gsrc = None
+        if ctx.needs_input_grad[2]:
+            gdisp = torch.empty_like(gpre)
+            with torch.cuda.device(gpre.device):
+                _lib.call("az_reproj_loss_bwd", _ptr(gpre), _ptr(stats), _ptr(gl), sign, _ptr(gdisp), B, C, H, W, ps,
+                          _stream(), batch=B)
+        if ctx.needs_input_grad[0] or ctx.needs_input_grad[1]:
+            gtgt = torch.empty_like(t) if ctx.needs_input_grad[0] else None  # fully written by the kernels
+            gsrc = torch.empty_like(s) if ctx.needs_input_grad[1] else None
+            reproj_image_backward_into(t, s, d, mask_u8, stats, gl, sign, ps, gtgt, gsrc)
+        return gtgt, gsrc, gdisp, None, None, None, None
 
 
 def reproj_loss(tgt, src, disp, mask=None, ps: int = 1, sign: float = -1.0, want_warped: bool = False):
     """-> (loss 0-dim, warped [B,C,H,W] or None).  ``warped`` is the warped image for ps == 1 and
-    the Fold visualisation image of get_reproj_error_patch for ps > 1 (same pass as the loss)."""
-    if tgt.requires_grad or src.requires_grad:
-        raise ValueError("reproj_loss is differentiable w.r.t. disp only; use warp() for image gradients")
+    the Fold visualisation image of get_reproj_error_patch for ps > 1 (same pass as the loss).
+    Differentiable w.r.t. ``disp``, ``tgt`` and ``src`` (``warped`` is not differentiable).  The image
+    gradients are deterministic; with an empty mask they are exactly zero (the loss is NaN)."""
     return ReprojLossFn.apply(tgt, src, disp, _mask_u8(mask, tgt), ps, sign, want_warped)
 
 

@@ -62,29 +62,17 @@ def get_reprojection_error_old(input_L, input_R, pred_disp_l, mask=None):
     return loss, warped, _int_mask(mask, input_L)
 
 
-def _patch_loss_autograd(input_L, input_R, pred_disp_l, mask, ps):
-    """reprojection.py:99-127 composed from Unfold + the differentiable warp kernel: taken only when an IMAGE
-    requires grad ("feature or image" in the reference's docstring); the trainer's IR patterns never do."""
-    bs, c, h, w = input_L.shape
-    unfold = torch.nn.Unfold(kernel_size=(ps, ps), padding=(ps - 1) // 2)
-    Lu = unfold(input_L).reshape(bs, -1, h, w)
-    Ru = unfold(input_R).reshape(bs, -1, h, w)
-    Wu = ops.warp(Ru, -pred_disp_l)
-    sel = mask.repeat(1, Lu.shape[1], 1, 1) if mask is not None else torch.ones_like(Lu).type(torch.bool)
-    loss = F.mse_loss(Wu[sel], Lu[sel])
-    warped = ops.patch_fold(input_R.detach(), pred_disp_l.detach(), ps) if RETURN_WARPED_PATCH_IMAGE else None
-    return loss, warped
-
-
 def get_reproj_error_patch(input_L, input_R, pred_disp_l, mask=None, ps=5):
     """reprojection.py:99-127 -- the loss the live trainer uses (ps = 11)."""
     assert ps % 2 == 1
-    if input_L.requires_grad or input_R.requires_grad:
-        loss, warped = _patch_loss_autograd(input_L, input_R, pred_disp_l, mask, ps)
-    else:
-        loss, warped = ops.reproj_loss(input_L, input_R, pred_disp_l, mask, ps=ps, sign=-1.0,
-                                       want_warped=RETURN_WARPED_PATCH_IMAGE)
-    return loss, warped, _int_mask(mask, input_L)
+    # An image that requires grad ("feature or image" in the reference's docstring) gets its gradient from the same
+    # fused operator.  That call always asks for the Fold image: the x-tiled kernel that computes the loss together
+    # with it is the one that stages the widest rows, so a wide input keeps working as it did under the reference's
+    # autograd composition.
+    img_grad = input_L.requires_grad or input_R.requires_grad
+    loss, warped = ops.reproj_loss(input_L, input_R, pred_disp_l, mask, ps=ps, sign=-1.0,
+                                   want_warped=RETURN_WARPED_PATCH_IMAGE or img_grad)
+    return loss, (warped if RETURN_WARPED_PATCH_IMAGE else None), _int_mask(mask, input_L)
 
 
 def get_reprojection_error_diff_ratio(input_L, input_R, pred_disp_l, mask=None):

@@ -214,6 +214,24 @@ int az_reproj_loss_fwd(const float* tgt, const float* src, const float* disp, fl
 /* gdisp[b,0,i,j] = gloss[0] * sign * 2/(K*sum m) * gpre[b,0,i,j] */
 int az_reproj_loss_bwd(const float* gpre, const double* stats, const float* gloss, float sign,
                        float* gdisp, int64_t B, int64_t C, int64_t H, int64_t W, int64_t ps, void* stream);
+/* Image gradients of the same loss (the reference differentiates its "feature or image" inputs too).  The
+ * arguments tgt .. ps and the shapes are the forward's; stats and gloss as for az_reproj_loss_bwd.  With
+ * r_k(i,j) = Wu_k(i,j) - Lu_k(i,j), p = (ps-1)/2 and rho_k(i,j) = gloss * 2 * m(i,j) * r_k(i,j) / (K * sum m):
+ *   gtgt[b,c,y,x] = - sum_{ky,kx} rho_{(c,ky,kx)}(y+p-ky, x+p-kx)   over in-image (i,j)  (adjoint of the Unfold)
+ *   gsrc[b,c,Y,X] = + sum rho_k(i,j) * wy_a(i) * wx_b(i,j)  over the bilinear corners (a,b) of the forward's sample
+ *                   position that are valid in the unfolded plane, with Y = y0(i)+a+ky-p, X = x0(i,j)+b+kx-p inside
+ *                   the image (adjoint of the warp of the unfolded planes)
+ * The residuals are recomputed from tgt, src, disp and mask (no [B,K,H,W] intermediate, no workspace, no host
+ * synchronisation).  gtgt and gsrc are [B,C,H,W] or NULL; every element of a non-NULL one is written exactly once
+ * (no zero-fill by the caller) and nothing else is written.  Deterministic: fixed-order sums and order-independent
+ * 64-bit fixed-point accumulation, no float atomics; two calls give bit-identical results.  sum m == 0 (empty mask)
+ * gives exact zeros (the reference's gradient of an empty selection).  A non-finite input read by a row of gsrc
+ * makes that row NaN.  Shapes: those of az_reproj_loss_fwd, any odd ps up to 4095.  Returns 0 at once when both
+ * outputs are NULL. */
+int az_reproj_loss_img_bwd(const float* tgt, const float* src, const float* disp, float sign, const uint8_t* mask,
+                           const float* lin_x, const float* lin_y, int64_t ps, const double* stats,
+                           const float* gloss, float* gtgt, float* gsrc,
+                           int64_t B, int64_t C, int64_t H, int64_t W, void* stream);
 /* Visualisation output of get_reproj_error_patch: Fold (overlap-sum) of the warped unfolded planes,
  * cropped by (ps-1)/2 (reprojection.py:120-125).  vis: [B,C,H,W]. */
 int az_patch_fold(const float* src, const float* disp, float sign, const float* lin_x, const float* lin_y,
