@@ -43,6 +43,8 @@ SIGNATURES = {
     "az_volume_conv0_bwd_16": (ctypes.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, ctypes.c_int, ctypes.c_int, _P]),
     "az_gwc_volume_fwd": (ctypes.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "az_gwc_volume_bwd": (ctypes.c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
+    "az_gwc_volume_fwd_16": (ctypes.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _I, ctypes.c_int, _P]),
+    "az_gwc_volume_bwd_16": (ctypes.c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, ctypes.c_int, _P]),
     "az_soft_argmin_fwd": (ctypes.c_int, [_P, _P, _P, _I, _I, _I, _I, _P]),
     "az_soft_argmin_bwd": (ctypes.c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "az_soft_argmin_fwd_16": (ctypes.c_int, [_P, _P, _P, _I, _I, _I, _I, ctypes.c_int, _P]),

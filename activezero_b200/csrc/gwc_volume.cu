@@ -10,11 +10,73 @@
 // per channel per four disparities).  Backward: direct 128-bit loads of the gradient planes (three
 // aligned float4 per plane: column x for gL, columns x+4m and x+4m+4 for the x+i diagonal of gR),
 // left/right rows in shared memory, fixed-order accumulation in registers: gather-style, atomic-free.
+//
+// The kernels the entry points run at their defaults are templated on the tensor dtype T (float, bf16, fp16; DESIGN.md
+// §4.15).  A 16-bit value is widened to fp32 exactly where it is read -- at the register load, or at the LDS from a
+// stage that a bulk copy filled with raw 16-bit bytes -- and from there on every instruction is the fp32 kernel's: the
+// fmaf chains in the same order, `inv` applied at the same place, fp32 accumulators, the same systolic hand-over.  Each
+// 16-bit result is rounded once, to nearest even, at its store, so a 16-bit kernel returns the fp32 kernel's result on
+// the widened inputs followed by .to(dtype).
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace az {
 
 constexpr int kGwcThreads = 256;
+
+// ---- element access of the templated kernels ----------------------------------------------------------------------
+// A quad is four consecutive elements: one 16-byte access in fp32, one 8-byte access in 16 bits (raw type GwcQuad<T>).
+// For T = float every helper is the plain access the fp32 kernels always made.
+template <typename T> struct GwcQuadT { using type = uint2; };
+template <> struct GwcQuadT<float> { using type = float4; };
+template <typename T> using GwcQuad = typename GwcQuadT<T>::type;
+
+template <typename T>
+__device__ __forceinline__ float4 widen4(const GwcQuad<T>& q) {
+    if constexpr (std::is_same<T, float>::value) {
+        return q;
+    } else if constexpr (std::is_same<T, __nv_bfloat16>::value) {
+        return make_float4(__uint_as_float(q.x << 16), __uint_as_float(q.x & 0xffff0000u), __uint_as_float(q.y << 16),
+                           __uint_as_float(q.y & 0xffff0000u));
+    } else {
+        const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&q.x));
+        const float2 b = __half22float2(*reinterpret_cast<const __half2*>(&q.y));
+        return make_float4(a.x, a.y, b.x, b.y);
+    }
+}
+// one RNE rounding per element; an fp16 value outside the format becomes +-inf, as .to(torch.float16) makes it
+template <typename T>
+__device__ __forceinline__ GwcQuad<T> narrow4(const float4& v) {
+    if constexpr (std::is_same<T, float>::value) {
+        return v;
+    } else if constexpr (std::is_same<T, __nv_bfloat16>::value) {
+        const __nv_bfloat162 a = __floats2bfloat162_rn(v.x, v.y), b = __floats2bfloat162_rn(v.z, v.w);
+        return make_uint2(*reinterpret_cast<const uint32_t*>(&a), *reinterpret_cast<const uint32_t*>(&b));
+    } else {
+        const __half2 a = __floats2half2_rn(v.x, v.y), b = __floats2half2_rn(v.z, v.w);
+        return make_uint2(*reinterpret_cast<const uint32_t*>(&a), *reinterpret_cast<const uint32_t*>(&b));
+    }
+}
+// quad k of the row at p (read-only path)
+template <typename T>
+__device__ __forceinline__ float4 ldg4(const T* p, int k = 0) {
+    return widen4<T>(__ldg(reinterpret_cast<const GwcQuad<T>*>(p) + k));
+}
+template <typename T>
+__device__ __forceinline__ void st4(T* p, const float4& v) {
+    *reinterpret_cast<GwcQuad<T>*>(p) = narrow4<T>(v);
+}
+template <typename T>
+__device__ __forceinline__ void st4_stream(T* p, const float4& v) {
+    __stcs(reinterpret_cast<GwcQuad<T>*>(p), narrow4<T>(v));
+}
+__device__ __forceinline__ float ldcs_f32(const float* p) { return __ldcs(p); }
+__device__ __forceinline__ float ldcs_f32(const __nv_bfloat16* p) { return __bfloat162float(__ldcs(p)); }
+__device__ __forceinline__ float ldcs_f32(const __half* p) { return __half2float(__ldcs(p)); }
+__device__ __forceinline__ void stcs_from_f32(float* p, float v) { __stcs(p, v); }
+__device__ __forceinline__ void stcs_from_f32(__nv_bfloat16* p, float v) { __stcs(p, __float2bfloat16_rn(v)); }
+__device__ __forceinline__ void stcs_from_f32(__half* p, float v) { __stcs(p, __float2half_rn(v)); }
 
 // window [k, k+4) of the 8 floats (a, b), k in 1..4 static after unrolling
 __device__ __forceinline__ float4 win8(const float4& a, const float4& b, int k) {
@@ -105,10 +167,9 @@ __global__ void __launch_bounds__(kGwcThreads) gwc_fwd_vec4_kernel(const float* 
 // (B of step m+1 is A of step m).  No shared memory, no barrier.
 // grid = (ceil(H*W/4 / 256), G * ceil(Dq/DG), B)
 // ------------------------------------------------------------------------------------------
-template <int CPG>
-__global__ void __launch_bounds__(kGwcThreads) gwc_fwd_planes_kernel(const float* __restrict__ L,
-                                                                    const float* __restrict__ R,
-                                                                    float* __restrict__ vol, int C, int G, int H, int W,
+template <typename T, int CPG>
+__global__ void __launch_bounds__(kGwcThreads) gwc_fwd_planes_kernel(const T* __restrict__ L, const T* __restrict__ R,
+                                                                    T* __restrict__ vol, int C, int G, int H, int W,
                                                                     int Dq, int DG, int ngroups) {
     const int W4 = W >> 2;
     const int g = blockIdx.y / ngroups, dg = blockIdx.y - g * ngroups, b = blockIdx.z;
@@ -117,23 +178,30 @@ __global__ void __launch_bounds__(kGwcThreads) gwc_fwd_planes_kernel(const float
     if (pp >= H * W4) return;
     const int x = (pp % W4) * 4;
     const size_t HW = (size_t)H * W;
-    const float* Lg = L + ((size_t)b * C + (size_t)g * CPG) * HW + (size_t)pp * 4;
-    const float* Rg = R + ((size_t)b * C + (size_t)g * CPG) * HW + (size_t)pp * 4;
+    const T* Lg = L + ((size_t)b * C + (size_t)g * CPG) * HW + (size_t)pp * 4;
+    const T* Rg = R + ((size_t)b * C + (size_t)g * CPG) * HW + (size_t)pp * 4;
     const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
     const float inv = 1.0f / (float)CPG;
     float4 l[CPG], Bw[CPG];
 #pragma unroll
     for (int c = 0; c < CPG; ++c) {
-        float4 t = __ldg(reinterpret_cast<const float4*>(Lg + (size_t)c * HW));
+        float4 t = ldg4(Lg + (size_t)c * HW);
         l[c] = make_float4(t.x * inv, t.y * inv, t.z * inv, t.w * inv);
-        Bw[c] = (x - i0 >= 0) ? __ldg(reinterpret_cast<const float4*>(Rg + (size_t)c * HW - i0)) : zero;
+        Bw[c] = (x - i0 >= 0) ? ldg4(Rg + (size_t)c * HW - i0) : zero;
     }
-    float* out = vol + ((size_t)b * G + g) * Dq * HW + (size_t)pp * 4;
+    T* out = vol + ((size_t)b * G + g) * Dq * HW + (size_t)pp * 4;
     for (int m4 = i0; m4 < i1; m4 += 4) {
         float4 A[CPG];
 #pragma unroll
-        for (int c = 0; c < CPG; ++c)
-            A[c] = (x - m4 - 4 >= 0) ? __ldg(reinterpret_cast<const float4*>(Rg + (size_t)c * HW - m4 - 4)) : zero;
+        for (int c = 0; c < CPG; ++c) {
+            if constexpr (std::is_same<T, float>::value) {
+                A[c] = (x - m4 - 4 >= 0) ? ldg4(Rg + (size_t)c * HW - m4 - 4) : zero;
+            } else {  // select the raw quad, then widen (a select after the widening made ptxas spill)
+                const uint2 a = (x - m4 - 4 >= 0) ? __ldg(reinterpret_cast<const uint2*>(Rg + (size_t)c * HW - m4 - 4))
+                                                  : make_uint2(0u, 0u);
+                A[c] = widen4<T>(a);
+            }
+        }
 #pragma unroll
         for (int r = 0; r < 4; ++r) {
             if (m4 + r < i1) {
@@ -146,7 +214,7 @@ __global__ void __launch_bounds__(kGwcThreads) gwc_fwd_planes_kernel(const float
                     acc.z = fmaf(l[c].z, w.z, acc.z);
                     acc.w = fmaf(l[c].w, w.w, acc.w);
                 }
-                st_stream(reinterpret_cast<float4*>(out + (size_t)(m4 + r) * HW), acc);
+                st4_stream(out + (size_t)(m4 + r) * HW, acc);
             }
         }
 #pragma unroll
@@ -155,9 +223,9 @@ __global__ void __launch_bounds__(kGwcThreads) gwc_fwd_planes_kernel(const float
 }
 
 // scalar fallback, any shape.  grid = (ceil(H*W/256), Dq, B*G)
-__global__ void __launch_bounds__(256) gwc_fwd_scalar_kernel(const float* __restrict__ L, const float* __restrict__ R,
-                                                             float* __restrict__ vol, int C, int G, int H, int W,
-                                                             int Dq) {
+template <typename T>
+__global__ void __launch_bounds__(256) gwc_fwd_scalar_kernel(const T* __restrict__ L, const T* __restrict__ R,
+                                                             T* __restrict__ vol, int C, int G, int H, int W, int Dq) {
     const int hw = blockIdx.x * 256 + threadIdx.x;
     if (hw >= H * W) return;
     const int i = blockIdx.y, bg = blockIdx.z, b = bg / G, g = bg - b * G;
@@ -165,12 +233,12 @@ __global__ void __launch_bounds__(256) gwc_fwd_scalar_kernel(const float* __rest
     const size_t HW = (size_t)H * W;
     float acc = 0.f;
     if (x >= i) {
-        const float* l = L + ((size_t)b * C + (size_t)g * cpg) * HW + hw;
-        const float* r = R + ((size_t)b * C + (size_t)g * cpg) * HW + hw - i;
-        for (int c = 0; c < cpg; ++c) acc = fmaf(__ldg(l + (size_t)c * HW), __ldg(r + (size_t)c * HW), acc);
+        const T* l = L + ((size_t)b * C + (size_t)g * cpg) * HW + hw;
+        const T* r = R + ((size_t)b * C + (size_t)g * cpg) * HW + hw - i;
+        for (int c = 0; c < cpg; ++c) acc = fmaf(ld_f32(l + (size_t)c * HW), ld_f32(r + (size_t)c * HW), acc);
         acc *= 1.0f / (float)cpg;
     }
-    st_stream(vol + (((size_t)bg * Dq + i) * H) * W + hw, acc);
+    stcs_from_f32(vol + (((size_t)bg * Dq + i) * H) * W + hw, acc);
 }
 
 // window [k, k+4) of the 8 floats (a, b), k in 0..4
@@ -189,11 +257,11 @@ __device__ __forceinline__ void fma4(float4& acc, const float4& u, const float4&
 //   gL[c,x] = inv * sum_{i<=x} g[i,x] * R[c,x-i];   gR[c,x] = inv * sum_{x+i<W} g[i,x+i] * L[c,x+i]
 // smem: Ls[CPT][rows_cap][W + tail] (zero tail) | Rs[CPT][rows_cap][pad + W] (zero prefix)
 // ------------------------------------------------------------------------------------------
-template <int CPG, int CPT>
-__global__ void __launch_bounds__(kGwcThreads, 3) gwc_bwd_direct_kernel(const float* __restrict__ gvol,
-                                                                       const float* __restrict__ L,
-                                                                       const float* __restrict__ R,
-                                                                       float* __restrict__ gL, float* __restrict__ gR,
+template <typename T, int CPG, int CPT>
+__global__ void __launch_bounds__(kGwcThreads, 3) gwc_bwd_direct_kernel(const T* __restrict__ gvol,
+                                                                       const T* __restrict__ L,
+                                                                       const T* __restrict__ R,
+                                                                       T* __restrict__ gL, T* __restrict__ gR,
                                                                        int C, int G, int H, int W, int Dq, int pad,
                                                                        int rows_cap) {
     extern __shared__ __align__(16) float smem[];
@@ -215,8 +283,8 @@ __global__ void __launch_bounds__(kGwcThreads, 3) gwc_bwd_direct_kernel(const fl
         const int y = rem / S4, q = rem - y * S4;
         const size_t row = cbase + (size_t)c * HW + (size_t)(y_first + y) * W;
         float4 rv = make_float4(0.f, 0.f, 0.f, 0.f), lv = rv;
-        if (q >= pad4) rv = __ldg(reinterpret_cast<const float4*>(R + row) + (q - pad4));
-        if (q < W4) lv = __ldg(reinterpret_cast<const float4*>(L + row) + q);
+        if (q >= pad4) rv = ldg4(R + row, q - pad4);
+        if (q < W4) lv = ldg4(L + row, q);
         reinterpret_cast<float4*>(Rs + c * ch_stride + y * S)[q] = rv;
         reinterpret_cast<float4*>(Ls + c * ch_stride + y * S)[q] = lv;
     }
@@ -227,7 +295,7 @@ __global__ void __launch_bounds__(kGwcThreads, 3) gwc_bwd_direct_kernel(const fl
     const int y = pp / W4, x = (pp - y * W4) * 4;
     const float* rp = Rs + (y - y_first) * S + pad + x;
     const float* lp = Ls + (y - y_first) * S + x;
-    const float* gp = gvol + ((size_t)b * G + g) * Dq * HW + (size_t)pp * 4;
+    const T* gp = gvol + ((size_t)b * G + g) * Dq * HW + (size_t)pp * 4;
     const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
     float4 aL[CPT], aR[CPT], RB[CPT], LA[CPT];
 #pragma unroll
@@ -243,11 +311,11 @@ __global__ void __launch_bounds__(kGwcThreads, 3) gwc_bwd_direct_kernel(const fl
 #pragma unroll
         for (int r = 0; r < 4; ++r) {
             const int i = m4 + r;
-            const float* q = gp + (size_t)i * HW;
+            const T* q = gp + (size_t)i * HW;
             const bool on = i < Dq;
-            gl[r] = (on && i <= x + 3) ? __ldg(reinterpret_cast<const float4*>(q)) : zero;
-            ga[r] = (on && inA) ? __ldg(reinterpret_cast<const float4*>(q + m4)) : zero;
-            gb[r] = (on && inB) ? __ldg(reinterpret_cast<const float4*>(q + m4 + 4)) : zero;
+            gl[r] = (on && i <= x + 3) ? ldg4(q) : zero;
+            ga[r] = (on && inA) ? ldg4(q + m4) : zero;
+            gb[r] = (on && inB) ? ldg4(q + m4 + 4) : zero;
         }
         float4 RA[CPT], LB[CPT];
 #pragma unroll
@@ -274,10 +342,8 @@ __global__ void __launch_bounds__(kGwcThreads, 3) gwc_bwd_direct_kernel(const fl
 #pragma unroll
     for (int c = 0; c < CPT; ++c) {
         const size_t o = cbase + (size_t)c * HW + (size_t)pp * 4;
-        if (gL != nullptr)
-            *reinterpret_cast<float4*>(gL + o) = make_float4(aL[c].x * inv, aL[c].y * inv, aL[c].z * inv, aL[c].w * inv);
-        if (gR != nullptr)
-            *reinterpret_cast<float4*>(gR + o) = make_float4(aR[c].x * inv, aR[c].y * inv, aR[c].z * inv, aR[c].w * inv);
+        if (gL != nullptr) st4(gL + o, make_float4(aL[c].x * inv, aL[c].y * inv, aL[c].z * inv, aL[c].w * inv));
+        if (gR != nullptr) st4(gR + o, make_float4(aR[c].x * inv, aR[c].y * inv, aR[c].z * inv, aR[c].w * inv));
     }
 }
 
@@ -422,17 +488,20 @@ __global__ void __launch_bounds__(kGwcRowThreads) gwc_bwd_row_kernel(const float
 // ------------------------------------------------------------------------------------------
 
 // LSM: left rows staged in shared memory (S = 4) or read straight into registers (S = 5: their 8 KB buy a stage)
-template <int CPG, int NT, int S, bool LSM>
-__global__ void __launch_bounds__(NT, 512 / NT) gwc_bwd_systolic_kernel(const float* __restrict__ gvol,
-                                                                       const float* __restrict__ L,
-                                                                       const float* __restrict__ R,
-                                                                       float* __restrict__ gL, float* __restrict__ gR,
+// 16 bits: the stages, Ls and Rs hold raw 16-bit quads (8 bytes), widened at the LDS; `hand` carries fp32 accumulators.
+template <typename T, int CPG, int NT, int S, bool LSM>
+__global__ void __launch_bounds__(NT, 512 / NT) gwc_bwd_systolic_kernel(const T* __restrict__ gvol,
+                                                                       const T* __restrict__ L,
+                                                                       const T* __restrict__ R,
+                                                                       T* __restrict__ gL, T* __restrict__ gR,
                                                                        int C, int G, int H, int W, int Dq, int rows) {
-    extern __shared__ __align__(128) float4 stage[];  // [S][4][NT] | Ls[CPG][NT] | Rs[CPG][NT]
+    using Q = GwcQuad<T>;
+    extern __shared__ __align__(128) float4 stage_smem[];
+    Q* stage = reinterpret_cast<Q*>(stage_smem);  // [S][4][NT] | Ls[CPG][NT] | Rs[CPG][NT]
     __shared__ __align__(8) uint64_t full[S];
     __shared__ __align__(8) uint64_t feat_bar;
     __shared__ float4 hand[2][NT / 32 + 1][CPG];  // slot w + 1: lane 31 of warp w; slot 0 stays zero
-    __shared__ float4 zslot;                      // stands in for the planes >= Dq of the last step
+    __shared__ Q zslot;                           // stands in for the planes >= Dq of the last step
     const int W4 = W >> 2;
     const int g = blockIdx.y, b = blockIdx.z;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -443,10 +512,10 @@ __global__ void __launch_bounds__(NT, 512 / NT) gwc_bwd_systolic_kernel(const fl
     const bool row_end = q == W4 - 1;
     const size_t HW = (size_t)H * W;
     const size_t p0 = (size_t)y0 * W;  // first float of the CTA's positions within a plane
-    const float* gbase = gvol + ((size_t)b * G + g) * Dq * HW + p0;
+    const T* gbase = gvol + ((size_t)b * G + g) * Dq * HW + p0;
     const size_t cbase = ((size_t)b * C + (size_t)g * CPG) * HW + p0 + (size_t)tid * 4;
     const int M = (Dq + 3) >> 2;
-    const uint32_t plane_bytes = (uint32_t)nact * 16u;
+    const uint32_t plane_bytes = (uint32_t)nact * (uint32_t)sizeof(Q);
     const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
 
     auto issue = [&](int m) {  // one thread: the four planes of step m -> stage m % S
@@ -455,8 +524,8 @@ __global__ void __launch_bounds__(NT, 512 / NT) gwc_bwd_systolic_kernel(const fl
         for (int r = 0; r < np; ++r)
             bulk_g2s(stage + (size_t)(s * 4 + r) * NT, gbase + (size_t)(4 * m + r) * HW, plane_bytes, &full[s]);
     };
-    float4* Ls = stage + (size_t)S * 4 * NT;
-    float4* Rs = Ls + (LSM ? (size_t)CPG * NT : 0);
+    Q* Ls = stage + (size_t)S * 4 * NT;
+    Q* Rs = Ls + (LSM ? (size_t)CPG * NT : 0);
     if (warp == 0) {
         // lane 0 arms the barriers, then the lanes issue the first copies
         if (lane == 0) {
@@ -467,7 +536,8 @@ __global__ void __launch_bounds__(NT, 512 / NT) gwc_bwd_systolic_kernel(const fl
             mbar_expect_tx(&feat_bar, plane_bytes * (uint32_t)((LSM ? 2 : 1) * CPG));
             for (int m = 0; m < min(M, S); ++m)
                 mbar_expect_tx(&full[m], plane_bytes * (uint32_t)min(4, Dq - 4 * m));
-            zslot = zero;
+            if constexpr (std::is_same<T, float>::value) zslot = zero;
+            else zslot = make_uint2(0u, 0u);
         }
         __syncwarp();
         const size_t fb = ((size_t)b * C + (size_t)g * CPG) * HW + p0;
@@ -478,6 +548,10 @@ __global__ void __launch_bounds__(NT, 512 / NT) gwc_bwd_systolic_kernel(const fl
         } else if (lane >= 8 && lane - 8 < min(Dq, 4 * S)) {
             const int i = lane - 8;  // plane i -> stage i / 4, slot i % 4
             bulk_g2s(stage + (size_t)i * NT, gbase + (size_t)i * HW, plane_bytes, &full[i >> 2]);
+            if constexpr (4 * S > 24) {  // a ring of more than six stages: the 24 lanes take further rounds
+                for (int i2 = i + 24; i2 < min(Dq, 4 * S); i2 += 24)
+                    bulk_g2s(stage + (size_t)i2 * NT, gbase + (size_t)i2 * HW, plane_bytes, &full[i2 >> 2]);
+            }
         }
     }
     if (tid < 2 * CPG) hand[tid / CPG][0][tid % CPG] = zero;
@@ -487,13 +561,20 @@ __global__ void __launch_bounds__(NT, 512 / NT) gwc_bwd_systolic_kernel(const fl
     if (!LSM) {
 #pragma unroll
         for (int c = 0; c < CPG; ++c)
-            l[c] = active ? __ldg(reinterpret_cast<const float4*>(L + cbase + (size_t)c * HW)) : zero;
+            l[c] = active ? ldg4(L + cbase + (size_t)c * HW) : zero;
     }
     mbar_wait(&feat_bar, 0);
 #pragma unroll
     for (int c = 0; c < CPG; ++c) {
-        if (LSM) l[c] = Ls[(size_t)c * NT + tid];  // threads without a quad read stale shared memory: their values never
-        Bw[c] = Rs[(size_t)c * NT + tid];  // reach a thread that owns one (the walk only moves right)
+        // threads without a quad read stale shared memory: their values never reach a thread that owns one (the walk
+        // only moves right)
+        if constexpr (std::is_same<T, float>::value) {
+            if (LSM) l[c] = Ls[(size_t)c * NT + tid];
+            Bw[c] = Rs[(size_t)c * NT + tid];
+        } else {
+            if (LSM) l[c] = widen4<T>(Ls[(size_t)c * NT + tid]);
+            Bw[c] = widen4<T>(Rs[(size_t)c * NT + tid]);
+        }
         aL[c] = zero;
         V[c] = zero;
     }
@@ -506,10 +587,13 @@ __global__ void __launch_bounds__(NT, 512 / NT) gwc_bwd_systolic_kernel(const fl
         mbar_wait(&full[s], (uint32_t)((m / S) & 1));
         float4 gq[4];
 #pragma unroll
-        for (int r = 0; r < 4; ++r) gq[r] = *((r < np) ? stage + (size_t)(s * 4 + r) * NT + tid : &zslot);
+        for (int r = 0; r < 4; ++r) gq[r] = widen4<T>(*((r < np) ? stage + (size_t)(s * 4 + r) * NT + tid : &zslot));
         float4 A[CPG];
 #pragma unroll
-        for (int c = 0; c < CPG; ++c) A[c] = (q - m - 1 >= 0) ? Rs[(size_t)c * NT + tid - m - 1] : zero;
+        for (int c = 0; c < CPG; ++c) {
+            if constexpr (std::is_same<T, float>::value) A[c] = (q - m - 1 >= 0) ? Rs[(size_t)c * NT + tid - m - 1] : zero;
+            else A[c] = (q - m - 1 >= 0) ? widen4<T>(Rs[(size_t)c * NT + tid - m - 1]) : zero;
+        }
 #pragma unroll
         for (int c = 0; c < CPG; ++c) {
             // gL: own columns; gR "high" part: targets j - r >= 0 of the quad this thread holds
@@ -530,8 +614,8 @@ __global__ void __launch_bounds__(NT, 512 / NT) gwc_bwd_systolic_kernel(const fl
             if (active && q - m >= 0 && gR != nullptr) {
 #pragma unroll
                 for (int c = 0; c < CPG; ++c)
-                    *reinterpret_cast<float4*>(gR + cbase + (size_t)c * HW - (size_t)(4 * m)) =
-                        make_float4(V[c].x * inv, V[c].y * inv, V[c].z * inv, V[c].w * inv);
+                    st4(gR + cbase + (size_t)c * HW - (size_t)(4 * m),
+                        make_float4(V[c].x * inv, V[c].y * inv, V[c].z * inv, V[c].w * inv));
             }
 #pragma unroll
             for (int c = 0; c < CPG; ++c) V[c] = zero;
@@ -572,85 +656,114 @@ __global__ void __launch_bounds__(NT, 512 / NT) gwc_bwd_systolic_kernel(const fl
     if (!active) return;
 #pragma unroll
     for (int c = 0; c < CPG; ++c) {
-        if (gL != nullptr)
-            *reinterpret_cast<float4*>(gL + cbase + (size_t)c * HW) =
-                make_float4(aL[c].x * inv, aL[c].y * inv, aL[c].z * inv, aL[c].w * inv);
+        if (gL != nullptr) st4(gL + cbase + (size_t)c * HW, make_float4(aL[c].x * inv, aL[c].y * inv, aL[c].z * inv, aL[c].w * inv));
         if (gR != nullptr && q - M >= 0)
-            *reinterpret_cast<float4*>(gR + cbase + (size_t)c * HW - (size_t)(4 * M)) =
-                make_float4(V[c].x * inv, V[c].y * inv, V[c].z * inv, V[c].w * inv);
+            st4(gR + cbase + (size_t)c * HW - (size_t)(4 * M), make_float4(V[c].x * inv, V[c].y * inv, V[c].z * inv, V[c].w * inv));
     }
 }
 
 // scalar fallback: one thread per (b, c, y, x).  grid = (ceil(H*W/256), C, B)
-__global__ void __launch_bounds__(256) gwc_bwd_scalar_kernel(const float* __restrict__ gvol,
-                                                             const float* __restrict__ L, const float* __restrict__ R,
-                                                             float* __restrict__ gL, float* __restrict__ gR, int C,
-                                                             int G, int H, int W, int Dq) {
+template <typename T>
+__global__ void __launch_bounds__(256) gwc_bwd_scalar_kernel(const T* __restrict__ gvol, const T* __restrict__ L,
+                                                             const T* __restrict__ R, T* __restrict__ gL,
+                                                             T* __restrict__ gR, int C, int G, int H, int W, int Dq) {
     const int hw = blockIdx.x * 256 + threadIdx.x;
     if (hw >= H * W) return;
     const int c = blockIdx.y, b = blockIdx.z;
     const int cpg = C / G, g = c / cpg, x = hw % W;
     const size_t HW = (size_t)H * W;
-    const float* gv = gvol + ((size_t)b * G + g) * Dq * HW + hw;
-    const float* l = L + ((size_t)b * C + c) * HW + hw;
-    const float* r = R + ((size_t)b * C + c) * HW + hw;
+    const T* gv = gvol + ((size_t)b * G + g) * Dq * HW + hw;
+    const T* l = L + ((size_t)b * C + c) * HW + hw;
+    const T* r = R + ((size_t)b * C + c) * HW + hw;
     float aL = 0.f, aR = 0.f;
     for (int i = 0; i < Dq; ++i) {
-        if (i <= x) aL = fmaf(ld_stream(gv + (size_t)i * HW), __ldg(r - i), aL);
-        if (x + i < W) aR = fmaf(ld_stream(gv + (size_t)i * HW + i), __ldg(l + i), aR);
+        if (i <= x) aL = fmaf(ldcs_f32(gv + (size_t)i * HW), ld_f32(r - i), aL);
+        if (x + i < W) aR = fmaf(ldcs_f32(gv + (size_t)i * HW + i), ld_f32(l + i), aR);
     }
     const float inv = 1.0f / (float)cpg;
-    if (gL != nullptr) gL[((size_t)b * C + c) * HW + hw] = aL * inv;
-    if (gR != nullptr) gR[((size_t)b * C + c) * HW + hw] = aR * inv;
+    if (gL != nullptr) st_from_f32(gL + ((size_t)b * C + c) * HW + hw, aL * inv);
+    if (gR != nullptr) st_from_f32(gR + ((size_t)b * C + c) * HW + hw, aR * inv);
 }
 
-template <int CPG>
-static int launch_gwc_fwd(const float* L, const float* R, float* vol, int B, int C, int G, int H, int W, int Dq,
-                          cudaStream_t st, bool* done) {
+// The 16-bit forms of the kernels follow the fp32 selection at its defaults and read no AZ_GWC_* knob.  Where a 16-bit
+// alignment rule excludes the kernel the fp32 entry point would run, a kernel with the same summation order runs:
+//   forward : the planes kernel pre-scales the left quads by inv = 1/cpg, a power of two for the cpg it serves, which
+//             commutes with every rounding outside fp32's subnormal range; the scalar kernel (sum of cpg products from
+//             zero in ascending c, then *inv -- the order of the fp32 grid-overflow kernel gwc_fwd_vec4_kernel) therefore
+//             returns the same values;
+//   backward: the systolic, direct and scalar kernels all sum the terms g * feature in ascending i from zero and scale by
+//             inv once at the end, so any of them returns the same gradient.
+// Stage ring of the 16-bit systolic backward.  A 16-bit stage holds half the bytes of an fp32 one, yet at config 2 the
+// 16-bit kernel takes the fp32 kernel's time with 5 or 6 stages and is slower with 8 or 10 (benchmarks/micro/
+// gwc16_stages.cu, DESIGN.md §4.15): it is bound by the per-step instructions it shares with the fp32 kernel, not by the
+// bytes in flight, so it keeps the fp32 ring.
+constexpr int kGwcSys16Stages = 5;
+
+inline bool aligned_to(const void* p, size_t n) { return (reinterpret_cast<uintptr_t>(p) % n) == 0; }
+
+template <typename T, int CPG>
+static int launch_gwc_fwd(const T* L, const T* R, T* vol, int B, int C, int G, int H, int W, int Dq, cudaStream_t st,
+                          bool* done) {
+    constexpr bool f32 = std::is_same<T, float>::value;
     const int W4 = W / 4;
     *done = false;
-    int DG = tuning("AZ_GWC_DG", 16);  // planes per CTA; 0 = round-1 kernel (all planes per CTA, rows in shared memory)
+    // planes per CTA; 0 = round-1 kernel (all planes per CTA, rows in shared memory)
+    int DG = f32 ? tuning("AZ_GWC_DG", 16) : 16;
     if (DG > 0) {
         DG = (DG + 3) & ~3;
         const int64_t ngroups = ceil_div(Dq, DG);
         if ((int64_t)G * ngroups <= 65535) {
             dim3 grid((unsigned)ceil_div((int64_t)H * W4, kGwcThreads), (unsigned)(G * ngroups), (unsigned)B);
-            gwc_fwd_planes_kernel<CPG><<<grid, kGwcThreads, 0, st>>>(L, R, vol, C, G, H, W, Dq, DG, (int)ngroups);
+            gwc_fwd_planes_kernel<T, CPG><<<grid, kGwcThreads, 0, st>>>(L, R, vol, C, G, H, W, Dq, DG, (int)ngroups);
             *done = true;
             return (int)cudaGetLastError();
         }
     }
-    const int pad = (Dq + 3) / 4 * 4 + 4;
-    const int rows_cap = (kGwcThreads + W4 - 1) / W4 + 1;
-    const size_t smem = (size_t)CPG * rows_cap * (pad + W) * sizeof(float);
-    if (smem > 200 * 1024) return 0;
-    cudaError_t e = cudaFuncSetAttribute(gwc_fwd_vec4_kernel<CPG>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         200 * 1024);
-    if (e != cudaSuccess) return (int)e;
-    dim3 grid((unsigned)ceil_div((int64_t)H * W4, kGwcThreads), (unsigned)G, (unsigned)B);
-    gwc_fwd_vec4_kernel<CPG><<<grid, kGwcThreads, smem, st>>>(L, R, vol, C, H, W, Dq, pad, rows_cap);
-    *done = true;
-    return (int)cudaGetLastError();
+    if constexpr (!f32) {
+        return 0;  // grid overflow: the scalar kernel
+    } else {
+        const int pad = (Dq + 3) / 4 * 4 + 4;
+        const int rows_cap = (kGwcThreads + W4 - 1) / W4 + 1;
+        const size_t smem = (size_t)CPG * rows_cap * (pad + W) * sizeof(float);
+        if (smem > 200 * 1024) return 0;
+        cudaError_t e = cudaFuncSetAttribute(gwc_fwd_vec4_kernel<CPG>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                             200 * 1024);
+        if (e != cudaSuccess) return (int)e;
+        dim3 grid((unsigned)ceil_div((int64_t)H * W4, kGwcThreads), (unsigned)G, (unsigned)B);
+        gwc_fwd_vec4_kernel<CPG><<<grid, kGwcThreads, smem, st>>>(L, R, vol, C, H, W, Dq, pad, rows_cap);
+        *done = true;
+        return (int)cudaGetLastError();
+    }
 }
 
-template <int CPG>
-static int launch_gwc_bwd(const float* gvol, const float* L, const float* R, float* gL, float* gR, int B, int C, int G,
-                          int H, int W, int Dq, cudaStream_t st, bool* done) {
+// systolic_ok: the bases and the row length suit the systolic kernel's bulk copies (16-byte addresses and sizes)
+template <typename T, int CPG>
+static int launch_gwc_bwd(const T* gvol, const T* L, const T* R, T* gL, T* gR, int B, int C, int G, int H, int W, int Dq,
+                          bool systolic_ok, cudaStream_t st, bool* done) {
+    constexpr bool f32 = std::is_same<T, float>::value;
     constexpr int CPT = CPG >= 2 ? 2 : 1;
     *done = false;
-    const int variant = tuning("AZ_GWC_BWD", 2);  // 2 = systolic one-pass (default), 1 = TMA row kernel, 0 = direct
-    if (variant == 2 && CPG <= 4 && W / 4 <= kGwcThreads && G <= 65535) {
+    const int variant = f32 ? tuning("AZ_GWC_BWD", 2) : 2;  // 2 = systolic one-pass (default), 1 = TMA row kernel, 0 = direct
+    if (variant == 2 && systolic_ok && CPG <= 4 && W / 4 <= kGwcThreads && G <= 65535) {
         constexpr int K = CPG <= 4 ? CPG : 1;
         const int W4 = W / 4;
         // 128-thread CTAs (four per SM) hide each other's pipeline fill better than two of 256
-        const bool small = W4 <= 128 && tuning("AZ_GWC_BWD_NT", 128) == 128;
-        const bool five = tuning("AZ_GWC_BWD_STAGES", 5) == 5;
+        const bool small = W4 <= 128 && (!f32 || tuning("AZ_GWC_BWD_NT", 128) == 128);
         const int nt = small ? 128 : 256, rows = nt / W4;
         const int64_t gx = ceil_div(H, rows);
         if (gx <= 0x7fffffff) {
-            const size_t smem_sys = (size_t)(five ? 5 * 4 + K : 4 * 4 + 2 * K) * nt * sizeof(float4);
-            auto kern = small ? (five ? gwc_bwd_systolic_kernel<K, 128, 5, false> : gwc_bwd_systolic_kernel<K, 128, 4, true>)
-                              : (five ? gwc_bwd_systolic_kernel<K, 256, 5, false> : gwc_bwd_systolic_kernel<K, 256, 4, true>);
+            void (*kern)(const T*, const T*, const T*, T*, T*, int, int, int, int, int, int);
+            size_t smem_sys;
+            if constexpr (f32) {
+                const bool five = tuning("AZ_GWC_BWD_STAGES", 5) == 5;
+                smem_sys = (size_t)(five ? 5 * 4 + K : 4 * 4 + 2 * K) * nt * sizeof(float4);
+                kern = small ? (five ? gwc_bwd_systolic_kernel<T, K, 128, 5, false> : gwc_bwd_systolic_kernel<T, K, 128, 4, true>)
+                             : (five ? gwc_bwd_systolic_kernel<T, K, 256, 5, false> : gwc_bwd_systolic_kernel<T, K, 256, 4, true>);
+            } else {
+                smem_sys = (size_t)(kGwcSys16Stages * 4 + K) * nt * sizeof(GwcQuad<T>);
+                kern = small ? gwc_bwd_systolic_kernel<T, K, 128, kGwcSys16Stages, false>
+                             : gwc_bwd_systolic_kernel<T, K, 256, kGwcSys16Stages, false>;
+            }
             cudaError_t es = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_sys);
             if (es != cudaSuccess) return (int)es;
             dim3 grid((unsigned)gx, (unsigned)G, (unsigned)B);
@@ -659,30 +772,89 @@ static int launch_gwc_bwd(const float* gvol, const float* L, const float* R, flo
             return (int)cudaGetLastError();
         }
     }
-    if (variant == 1 && H <= 65535) {  // one-pass row kernel (TMA bulk staging)
-        const int padr = (Dq + 3) / 4 * 4 + 4, GP = (W + Dq + 8 + 3) & ~3;
-        const size_t smem_row = ((size_t)(Dq + CPG) * GP + (size_t)CPG * (padr + W)) * sizeof(float);
-        if (smem_row <= 200 * 1024 && (size_t)(Dq + 2 * CPG) * W * 4 < (1u << 20)) {
-            cudaError_t er = cudaFuncSetAttribute(gwc_bwd_row_kernel<CPG>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                  200 * 1024);
-            if (er != cudaSuccess) return (int)er;
-            dim3 grid((unsigned)H, (unsigned)G, (unsigned)B);
-            gwc_bwd_row_kernel<CPG><<<grid, kGwcRowThreads, smem_row, st>>>(gvol, L, R, gL, gR, C, G, H, W, Dq, GP, padr);
-            *done = true;
-            return (int)cudaGetLastError();
+    if constexpr (f32) {
+        if (variant == 1 && H <= 65535) {  // one-pass row kernel (TMA bulk staging)
+            const int padr = (Dq + 3) / 4 * 4 + 4, GP = (W + Dq + 8 + 3) & ~3;
+            const size_t smem_row = ((size_t)(Dq + CPG) * GP + (size_t)CPG * (padr + W)) * sizeof(float);
+            if (smem_row <= 200 * 1024 && (size_t)(Dq + 2 * CPG) * W * 4 < (1u << 20)) {
+                cudaError_t er = cudaFuncSetAttribute(gwc_bwd_row_kernel<CPG>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                      200 * 1024);
+                if (er != cudaSuccess) return (int)er;
+                dim3 grid((unsigned)H, (unsigned)G, (unsigned)B);
+                gwc_bwd_row_kernel<CPG><<<grid, kGwcRowThreads, smem_row, st>>>(gvol, L, R, gL, gR, C, G, H, W, Dq, GP, padr);
+                *done = true;
+                return (int)cudaGetLastError();
+            }
         }
     }
     const int W4 = W / 4, pad = (Dq + 3) / 4 * 4 + 4;
     const int rows_cap = (kGwcThreads + W4 - 1) / W4 + 1;
-    const size_t smem = (size_t)2 * CPT * rows_cap * (pad + W) * sizeof(float);
+    const size_t smem = (size_t)2 * CPT * rows_cap * (pad + W) * sizeof(float);  // rows staged widened to fp32
     if (smem > 100 * 1024 || (long long)G * (CPG / CPT) > 65535) return 0;
-    cudaError_t e = cudaFuncSetAttribute(gwc_bwd_direct_kernel<CPG, CPT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(gwc_bwd_direct_kernel<T, CPG, CPT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          100 * 1024);
     if (e != cudaSuccess) return (int)e;
     dim3 grid((unsigned)ceil_div((int64_t)H * W4, kGwcThreads), (unsigned)(G * (CPG / CPT)), (unsigned)B);
-    gwc_bwd_direct_kernel<CPG, CPT><<<grid, kGwcThreads, smem, st>>>(gvol, L, R, gL, gR, C, G, H, W, Dq, pad, rows_cap);
+    gwc_bwd_direct_kernel<T, CPG, CPT><<<grid, kGwcThreads, smem, st>>>(gvol, L, R, gL, gR, C, G, H, W, Dq, pad, rows_cap);
     *done = true;
     return (int)cudaGetLastError();
+}
+
+// Kernel selection shared by the fp32 and 16-bit entry points (arguments already checked).  The quad kernels need
+// W % 4 == 0 and quad-aligned bases (16 bytes in fp32, 8 bytes in 16 bits); everything else runs the scalar kernels.
+template <typename T>
+static int gwc_fwd(const T* L, const T* R, T* vol, int64_t B, int64_t C, int64_t H, int64_t W, int64_t Dq, int64_t G,
+                   cudaStream_t st) {
+    const size_t qb = sizeof(GwcQuad<T>);
+    const int64_t cpg = C / G;
+    if ((W % 4 == 0) && aligned_to(L, qb) && aligned_to(R, qb) && aligned_to(vol, qb)) {
+        bool done = false;
+        int rc = 0;
+        switch (cpg) {
+            case 1: rc = launch_gwc_fwd<T, 1>(L, R, vol, (int)B, (int)C, (int)G, (int)H, (int)W, (int)Dq, st, &done); break;
+            case 2: rc = launch_gwc_fwd<T, 2>(L, R, vol, (int)B, (int)C, (int)G, (int)H, (int)W, (int)Dq, st, &done); break;
+            case 4: rc = launch_gwc_fwd<T, 4>(L, R, vol, (int)B, (int)C, (int)G, (int)H, (int)W, (int)Dq, st, &done); break;
+            case 8: rc = launch_gwc_fwd<T, 8>(L, R, vol, (int)B, (int)C, (int)G, (int)H, (int)W, (int)Dq, st, &done); break;
+            default: break;
+        }
+        if (rc != 0) return rc;
+        if (done) return 0;
+    }
+    if (Dq > 65535 || B * G > 65535) return AZ_ERR_BAD_ARG;
+    dim3 grid((unsigned)ceil_div(H * W, 256), (unsigned)Dq, (unsigned)(B * G));
+    gwc_fwd_scalar_kernel<T><<<grid, 256, 0, st>>>(L, R, vol, (int)C, (int)G, (int)H, (int)W, (int)Dq);
+    AZ_LAUNCH_CHECK();
+    return 0;
+}
+
+template <typename T>
+static int gwc_bwd(const T* gvol, const T* L, const T* R, T* gL, T* gR, int64_t B, int64_t C, int64_t H, int64_t W,
+                   int64_t Dq, int64_t G, cudaStream_t st) {
+    const size_t qb = sizeof(GwcQuad<T>);
+    const int64_t cpg = C / G;
+    auto all_aligned = [&](size_t n) {
+        return aligned_to(gvol, n) && aligned_to(L, n) && aligned_to(R, n) && (!gL || aligned_to(gL, n)) &&
+               (!gR || aligned_to(gR, n));
+    };
+    if ((W % 4 == 0) && all_aligned(qb)) {
+        // 16 bits: a CTA's plane run of nact = rows * W/4 quads is a multiple of 16 bytes when W % 8 == 0
+        const bool systolic_ok = std::is_same<T, float>::value || ((W % 8 == 0) && all_aligned(16));
+        bool done = false;
+        int rc = 0;
+        switch (cpg) {
+            case 1: rc = launch_gwc_bwd<T, 1>(gvol, L, R, gL, gR, (int)B, (int)C, (int)G, (int)H, (int)W, (int)Dq, systolic_ok, st, &done); break;
+            case 2: rc = launch_gwc_bwd<T, 2>(gvol, L, R, gL, gR, (int)B, (int)C, (int)G, (int)H, (int)W, (int)Dq, systolic_ok, st, &done); break;
+            case 4: rc = launch_gwc_bwd<T, 4>(gvol, L, R, gL, gR, (int)B, (int)C, (int)G, (int)H, (int)W, (int)Dq, systolic_ok, st, &done); break;
+            case 8: rc = launch_gwc_bwd<T, 8>(gvol, L, R, gL, gR, (int)B, (int)C, (int)G, (int)H, (int)W, (int)Dq, systolic_ok, st, &done); break;
+            default: break;
+        }
+        if (rc != 0) return rc;
+        if (done) return 0;
+    }
+    dim3 grid((unsigned)ceil_div(H * W, 256), (unsigned)C, (unsigned)B);
+    gwc_bwd_scalar_kernel<T><<<grid, 256, 0, st>>>(gvol, L, R, gL, gR, (int)C, (int)G, (int)H, (int)W, (int)Dq);
+    AZ_LAUNCH_CHECK();
+    return 0;
 }
 
 }  // namespace az
@@ -694,26 +866,7 @@ extern "C" int az_gwc_volume_fwd(const float* L, const float* R, float* vol, int
     if (!L || !R || !vol || B <= 0 || C <= 0 || H <= 0 || W <= 0 || Dq <= 0 || G <= 0 || C % G != 0)
         return AZ_ERR_BAD_ARG;
     if (H * W >= (1ll << 31) / 4 || B > 65535 || G > 65535) return AZ_ERR_BAD_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-    const int64_t cpg = C / G;
-    if ((W % 4 == 0) && aligned16(L) && aligned16(R) && aligned16(vol)) {
-        bool done = false;
-        int rc = 0;
-        switch (cpg) {
-            case 1: rc = launch_gwc_fwd<1>(L, R, vol, (int)B, (int)C, (int)G, (int)H, (int)W, (int)Dq, st, &done); break;
-            case 2: rc = launch_gwc_fwd<2>(L, R, vol, (int)B, (int)C, (int)G, (int)H, (int)W, (int)Dq, st, &done); break;
-            case 4: rc = launch_gwc_fwd<4>(L, R, vol, (int)B, (int)C, (int)G, (int)H, (int)W, (int)Dq, st, &done); break;
-            case 8: rc = launch_gwc_fwd<8>(L, R, vol, (int)B, (int)C, (int)G, (int)H, (int)W, (int)Dq, st, &done); break;
-            default: break;
-        }
-        if (rc != 0) return rc;
-        if (done) return 0;
-    }
-    if (Dq > 65535 || B * G > 65535) return AZ_ERR_BAD_ARG;
-    dim3 grid((unsigned)ceil_div(H * W, 256), (unsigned)Dq, (unsigned)(B * G));
-    gwc_fwd_scalar_kernel<<<grid, 256, 0, st>>>(L, R, vol, (int)C, (int)G, (int)H, (int)W, (int)Dq);
-    AZ_LAUNCH_CHECK();
-    return 0;
+    return gwc_fwd(L, R, vol, B, C, H, W, Dq, G, (cudaStream_t)stream);
 }
 
 extern "C" int az_gwc_volume_bwd(const float* gvol, const float* L, const float* R, float* gL, float* gR, int64_t B,
@@ -722,24 +875,37 @@ extern "C" int az_gwc_volume_bwd(const float* gvol, const float* L, const float*
         return AZ_ERR_BAD_ARG;
     if (H * W >= (1ll << 31) / 4 || B > 65535 || C > 65535 || H > 65535) return AZ_ERR_BAD_ARG;
     if (!gL && !gR) return 0;
+    return gwc_bwd(gvol, L, R, gL, gR, B, C, H, W, Dq, G, (cudaStream_t)stream);
+}
+
+extern "C" int az_gwc_volume_fwd_16(const void* L, const void* R, void* vol, int64_t B, int64_t C, int64_t H, int64_t W,
+                                    int64_t Dq, int64_t G, int dtype, void* stream) {
+    if (dtype != AZ_DTYPE_BF16 && dtype != AZ_DTYPE_F16) return AZ_ERR_BAD_ARG;
+    if (!L || !R || !vol || B <= 0 || C <= 0 || H <= 0 || W <= 0 || Dq <= 0 || G <= 0 || C % G != 0)
+        return AZ_ERR_BAD_ARG;
+    if (H * W >= (1ll << 31) / 4 || B > 65535 || G > 65535) return AZ_ERR_BAD_ARG;
     cudaStream_t st = (cudaStream_t)stream;
-    const int64_t cpg = C / G;
-    if ((W % 4 == 0) && aligned16(gvol) && aligned16(L) && aligned16(R) && (!gL || aligned16(gL)) &&
-        (!gR || aligned16(gR))) {
-        bool done = false;
-        int rc = 0;
-        switch (cpg) {
-            case 1: rc = launch_gwc_bwd<1>(gvol, L, R, gL, gR, (int)B, (int)C, (int)G, (int)H, (int)W, (int)Dq, st, &done); break;
-            case 2: rc = launch_gwc_bwd<2>(gvol, L, R, gL, gR, (int)B, (int)C, (int)G, (int)H, (int)W, (int)Dq, st, &done); break;
-            case 4: rc = launch_gwc_bwd<4>(gvol, L, R, gL, gR, (int)B, (int)C, (int)G, (int)H, (int)W, (int)Dq, st, &done); break;
-            case 8: rc = launch_gwc_bwd<8>(gvol, L, R, gL, gR, (int)B, (int)C, (int)G, (int)H, (int)W, (int)Dq, st, &done); break;
-            default: break;
-        }
-        if (rc != 0) return rc;
-        if (done) return 0;
+    if (dtype == AZ_DTYPE_BF16)
+        return gwc_fwd(static_cast<const __nv_bfloat16*>(L), static_cast<const __nv_bfloat16*>(R),
+                       static_cast<__nv_bfloat16*>(vol), B, C, H, W, Dq, G, st);
+    return gwc_fwd(static_cast<const __half*>(L), static_cast<const __half*>(R), static_cast<__half*>(vol), B, C, H, W,
+                   Dq, G, st);
+}
+
+extern "C" int az_gwc_volume_bwd_16(const void* gvol, const void* L, const void* R, void* gL, void* gR, int64_t B,
+                                    int64_t C, int64_t H, int64_t W, int64_t Dq, int64_t G, int dtype, void* stream) {
+    if (dtype != AZ_DTYPE_BF16 && dtype != AZ_DTYPE_F16) return AZ_ERR_BAD_ARG;
+    if (!gvol || !L || !R || B <= 0 || C <= 0 || H <= 0 || W <= 0 || Dq <= 0 || G <= 0 || C % G != 0)
+        return AZ_ERR_BAD_ARG;
+    if (H * W >= (1ll << 31) / 4 || B > 65535 || C > 65535 || H > 65535) return AZ_ERR_BAD_ARG;
+    if (!gL && !gR) return 0;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dtype == AZ_DTYPE_BF16) {
+        using T = __nv_bfloat16;
+        return gwc_bwd(static_cast<const T*>(gvol), static_cast<const T*>(L), static_cast<const T*>(R), static_cast<T*>(gL),
+                       static_cast<T*>(gR), B, C, H, W, Dq, G, st);
     }
-    dim3 grid((unsigned)ceil_div(H * W, 256), (unsigned)C, (unsigned)B);
-    gwc_bwd_scalar_kernel<<<grid, 256, 0, st>>>(gvol, L, R, gL, gR, (int)C, (int)G, (int)H, (int)W, (int)Dq);
-    AZ_LAUNCH_CHECK();
-    return 0;
+    using T = __half;
+    return gwc_bwd(static_cast<const T*>(gvol), static_cast<const T*>(L), static_cast<const T*>(R), static_cast<T*>(gL),
+                   static_cast<T*>(gR), B, C, H, W, Dq, G, st);
 }

@@ -43,7 +43,8 @@ from .ops import (DTYPE16, _cuda_f32, _mask_u8, _ptr, _stream, check_feature_pai
                   soft_argmin_backward_into, soft_argmin_forward_into, upsample_soft_argmin_backward_into,
                   upsample_soft_argmin_forward_into)
 from .ops import concat_volume_backward as concat_volume_backward_into
-from .ops import concat_volume_forward
+from .ops import concat_volume_forward, gwc_volume_forward
+from .ops import gwc_volume_backward as gwc_volume_backward_into
 
 NS = "az_stereo"
 _FLOAT_DTYPES = (torch.float32, *DTYPE16)
@@ -243,21 +244,11 @@ def reproj_loss(tgt: Tensor, src: Tensor, disp: Tensor, mask: Tensor, ps: int = 
 # ---------------------------------------------------------------------------------------------
 # group-wise correlation volume (a3)
 # ---------------------------------------------------------------------------------------------
-def _gwc_dims(L: Tensor, num_disp: int, num_groups: int, what: str):
-    B, C, H, W = L.shape
-    if num_disp <= 0 or num_groups <= 0 or C % num_groups != 0:
-        raise ValueError(f"{what}: num_disp > 0 and num_groups dividing C={C} expected")
-    return B, C, H, W
-
-
 @torch.library.custom_op(f"{NS}::gwc_volume", mutates_args=(), device_types="cuda")
 def gwc_volume(ref: Tensor, tgt: Tensor, num_disp: int, num_groups: int) -> Tensor:
-    L, R = check_feature_pair(ref, tgt, "az_stereo::gwc_volume")
-    B, C, H, W = _gwc_dims(L, num_disp, num_groups, "az_stereo::gwc_volume")
-    vol = torch.empty((B, num_groups, num_disp, H, W), dtype=torch.float32, device=L.device)
-    with torch.cuda.device(L.device):
-        _lib.call("az_gwc_volume_fwd", _ptr(L), _ptr(R), _ptr(vol), B, C, H, W, num_disp, num_groups, _stream(), batch=B)
-    return vol
+    # float32 features, or two bfloat16 / two float16 features (the volume has their dtype; ops.build_gwc_volume)
+    L, R = check_feature_pair(ref, tgt, "az_stereo::gwc_volume", allow16=True)
+    return gwc_volume_forward(L, R, num_disp, num_groups)
 
 
 @gwc_volume.register_fake
@@ -268,16 +259,9 @@ def _(ref, tgt, num_disp, num_groups):
 
 @torch.library.custom_op(f"{NS}::gwc_volume_backward", mutates_args=(), device_types="cuda")
 def gwc_volume_backward(gvol: Tensor, ref: Tensor, tgt: Tensor) -> Tuple[Tensor, Tensor]:
-    L, R = check_feature_pair(ref, tgt, "az_stereo::gwc_volume_backward")
-    g = _cuda_f32(gvol, "grad_volume")
-    if g.dim() != 5 or g.shape[0] != L.shape[0] or tuple(g.shape[3:]) != tuple(L.shape[2:]) or g.device != L.device:
-        raise ValueError("az_stereo::gwc_volume_backward: gvol must be [B,G,Dq,H,W] on the features' device")
-    G, Dq = int(g.shape[1]), int(g.shape[2])
-    B, C, H, W = _gwc_dims(L, Dq, G, "az_stereo::gwc_volume_backward")
-    gL, gR = torch.empty_like(L), torch.empty_like(R)
-    with torch.cuda.device(L.device):
-        _lib.call("az_gwc_volume_bwd", _ptr(g), _ptr(L), _ptr(R), _ptr(gL), _ptr(gR), B, C, H, W, Dq, G, _stream(), batch=B)
-    return gL, gR
+    # gvol has the features' dtype; so have gL, gR
+    L, R = check_feature_pair(ref, tgt, "az_stereo::gwc_volume_backward", allow16=True)
+    return gwc_volume_backward_into(gvol, L, R)
 
 
 @gwc_volume_backward.register_fake

@@ -322,20 +322,63 @@ def volume_conv(ref_feat, tgt_feat, weight, num_disp: int):
 # ----------------------------------------------------------------------------
 # a3 group-wise correlation volume (no reference counterpart)
 # ----------------------------------------------------------------------------
+def gwc_volume_forward(L, R, num_disp: int, num_groups: int):
+    """Enqueues the group-wise correlation volume [B,G,Dq,H,W] of validated features (both float32, or both bfloat16 /
+    both float16: the volume has their dtype, DESIGN.md §4.15).  Shared by GwcVolumeFn and library_ops."""
+    B, C, H, W = L.shape
+    if int(num_disp) <= 0 or int(num_groups) <= 0 or C % int(num_groups) != 0:
+        raise ValueError(f"gwc volume: num_disp > 0 and num_groups dividing C={C} expected")
+    vol = torch.empty((B, int(num_groups), int(num_disp), H, W), dtype=L.dtype, device=L.device)
+    dt = DTYPE16.get(L.dtype)
+    with torch.cuda.device(L.device):
+        if dt is None:
+            _lib.call("az_gwc_volume_fwd", _ptr(L), _ptr(R), _ptr(vol), B, C, H, W, int(num_disp), int(num_groups),
+                      _stream(), batch=B)
+        else:
+            _lib.call("az_gwc_volume_fwd_16", _ptr(L), _ptr(R), _ptr(vol), B, C, H, W, int(num_disp), int(num_groups), dt,
+                      _stream(), batch=B)
+    return vol
+
+
+def gwc_volume_backward(gvol, L, R, need_l: bool = True, need_r: bool = True):
+    """gL, gR (each None when not needed) of the gwc volume for validated features and a CUDA gradient [B,G,Dq,H,W] of
+    the features' dtype on their device; the gradients have that dtype.  Shared by GwcVolumeFn and library_ops."""
+    B, C, H, W = L.shape
+    if not isinstance(gvol, torch.Tensor) or not gvol.is_cuda or gvol.dtype != L.dtype:
+        raise ValueError(f"gwc volume backward: grad_volume must be a {L.dtype} CUDA tensor, got "
+                         f"{getattr(gvol, 'dtype', type(gvol))}")
+    g = gvol.contiguous()
+    if g.dim() != 5 or g.shape[0] != B or tuple(g.shape[3:]) != (H, W) or g.device != L.device:
+        raise ValueError("gwc volume backward: grad_volume must be [B,G,Dq,H,W] on the features' device, got "
+                         f"{tuple(g.shape)}")
+    G, Dq = int(g.shape[1]), int(g.shape[2])
+    if Dq <= 0 or G <= 0 or C % G != 0:
+        raise ValueError(f"gwc volume backward: num_disp > 0 and num_groups dividing C={C} expected")
+    gL = torch.empty_like(L) if need_l else None
+    gR = torch.empty_like(R) if need_r else None
+    dt = DTYPE16.get(L.dtype)
+    with torch.cuda.device(L.device):
+        if dt is None:
+            _lib.call("az_gwc_volume_bwd", _ptr(g), _ptr(L), _ptr(R), _ptr(gL), _ptr(gR), B, C, H, W, Dq, G, _stream(),
+                      batch=B)
+        else:
+            _lib.call("az_gwc_volume_bwd_16", _ptr(g), _ptr(L), _ptr(R), _ptr(gL), _ptr(gR), B, C, H, W, Dq, G, dt,
+                      _stream(), batch=B)
+    return gL, gR
+
+
 class GwcVolumeFn(torch.autograd.Function):
+    """Group-wise correlation volume and its autograd.  Outside torch.autocast, two bfloat16 (or two float16) features
+    give a volume and feature gradients of their dtype, equal to the float32 operator on the widened features followed
+    by .to(dtype), bit for bit (DESIGN.md §4.15); the saved features stay 16-bit.  Inside autocast the inputs are cast to
+    float32 as before."""
+
     @staticmethod
     @_fwd32
     def forward(ctx, ref_feat, tgt_feat, num_disp: int, num_groups: int):
-        L, R = check_feature_pair(ref_feat, tgt_feat, "gwc volume")
-        B, C, H, W = L.shape
-        if int(num_disp) <= 0 or int(num_groups) <= 0 or C % int(num_groups) != 0:
-            raise ValueError(f"gwc volume: num_disp > 0 and num_groups dividing C={C} expected")
-        vol = torch.empty((B, int(num_groups), int(num_disp), H, W), dtype=torch.float32, device=L.device)
-        with torch.cuda.device(L.device):
-            _lib.call("az_gwc_volume_fwd", _ptr(L), _ptr(R), _ptr(vol), B, C, H, W, int(num_disp), int(num_groups),
-                      _stream(), batch=B)
+        L, R = check_feature_pair(ref_feat, tgt_feat, "gwc volume", allow16=True)
+        vol = gwc_volume_forward(L, R, num_disp, num_groups)
         ctx.save_for_backward(L, R)
-        ctx.dims = (B, C, H, W, int(num_disp), int(num_groups))
         return vol
 
     @staticmethod
@@ -343,16 +386,20 @@ class GwcVolumeFn(torch.autograd.Function):
     @_bwd
     def backward(ctx, gvol):
         L, R = ctx.saved_tensors
-        B, C, H, W, Dq, G = ctx.dims
-        g = _cuda_f32(gvol, "grad_volume")
-        gL = torch.empty_like(L) if ctx.needs_input_grad[0] else None
-        gR = torch.empty_like(R) if ctx.needs_input_grad[1] else None
-        with torch.cuda.device(g.device):
-            _lib.call("az_gwc_volume_bwd", _ptr(g), _ptr(L), _ptr(R), _ptr(gL), _ptr(gR), B, C, H, W, Dq, G, _stream(), batch=B)
+        gL, gR = gwc_volume_backward(gvol, L, R, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
         return gL, gR, None, None
 
 
 def build_gwc_volume(ref_feat, tgt_feat, num_disp: int, num_groups: int):
+    """[B,C,H,W] x2 -> [B,num_groups,num_disp,H,W]: vol[b,g,i,y,x] = mean over the channels c of group g of
+    L[b,c,y,x] * R[b,c,y,x-i] (zero for x < i).  float32 features give a float32 volume (also under torch.autocast, whose
+    16-bit features are cast to float32).  Outside autocast, two bfloat16 or two float16 features give a volume and
+    gradients of their dtype.  To keep a native 16-bit volume inside an autocast region, call it with autocast switched
+    off, as PSMNet does for the concat volume (``_native16`` in ``nets/psmnet/_backbone.py``)::
+
+        with torch.autocast("cuda", enabled=False):
+            vol = build_gwc_volume(ref16, tgt16, num_disp, num_groups)
+    """
     return GwcVolumeFn.apply(ref_feat, tgt_feat, num_disp, num_groups)
 
 

@@ -127,6 +127,18 @@ int az_gwc_volume_fwd(const float* L, const float* R, float* vol,
                       int64_t B, int64_t C, int64_t H, int64_t W, int64_t Dq, int64_t G, void* stream);
 int az_gwc_volume_bwd(const float* gvol, const float* L, const float* R, float* gL, float* gR,
                       int64_t B, int64_t C, int64_t H, int64_t W, int64_t Dq, int64_t G, void* stream);
+/* The same operator with 16-bit tensors: L, R, vol, gvol, gL and gR are bf16 or fp16 (dtype AZ_DTYPE_BF16 or
+ * AZ_DTYPE_F16, else AZ_ERR_BAD_ARG).  Each 16-bit value is widened exactly where it is read, every instruction after
+ * that is the fp32 kernels' (the kernel picked by the fp32 rule, or one with the same summation order where a 16-bit
+ * alignment rule excludes it), and each result is rounded ONCE, to nearest even, at its store:
+ *   vol    = RNE16(az_gwc_volume_fwd(L.float(), R.float()))
+ *   gL, gR = RNE16(az_gwc_volume_bwd(gvol.float(), L.float(), R.float()))
+ * bit for bit.  fp16 results too large for the format become +-inf, as .to(torch.float16) makes them.  Size limits and
+ * the NULL-gradient rules are the fp32 entry points'. */
+int az_gwc_volume_fwd_16(const void* L, const void* R, void* vol,
+                         int64_t B, int64_t C, int64_t H, int64_t W, int64_t Dq, int64_t G, int dtype, void* stream);
+int az_gwc_volume_bwd_16(const void* gvol, const void* L, const void* R, void* gL, void* gR,
+                         int64_t B, int64_t C, int64_t H, int64_t W, int64_t Dq, int64_t G, int dtype, void* stream);
 
 /* ---- a4/a5: soft-argmin = F.softmax(cost,1) + DisparityRegression --
  *      nets/psmnet/psmnet.py:200-201,204-205,212-217 + nets/psmnet/psmnet_submodule.py:80-89 ----
